@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 corruption path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): horizontal motion blur k=9 / angle 0 on 256 synthetic
 1360x765 uint8 BGR images PER GPU (device-resident [256,765,1360,3], 799 MB in + 799 MB out,
@@ -11,7 +11,9 @@ scaling: per-GPU work fixed); only per-rank timings are gathered.
 
 One JSON line on stdout (rank 0); see the keys in main().  `--impl reference` times the
 reference's own CPU implementation of the same workload (OpenCV filter2D via oracle/cv2_port.py)
-on the host cores.
+on the host cores.  `--dump-outputs DIR` writes what the last timed step computed (see
+dump_outputs()); the inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -183,8 +185,7 @@ def cpu_baseline():
 def run_reference(args):
     """--impl reference: the reference's own CPU implementation of the SAME workload (configs[1]: motion blur k=9 on 256
     images of 1360x765 per step; OpenCV filter2D through oracle/cv2_port.py, the calls augmentations.py:36-38 makes) on
-    all host cores.  W warm-up + K timed steps, each step one pass over 256 images, timed inside the loop; when K steps
-    take less than 2 s more passes are timed (config.timed_passes) so that the figure is stable."""
+    all host cores.  W warm-up + K timed steps, each step one pass over 256 images, timed inside the loop."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -195,7 +196,7 @@ def run_reference(args):
     else:
         pool = CpuPool()
         try:
-            r = pool.rate("blur", warmup=max(1, args.warmup), passes=args.steps, min_seconds=2.0)
+            r = pool.rate("blur", warmup=max(1, args.warmup), passes=args.steps, min_seconds=0.0)
         finally:
             pool.close()
         v, cores, ms, passes = r["value"], pool.workers, r["ms_per_pass"], r["passes"]
@@ -232,6 +233,25 @@ def bind_to_gpu_cpus(gpu_index):
         return f"unavailable ({type(e).__name__})"
 
 
+DUMP_SAMPLE = 1 << 22   # elements of the seeded sample of the batch: 16 MiB as float32
+
+
+def dump_outputs(out_dir, dst, torch, np):
+    """--dump-outputs: the blurred batch dst [n, 765, 1360, 3] uint8 (799 MB), reduced to 29 MB of .npy files:
+      blur_dst_image0.npy      image 0 in full, float32 [765, 1360, 3]
+      blur_dst_sample.npy      float32 [4 Mi]: dst.reshape(-1) at the sorted flat indices
+                               np.random.default_rng(0).integers(0, dst.numel(), 4 Mi) (the same on every run)
+      blur_dst_image_sums.npy  float64 [n]: the sum of every image's bytes (exact: at most 3 121 200 * 255)"""
+    os.makedirs(out_dir, exist_ok=True)
+    flat = dst.reshape(-1)
+    idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), DUMP_SAMPLE))
+    arrays = {"blur_dst_image0": dst[0].float(),
+              "blur_dst_sample": flat[torch.from_numpy(idx).to(dst.device)].float(),
+              "blur_dst_image_sums": dst.reshape(dst.shape[0], -1).sum(1).double()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def time_device(fn, steps, warmup, torch, dist=None):
     """W untimed + K timed calls of fn() bracketed by barrier + synchronize; CUDA events on the
     current stream; returns this rank's elapsed ms."""
@@ -260,7 +280,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the per-op side measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output of the last one as DIR/<name>.npy (rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the device output of --impl ours")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -300,6 +326,8 @@ def main():
     sampler.start()
     ms = time_device(lambda: plan.blur(src, dst), args.steps, args.warmup, torch, dist)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:   # before the side measurements below reuse dst
+        dump_outputs(args.dump_outputs, dst, torch, np)
     rec = gather_records({"rank": rank, "ms": ms, "images": n})
     max_ms = max(r["ms"] for r in rec)
     total_images = sum(r["images"] for r in rec)

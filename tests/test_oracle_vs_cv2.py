@@ -29,40 +29,3 @@ def test_letterbox_resize_matches_cv2():
         img = synth(h + w, h, w)
         nh, nw, top, left = orc.letterbox_geometry(h, w, 640, 640)
         assert np.array_equal(orc.resize_linear(img, nh, nw), cv2.resize(img, (nw, nh), interpolation=cv2.INTER_LINEAR))
-
-
-def test_reference_build_script_equals_restated_loop(tmp_path):
-    """Build container only (skipped where /root/reference is absent): the UNMODIFIED scripts/build_corrupted_testsets.py
-    run on a small synthetic JPEG tree produces exactly the files the restated loop (oracle ops + cv2 codec, same glob order,
-    np.random.seed(42)) predicts -- the expectation tests/test_gpu_parity.py::test_build_corrupted_testsets_drop_in uses."""
-    import importlib.util
-    import os
-    import sys
-    ref = "/root/reference/scripts/build_corrupted_testsets.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference not mounted")
-    import cv2
-    from tests.helpers import synth
-    shapes = [(120, 200), (97, 133), (64, 64), (81, 90)]
-    img_dir = tmp_path / "yolo" / "images" / "val"
-    img_dir.mkdir(parents=True)
-    (tmp_path / "yolo" / "labels" / "val").mkdir(parents=True)
-    for i, (h, w) in enumerate(shapes):
-        cv2.imwrite(str(img_dir / f"f{i}.jpg"), cv2.GaussianBlur(synth(7000 + i, h, w), (0, 0), 2.0))
-        (tmp_path / "yolo" / "labels" / "val" / f"f{i}.txt").write_text("0 0.5 0.5 0.1 0.1\n")
-    (img_dir / "broken.jpg").write_bytes(b"nope")
-    spec = importlib.util.spec_from_file_location("ref_build", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    mod.YOLO_SRC, mod.OUT_ROOT = tmp_path / "yolo", tmp_path / "out"
-    mod.set_seed(mod.SEED)
-    mod.build_yolo_testsets()
-    np.random.seed(42)
-    for v, op in (("Test_Clean", 0), ("Test_Noise", 1), ("Test_Blur", 2), ("Test_LowRes", 3)):
-        for p in img_dir.glob("*.*"):
-            img = cv2.imread(str(p))
-            out = tmp_path / "out" / "yolo6" / v / "images" / "val" / p.name
-            if img is None:
-                assert not out.exists()
-                continue
-            assert out.read_bytes() == cv2.imencode(p.suffix, orc.apply_op(img, op))[1].tobytes(), (v, p.name)
