@@ -1,6 +1,4 @@
 // api.cu -- extern "C" entry points of librod_b200.so (declared in include/rod_b200.h).
-#include <stdlib.h>
-
 #include <algorithm>
 #include <vector>
 
@@ -135,12 +133,9 @@ extern "C" int rod_plan_launches(const rod_plan* plan, int op) {
         case ROD_OP_NONE: case ROD_OP_NOISE: case ROD_OP_BLUR: return 1;
         case ROD_OP_LOWRES: {  // one launch per non-empty tile list (known once the resize tables exist)
             if (plan->d_shapes == nullptr) return 1;
-            const int n = (plan->n_lowres_tiles > 0) + (plan->n_lowres_x2w_tiles > 0) + (plan->n_lowres_x2w4_tiles > 0) +
-                          (plan->n_lowres_x2_rest_tiles > 0) + (plan->n_lowres_x2p_tiles[0] > 0) + (plan->n_lowres_x2p_tiles[1] > 0) +
-                          (plan->n_lowres_x2p_tiles[2] > 0) + (plan->n_lowres_x2f_tiles[0] > 0) + (plan->n_lowres_x2f_tiles[1] > 0) +
-                          (plan->n_lowres_x2f_tiles[2] > 0) + (plan->n_lowres_x2g_tiles > 0) + (plan->n_lowres_x2h_tiles[0] > 0) +
-                          (plan->n_lowres_x2h_tiles[1] > 0) + (plan->n_lowres_x2h_tiles[2] > 0) + (plan->n_lowres_x2i_tiles[0] > 0) +
-                          (plan->n_lowres_x2i_tiles[1] > 0);
+            // except the full strip list: it runs only when the base pointers are not 4-byte aligned, in place of the others
+            int n = 0;
+            for (int l = 0; l < LR_NUM_LISTS; ++l) n += l != LR_X2_STRIP && plan->lowres[l].n > 0;
             return n > 0 ? n : 1;
         }
         case 100: return 4;  // rod_corrupt_batch_u8: copy + noise + blur + lowres
@@ -246,10 +241,9 @@ extern "C" int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, con
     }
     // Fused path: noise / blur / clean rows are produced inside the letterbox kernel (no full-resolution round trip);
     // only LowRes images go through the scratch.  Needs plain linear letterboxes, the angle-0 blur and Philox sigma
-    // in range; ROD_FUSED_LETTERBOX=0 selects the unfused kernels (benchmark knob).
-    const char* e_fused = getenv("ROD_FUSED_LETTERBOX");
+    // in range.
     const bool fused = plan->lb_all_linear && plan->f2d_ntaps == 0 && blur_supported(k, 0.0) && k >= 3 &&
-                       (noise != nullptr || sigma <= kPhiloxMaxSigma) && !(e_fused && atoi(e_fused) == 0);
+                       (noise != nullptr || sigma <= kPhiloxMaxSigma);
     if (fused) {
         rc = ensure_lowres_tables(plan, factor);
         if (rc != ROD_OK) return rc;
@@ -360,13 +354,9 @@ extern "C" int rod_apply_host(rod_plan* plan, int op, const uint8_t* src_host, u
     if (compat && plan->d_stage_noise == nullptr)
         ROD_CUDA(cudaMalloc((void**)&plan->d_stage_noise, plan->payload_bytes * sizeof(float) + 64));
 
-    // chunking: ~16 MiB of payload per chunk when the layout allows per-chunk byte ranges (knob: ROD_HOST_CHUNK_MB;
-    // measured e2e on a B200 box: 16 MiB 13.9 k img/s, 32: 13.6, 64: 13.7, 128: 13.3)
-    static const uint64_t chunk_bytes = [] {
-        const char* e = getenv("ROD_HOST_CHUNK_MB");
-        const int mb = e ? atoi(e) : 16;
-        return (uint64_t)(mb >= 1 && mb <= 4096 ? mb : 16) << 20;
-    }();
+    // chunking: ~16 MiB of payload per chunk when the layout allows per-chunk byte ranges
+    // (measured e2e on a B200 box: 16 MiB 13.9 k img/s, 32: 13.6, 64: 13.7, 128: 13.3)
+    const uint64_t chunk_bytes = 16ull << 20;
     const int n = plan->n_images;
     std::vector<int> cuts{0};
     if (plan->monotonic && n > 1) {

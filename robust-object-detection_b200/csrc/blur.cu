@@ -9,7 +9,6 @@
 // the reflected halo is written next to it, and every lane then produces 16 output bytes per
 // step from three 128-bit shared-memory loads and stores them with one 128-bit global store.
 // No block-level barrier is used (warps never share data), only __syncwarp().
-#include <stdlib.h>
 
 #include "rod_internal.h"
 
@@ -156,13 +155,12 @@ __global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
 
 int launch_blur(const rod_plan* plan, const uint8_t* src, uint8_t* dst, int k, const uint8_t* opcodes,
                 cudaStream_t stream, int img_lo, int img_hi) {
-    if (plan->n_blur_tiles == 0) return ROD_OK;
+    const auto [tiles, n_tiles] = plan->blur_tiles.range(img_lo, img_hi);
+    if (n_tiles == 0) return ROD_OK;
     BlurParams p;
     p.images = plan->d_images;
-    const int t_lo = plan->blur_tile_start[img_lo], t_hi = plan->blur_tile_start[img_hi];
-    if (t_hi <= t_lo) return ROD_OK;
-    p.tiles = plan->d_blur_tiles + t_lo;
-    p.n_tiles = t_hi - t_lo;
+    p.tiles = tiles;
+    p.n_tiles = n_tiles;
     p.src = src; p.dst = dst; p.opcodes = opcodes; p.k = k;
     // per-warp buffer: kBlurLeft | (shift + 3w rounded up to 16) | 16 (right window) + halo, 16-byte multiple
     const int row_bytes = 3 * plan->max_w;
@@ -176,8 +174,6 @@ int launch_blur(const rod_plan* plan, const uint8_t* src, uint8_t* dst, int k, c
     if (ctas_per_sm < 1) ctas_per_sm = 1;
     // measured on B200 (256 x 1360x765): 4 resident CTAs (32 warps) per SM -> 5.79 TB/s; 5 -> 5.62; 6 -> 5.57; 3 -> 5.66
     if (ctas_per_sm > 4) ctas_per_sm = 4;
-    const char* e_ctas = getenv("ROD_BLUR_CTAS");
-    if (e_ctas && atoi(e_ctas) >= 1 && atoi(e_ctas) <= 4) ctas_per_sm = atoi(e_ctas);
     p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
     ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), stream));
     const int grid = grid_for(plan, (p.n_tiles + warps - 1) / warps, ctas_per_sm);

@@ -117,13 +117,12 @@ __global__ void __launch_bounds__(256) filter2d_kernel(Filter2dParams p) {
 
 int launch_filter2d(const rod_plan* plan, const uint8_t* src, uint8_t* dst, const uint8_t* opcodes, cudaStream_t stream,
                     int img_lo, int img_hi) {
-    if (plan->n_f2d_tiles == 0 || plan->f2d_ntaps == 0) return ROD_OK;
-    const int t_lo = plan->f2d_tile_start[img_lo], t_hi = plan->f2d_tile_start[img_hi];
-    if (t_hi <= t_lo) return ROD_OK;
+    const auto [tiles, n_tiles] = plan->f2d_tiles.range(img_lo, img_hi);
+    if (n_tiles == 0 || plan->f2d_ntaps == 0) return ROD_OK;
     Filter2dParams p;
     p.images = plan->d_images;
-    p.tiles = plan->d_f2d_tiles + t_lo;
-    p.n_tiles = t_hi - t_lo;
+    p.tiles = tiles;
+    p.n_tiles = n_tiles;
     p.src = src; p.dst = dst; p.opcodes = opcodes;
     p.taps = plan->d_f2d_taps;
     p.n_taps = plan->f2d_ntaps;

@@ -655,10 +655,8 @@ int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8
     p.buf_bytes = kFusedLeft + ((3 * plan->max_w + 15) & ~15) + 128;  // also holds two low-res rows (3 * max_w / 2 + 39 each)
     p.xtab_bytes = ((p.out_w * 8 + 15) & ~15) + 16;  // + the broadcast slot of the dynamic tile index
     // 4 rows per tile: more, smaller tiles balance the expensive noise / blur / LowRes rows (measured 6 % faster than 8 at
-    // batch 64, equal at batch 16); knob ROD_FUSED_WARPS
-    const char* e_nw = getenv("ROD_FUSED_WARPS");
-    int nw = 4;
-    if (e_nw && (atoi(e_nw) == 4 || atoi(e_nw) == 8)) nw = atoi(e_nw);
+    // batch 64, equal at batch 16)
+    constexpr int nw = 4;
     // version 2 (row per warp, two columns per lane) whenever out_w is even.  Measured on a B200 (1360x765 sources, seed-42
     // mix): batch 64 152 us (version 1: 161 us), batch 16 43.5 us (43.1 us).  Knob ROD_FUSED_V2 = 0 forces version 1.
     // (Tried and dropped: a version 3 that keeps the NEXT row's source rows in flight during the resampling loop -- four row
@@ -673,39 +671,29 @@ int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8
     p.counter = nullptr;
     if (v2) {   // one output row per warp, dealt round-robin (no work counter: one launch, nothing else on the stream)
         const int ctas = (plan->n_images * p.out_h + nw - 1) / nw;
-        if (nw == 4) {
-            ROD_CUDA(cudaFuncSetAttribute(fused_letterbox2_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            fused_letterbox2_kernel<4><<<grid_for(plan, ctas, per_sm), 128, smem, stream>>>(p);
-        } else {
-            ROD_CUDA(cudaFuncSetAttribute(fused_letterbox2_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            fused_letterbox2_kernel<8><<<grid_for(plan, ctas, per_sm), 256, smem, stream>>>(p);
-        }
+        ROD_CUDA(cudaFuncSetAttribute(fused_letterbox2_kernel<nw>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        fused_letterbox2_kernel<nw><<<grid_for(plan, ctas, per_sm), 32 * nw, smem, stream>>>(p);
         ROD_CUDA(cudaGetLastError());
         return ROD_OK;
     }
     p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
     ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), stream));
     const int tiles = plan->n_images * ((p.out_h + nw - 1) / nw);
-    if (nw == 4) {
-        ROD_CUDA(cudaFuncSetAttribute(fused_letterbox_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        fused_letterbox_kernel<4><<<grid_for(plan, tiles, per_sm), 128, smem, stream>>>(p);
-    } else {
-        ROD_CUDA(cudaFuncSetAttribute(fused_letterbox_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        fused_letterbox_kernel<8><<<grid_for(plan, tiles, per_sm), 256, smem, stream>>>(p);
-    }
+    ROD_CUDA(cudaFuncSetAttribute(fused_letterbox_kernel<nw>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fused_letterbox_kernel<nw><<<grid_for(plan, tiles, per_sm), 32 * nw, smem, stream>>>(p);
     ROD_CUDA(cudaGetLastError());
     return ROD_OK;
 }
 
 int launch_letterbox(const rod_plan* plan, const uint8_t* img, const uint8_t* src, const uint8_t* opcodes, void* out_f16,
                      int pad_value, cudaStream_t stream) {
-    if (plan->n_lb_tiles == 0) return ROD_OK;
+    if (plan->lb_tiles.n == 0) return ROD_OK;
     LbParams p;
     p.images = plan->d_images;
     p.lb = plan->d_lb;
     p.tab = plan->d_lb_tab;
-    p.tiles = plan->d_lb_tiles;
-    p.n_tiles = plan->n_lb_tiles;
+    p.tiles = plan->lb_tiles.d;
+    p.n_tiles = plan->lb_tiles.n;
     p.img = img;
     p.src = src;
     p.opcodes = opcodes;
@@ -713,7 +701,7 @@ int launch_letterbox(const rod_plan* plan, const uint8_t* img, const uint8_t* sr
     p.out_h = plan->lb_out_h;
     p.out_w = plan->lb_out_w;
     p.pad = pad_value;
-    const int grid = grid_for(plan, plan->n_lb_tiles, 8);
+    const int grid = grid_for(plan, plan->lb_tiles.n, 8);
     letterbox_kernel<<<grid, 256, 0, stream>>>(p);
     ROD_CUDA(cudaGetLastError());
     return ROD_OK;

@@ -11,7 +11,6 @@
 //                  per source row into a float buffer, then the y taps -> low-res tile P (u8, shared)
 //     phase C1   : horizontal fixed-point pass  hx = (P[s0]*a0 + P[s1]*a1) >> 4   (u16, shared)
 //     phase C2   : vertical pass + pack; each thread owns 8 byte columns and marches down 8 rows
-#include <stdlib.h>
 
 #include <algorithm>
 #include <mutex>
@@ -311,8 +310,8 @@ __device__ __forceinline__ void x2_emit_row(const float* xlo, const float* xhi, 
     }
 }
 
-template <int NT, int MINB>
-__global__ void __launch_bounds__(NT, MINB) lowres_x2_kernel(LowresX2Params p) {
+template <int NT>
+__global__ void __launch_bounds__(NT, 4) lowres_x2_kernel(LowresX2Params p) {
     extern __shared__ __align__(16) uint8_t smem[];
     for (int ti = blockIdx.x; ti < p.n_tiles; ti += gridDim.x) {
         const Tile t = p.tiles[ti];
@@ -562,9 +561,15 @@ struct X2wWarpTables {
     uint32_t ys[kX2wMaxBandRows]; // s0 | s1 << 16 per output row
 };
 
+// Resident CTAs per SM of the band kernels: their __launch_bounds__ minimum and the grid of their launches.
+// Measured on a B200 (128 x 1920x1080): lowres_x2p_kernel 3 CTAs/SM 5.88 TB/s, 4: 5.79, 2: 5.17.  The float-tap kernels
+// are issue-bound and gain from more warps: lowres_x2f_kernel 4: 3.69, 3: 3.34, 2: 2.74 TB/s.  lowres_x2i_kernel at 4
+// (128 registers): -5...+1 % (DESIGN section 4).  lowres_x2w_kernel: see below.
+constexpr int kX2wCtasPerSm = 4, kX2pCtasPerSm = 3, kX2fCtasPerSm = 4, kX2hCtasPerSm = 4, kX2gCtasPerSm = 3, kX2iCtasPerSm = 3;
+
 template <bool AL8>  // 128 registers, 4 CTAs per SM.  Measured alternatives: 96 registers / 5 CTAs (spills) -35 %;
                      // a 4-pixel-chunk variant with 80 registers / 6 CTAs -14 %: the kernel is issue-bound, not latency-bound
-__global__ void __launch_bounds__(128, 4) lowres_x2w_kernel(LowresX2wParams p) {
+__global__ void __launch_bounds__(128, kX2wCtasPerSm) lowres_x2w_kernel(LowresX2wParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
     X2wWarpTables& tb = reinterpret_cast<X2wWarpTables*>(smem)[warp];
@@ -847,8 +852,8 @@ __device__ __forceinline__ void x2p_tile(const LowresX2wParams& p, const Tile& t
 }
 
 // U: copy unit in bytes (16: image width a multiple of 16 and 16-byte aligned rows; 8; 4)
-template <int U, int MINB>
-__global__ void __launch_bounds__(128, MINB) lowres_x2p_kernel(LowresX2wParams p) {
+template <int U>
+__global__ void __launch_bounds__(128, kX2pCtasPerSm) lowres_x2p_kernel(LowresX2wParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     X2pWarpSmem& ws = reinterpret_cast<X2pWarpSmem*>(smem)[threadIdx.x >> 5];
@@ -1036,8 +1041,8 @@ __device__ __forceinline__ void x2f_tile(const LowresX2wParams& p, const Tile& t
     cp_async_wait<0>();
 }
 
-template <int U, int MINB>
-__global__ void __launch_bounds__(128, MINB) lowres_x2f_kernel(LowresX2wParams p) {
+template <int U>
+__global__ void __launch_bounds__(128, kX2fCtasPerSm) lowres_x2f_kernel(LowresX2wParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     X2fWarpSmem& ws = reinterpret_cast<X2fWarpSmem*>(smem)[threadIdx.x >> 5];
@@ -1284,8 +1289,8 @@ __device__ __forceinline__ void x2h_tile(const LowresX2wParams& p, const Tile& t
     cp_async_wait<0>();
 }
 
-template <int U, int MINB>
-__global__ void __launch_bounds__(128, MINB) lowres_x2h_kernel(LowresX2wParams p) {
+template <int U>
+__global__ void __launch_bounds__(128, kX2hCtasPerSm) lowres_x2h_kernel(LowresX2wParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     X2hWarpSmem& ws = reinterpret_cast<X2hWarpSmem*>(smem)[threadIdx.x >> 5];
@@ -1376,8 +1381,7 @@ __device__ __forceinline__ void x2g_store_row(uint8_t* ob, bool stores, const fl
         if (lane + 32 * k < nbody) stg4s(gb + lane + 32 * k, sb[lane + 32 * k]);
 }
 
-template <int MINB>
-__global__ void __launch_bounds__(128, MINB) lowres_x2g_kernel(LowresX2wParams p) {
+__global__ void __launch_bounds__(128, kX2gCtasPerSm) lowres_x2g_kernel(LowresX2wParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     X2fWarpSmem& ws = reinterpret_cast<X2fWarpSmem*>(smem)[threadIdx.x >> 5];
@@ -1821,8 +1825,8 @@ __device__ __forceinline__ void x2i_tile(const LowresX2wParams& p, const Tile& t
     cp_async_wait<0>();
 }
 
-template <bool CARRY, int MINB>
-__global__ void __launch_bounds__(128, MINB) lowres_x2i_kernel(LowresX2wParams p) {
+template <bool CARRY>
+__global__ void __launch_bounds__(128, kX2iCtasPerSm) lowres_x2i_kernel(LowresX2wParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31;
     X2iWarpSmem& ws = reinterpret_cast<X2iWarpSmem*>(smem)[threadIdx.x >> 5];
@@ -1846,237 +1850,105 @@ namespace {
 struct LrStreams {
     cudaStream_t s[3];
     int n, i;
-    bool lanes = false;   // issue-bound kernels on s[1], the HBM-bound ones on s[0]: a kernel of each kind shares every SM
-    cudaStream_t pick() {
-        if (lanes && n == 3) return s[0];
-        const cudaStream_t r = s[i]; i = (i + 1) % n; return r;
-    }
-    cudaStream_t lane(bool issue_bound) { return (lanes && n == 3 && issue_bound) ? s[1] : pick(); }
+    cudaStream_t pick() { const cudaStream_t r = s[i]; i = (i + 1) % n; return r; }
 };
 
-int env_int(const char* name, int lo, int hi, int dflt) {
-    const char* e = getenv(name);
-    if (!e) return dflt;
-    const int v = atoi(e);
-    return (v >= lo && v <= hi) ? v : dflt;
-}
+using BandKernel = void (*)(LowresX2wParams);
+// staged kernels by copy unit: 16, 8, 4 bytes
+const BandKernel kX2pKernels[3] = {lowres_x2p_kernel<16>, lowres_x2p_kernel<8>, lowres_x2p_kernel<4>};
+const BandKernel kX2fKernels[3] = {lowres_x2f_kernel<16>, lowres_x2f_kernel<8>, lowres_x2f_kernel<4>};
+const BandKernel kX2hKernels[3] = {lowres_x2h_kernel<16>, lowres_x2h_kernel<8>, lowres_x2h_kernel<4>};
 
+// The order of the launches decides the stream each one is dealt to: generic, x2g, x2i, the staged kernels, x2w, strips.
 int launch_lowres_lists(const rod_plan* plan, const uint8_t* src, uint8_t* dst, const uint8_t* opcodes, LrStreams& ls,
                         int img_lo, int img_hi) {
-    // generic tiles (shapes that are not exact-2x in x)
-    {
-        const int t_lo = plan->lowres_tile_start[img_lo], t_hi = plan->lowres_tile_start[img_hi];
-        if (t_hi > t_lo) {
-            LowresParams p;
-            const cudaStream_t lst = ls.pick();
-            p.images = plan->d_images;
-            p.tiles = plan->d_lowres_tiles + t_lo;
-            p.n_tiles = t_hi - t_lo;
-            p.shapes = plan->d_shapes;
-            p.tab = plan->d_tab;
-            p.src = src; p.dst = dst; p.opcodes = opcodes;
-            p.half_rows = plan->lowres_half_rows;
-            p.p_pitch = (3 * (plan->lowres_half_cols + 3) + 15) & ~15;
-            p.hb_pitch = 3 * plan->lowres_half_cols + 1;
-            const size_t un = (std::max((size_t)plan->lowres_src_rows * p.hb_pitch * 4, (size_t)p.half_rows * kHxPitch * 2) + 15) & ~(size_t)15;
-            p.union_bytes = (int)un;
-            const size_t smem = (((size_t)p.half_rows * p.p_pitch + 15) & ~(size_t)15) + un + (size_t)p.half_rows * (2 + kMaxAreaTaps) * 4 + 16;
-            if (smem > 227 * 1024) return ROD_ERR_UNSUPPORTED;
-            ROD_CUDA(cudaFuncSetAttribute(lowres_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            int ctas_per_sm = (int)((220 * 1024) / (smem + 1024));
-            ctas_per_sm = ctas_per_sm < 1 ? 1 : (ctas_per_sm > 3 ? 3 : ctas_per_sm);
-            lowres_kernel<<<grid_for(plan, p.n_tiles, ctas_per_sm), 256, smem, lst>>>(p);
-            ROD_CUDA(cudaGetLastError());
-        }
-    }
-    // odd widths at factor 0.5: the staged odd-width kernel (no alignment requirement)
-    if (plan->n_lowres_x2g_tiles > 0) {
-        const int t_lo = plan->lowres_x2g_tile_start[img_lo], t_hi = plan->lowres_x2g_tile_start[img_hi];
-        if (t_hi > t_lo) {
-            LowresX2wParams p;
-            const cudaStream_t lst = ls.lane(true);
-            p.images = plan->d_images;
-            p.tiles = plan->d_lowres_x2g_tiles + t_lo;
-            p.n_tiles = t_hi - t_lo;
-            p.shapes = plan->d_shapes;
-            p.tab = plan->d_tab;
-            p.src = src; p.dst = dst; p.opcodes = opcodes;
-            p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
-            ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), lst));
-            const int ctas = (p.n_tiles + 3) / 4;
-            const size_t smem = 4 * sizeof(X2fWarpSmem);
-            int per_sm = 3;  // knob ROD_X2G_CTAS = 2 | 3 | 4
-            const char* e_ctas = getenv("ROD_X2G_CTAS");
-            if (e_ctas && atoi(e_ctas) >= 2 && atoi(e_ctas) <= 4) per_sm = atoi(e_ctas);
-#define ROD_X2G_LAUNCH(B)                                                                                              \
-    do {                                                                                                               \
-        ROD_CUDA(cudaFuncSetAttribute(lowres_x2g_kernel<B>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        lowres_x2g_kernel<B><<<grid_for(plan, ctas, B), 128, smem, lst>>>(p);                                       \
-    } while (0)
-            if (per_sm == 2) ROD_X2G_LAUNCH(2);
-            else if (per_sm == 4) ROD_X2G_LAUNCH(4);
-            else ROD_X2G_LAUNCH(3);
-#undef ROD_X2G_LAUNCH
-            ROD_CUDA(cudaGetLastError());
-        }
-    }
-    // ... and of those, the shapes with a regular y axis: the low-res-row loop kernel ([0]: odd h, carried tap row; [1]: even h)
-    auto launch_x2i = [&]() -> int {
-    for (int u = 0; u < 2; ++u) {
-        if (plan->n_lowres_x2i_tiles[u] == 0) continue;
-        const int t_lo = plan->lowres_x2i_tile_start[u][img_lo], t_hi = plan->lowres_x2i_tile_start[u][img_hi];
-        if (t_hi <= t_lo) continue;
+    // tile list `l` with a band kernel: four warps per CTA take tiles from a fresh work counter (launches of one plan may
+    // overlap on different streams), grid sized for `per_sm` resident CTAs
+    auto band = [&](int l, BandKernel kernel, size_t smem, int per_sm) -> int {
+        const auto [tiles, n_tiles] = plan->lowres[l].range(img_lo, img_hi);
+        if (n_tiles == 0) return ROD_OK;
         LowresX2wParams p;
-        const cudaStream_t lst = ls.lane(true);
+        const cudaStream_t lst = ls.pick();
         p.images = plan->d_images;
-        p.tiles = plan->d_lowres_x2i_tiles[u] + t_lo;
-        p.n_tiles = t_hi - t_lo;
+        p.tiles = tiles;
+        p.n_tiles = n_tiles;
         p.shapes = plan->d_shapes;
         p.tab = plan->d_tab;
         p.src = src; p.dst = dst; p.opcodes = opcodes;
         p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
         ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), lst));
-        const int ctas = (p.n_tiles + 3) / 4;
-        const size_t smem = 4 * sizeof(X2iWarpSmem);
-        int per_sm = 3;  // knob ROD_X2I_CTAS = 2 | 3 | 4
-        const char* e_ctas = getenv("ROD_X2I_CTAS");
-        if (e_ctas && atoi(e_ctas) >= 2 && atoi(e_ctas) <= 4) per_sm = atoi(e_ctas);
-        const int grid_mult = env_int("ROD_X2I_GRID", 1, 4, per_sm);
-#define ROD_X2I_LAUNCH(C, B)                                                                                              \
-    do {                                                                                                                  \
-        ROD_CUDA(cudaFuncSetAttribute(lowres_x2i_kernel<C, B>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-        lowres_x2i_kernel<C, B><<<grid_for(plan, ctas, grid_mult), 128, smem, lst>>>(p);                                       \
-    } while (0)
-        if (u == 0) {
-            if (per_sm == 2) ROD_X2I_LAUNCH(true, 2);
-            else if (per_sm == 4) ROD_X2I_LAUNCH(true, 4);
-            else ROD_X2I_LAUNCH(true, 3);
-        } else {
-            if (per_sm == 2) ROD_X2I_LAUNCH(false, 2);
-            else if (per_sm == 4) ROD_X2I_LAUNCH(false, 4);
-            else ROD_X2I_LAUNCH(false, 3);
-        }
-#undef ROD_X2I_LAUNCH
+        ROD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kernel<<<grid_for(plan, (n_tiles + 3) / 4, per_sm), 128, smem, lst>>>(p);
+        ROD_CUDA(cudaGetLastError());
+        return ROD_OK;
+    };
+    // generic tiles (shapes that are not exact-2x in x)
+    if (const auto [tiles, n_tiles] = plan->lowres[LR_GENERIC].range(img_lo, img_hi); n_tiles > 0) {
+        LowresParams p;
+        const cudaStream_t lst = ls.pick();
+        p.images = plan->d_images;
+        p.tiles = tiles;
+        p.n_tiles = n_tiles;
+        p.shapes = plan->d_shapes;
+        p.tab = plan->d_tab;
+        p.src = src; p.dst = dst; p.opcodes = opcodes;
+        p.half_rows = plan->lowres_half_rows;
+        p.p_pitch = (3 * (plan->lowres_half_cols + 3) + 15) & ~15;
+        p.hb_pitch = 3 * plan->lowres_half_cols + 1;
+        const size_t un = (std::max((size_t)plan->lowres_src_rows * p.hb_pitch * 4, (size_t)p.half_rows * kHxPitch * 2) + 15) & ~(size_t)15;
+        p.union_bytes = (int)un;
+        const size_t smem = (((size_t)p.half_rows * p.p_pitch + 15) & ~(size_t)15) + un + (size_t)p.half_rows * (2 + kMaxAreaTaps) * 4 + 16;
+        if (smem > 227 * 1024) return ROD_ERR_UNSUPPORTED;
+        ROD_CUDA(cudaFuncSetAttribute(lowres_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int ctas_per_sm = (int)((220 * 1024) / (smem + 1024));
+        ctas_per_sm = ctas_per_sm < 1 ? 1 : (ctas_per_sm > 3 ? 3 : ctas_per_sm);
+        lowres_kernel<<<grid_for(plan, p.n_tiles, ctas_per_sm), 256, smem, lst>>>(p);
         ROD_CUDA(cudaGetLastError());
     }
-    return ROD_OK;
-    };
-    const bool x2i_last = env_int("ROD_LR_X2I_LAST", 0, 1, 0) != 0;
-    if (!x2i_last) { const int rc = launch_x2i(); if (rc != ROD_OK) return rc; }
-    // exact-2x shapes: warp-marching kernel when the rows are 4-byte aligned, full-width strips otherwise
-    const int n_packed = plan->n_lowres_x2p_tiles[0] + plan->n_lowres_x2p_tiles[1] + plan->n_lowres_x2p_tiles[2] +
-                         plan->n_lowres_x2f_tiles[0] + plan->n_lowres_x2f_tiles[1] + plan->n_lowres_x2f_tiles[2] +
-                         plan->n_lowres_x2h_tiles[0] + plan->n_lowres_x2h_tiles[1] + plan->n_lowres_x2h_tiles[2];
-    const bool use_bands = (plan->n_lowres_x2w_tiles + plan->n_lowres_x2w4_tiles + n_packed) > 0 &&
+    // odd widths at factor 0.5: the staged odd-width kernel (no alignment requirement) ...
+    int rc = band(LR_X2G, lowres_x2g_kernel, 4 * sizeof(X2fWarpSmem), kX2gCtasPerSm);
+    // ... and of those, the shapes with a regular y axis: the low-res-row loop kernel (odd h: carried tap row; even h)
+    if (rc == ROD_OK) rc = band(LR_X2I_CARRY, lowres_x2i_kernel<true>, 4 * sizeof(X2iWarpSmem), kX2iCtasPerSm);
+    if (rc == ROD_OK) rc = band(LR_X2I_EVEN, lowres_x2i_kernel<false>, 4 * sizeof(X2iWarpSmem), kX2iCtasPerSm);
+    if (rc != ROD_OK) return rc;
+    // exact-2x shapes: warp-marching kernels when the rows are 4-byte aligned, full-width strips otherwise
+    int n_packed = 0;
+    for (int l = LR_X2P16; l <= LR_X2H4; ++l) n_packed += plan->lowres[l].n;
+    const bool use_bands = (plan->lowres[LR_X2W8].n + plan->lowres[LR_X2W4].n + n_packed) > 0 &&
                            (((uintptr_t)src) & 3) == 0 && (n_packed == 0 || (((uintptr_t)dst) & 3) == 0);
-    // staged kernels (packed-integer: exact 2x in both axes; float taps: exact-2x width only), one launch per copy-unit class
-    for (int kind = 0; kind < 3 && use_bands; ++kind) {   // 0: packed-integer, 1: float taps, 2: regular three-tap
-        for (int u = 0; u < 3; ++u) {
-            const int n_list = kind == 0 ? plan->n_lowres_x2p_tiles[u] : kind == 1 ? plan->n_lowres_x2f_tiles[u] : plan->n_lowres_x2h_tiles[u];
-            if (n_list == 0) continue;
-            const std::vector<int>& st = kind == 0 ? plan->lowres_x2p_tile_start[u] : kind == 1 ? plan->lowres_x2f_tile_start[u] : plan->lowres_x2h_tile_start[u];
-            const int t_lo = st[img_lo], t_hi = st[img_hi];
-            if (t_hi <= t_lo) continue;
-            LowresX2wParams p;
-            const cudaStream_t lst = ls.lane(kind != 0);
-            p.images = plan->d_images;
-            p.tiles = (kind == 0 ? plan->d_lowres_x2p_tiles[u] : kind == 1 ? plan->d_lowres_x2f_tiles[u] : plan->d_lowres_x2h_tiles[u]) + t_lo;
-            p.n_tiles = t_hi - t_lo;
-            p.shapes = plan->d_shapes;
-            p.tab = plan->d_tab;
-            p.src = src; p.dst = dst; p.opcodes = opcodes;
-            p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
-            ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), lst));
-            const int ctas = (p.n_tiles + 3) / 4;
-            // measured on a B200 (128 x 1920x1080, packed): 3 CTAs/SM 5.88 TB/s, 4: 5.79, 2: 5.17; knobs ROD_X2P_CTAS / ROD_X2F_CTAS
-            int per_sm = kind == 0 ? 3 : 4;  // the float-tap kernel is issue-bound: more warps win (4: 3.69, 3: 3.34, 2: 2.74 TB/s)
-            const char* e_ctas = getenv(kind == 0 ? "ROD_X2P_CTAS" : kind == 1 ? "ROD_X2F_CTAS" : "ROD_X2H_CTAS");
-            if (e_ctas && atoi(e_ctas) >= 2 && atoi(e_ctas) <= 4) per_sm = atoi(e_ctas);
-            const int grid_mult = env_int(kind == 0 ? "ROD_X2P_GRID" : kind == 1 ? "ROD_X2F_GRID" : "ROD_X2H_GRID", 1, 4, per_sm);
-            // the list's copy unit holds for offsets and pitches; the base pointers may be less aligned
-            const uintptr_t base = (uintptr_t)src | (uintptr_t)dst;
-            const int unit = std::min(u == 0 ? 16 : (u == 1 ? 8 : 4), (base & 15) == 0 ? 16 : ((base & 7) == 0 ? 8 : 4));
-            const size_t smem = 4 * (kind == 0 ? sizeof(X2pWarpSmem) : kind == 1 ? sizeof(X2fWarpSmem) : sizeof(X2hWarpSmem));
-#define ROD_STAGED_LAUNCH(K, U, B)                                                                         \
-    do {                                                                                                   \
-        ROD_CUDA(cudaFuncSetAttribute(K<U, B>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-        K<U, B><<<grid_for(plan, ctas, grid_mult), 128, smem, lst>>>(p);                                        \
-    } while (0)
-#define ROD_STAGED_LAUNCH_B(K, U)                                 \
-    do {                                                          \
-        if (per_sm == 2) ROD_STAGED_LAUNCH(K, U, 2);              \
-        else if (per_sm == 4) ROD_STAGED_LAUNCH(K, U, 4);         \
-        else ROD_STAGED_LAUNCH(K, U, 3);                          \
-    } while (0)
-#define ROD_STAGED_LAUNCH_U(K)                                    \
-    do {                                                          \
-        if (unit == 16) ROD_STAGED_LAUNCH_B(K, 16);               \
-        else if (unit == 8) ROD_STAGED_LAUNCH_B(K, 8);            \
-        else ROD_STAGED_LAUNCH_B(K, 4);                           \
-    } while (0)
-            if (kind == 0) ROD_STAGED_LAUNCH_U(lowres_x2p_kernel);
-            else if (kind == 1) ROD_STAGED_LAUNCH_U(lowres_x2f_kernel);
-            else ROD_STAGED_LAUNCH_U(lowres_x2h_kernel);
-#undef ROD_STAGED_LAUNCH_U
-#undef ROD_STAGED_LAUNCH_B
-#undef ROD_STAGED_LAUNCH
-            ROD_CUDA(cudaGetLastError());
-        }
-    }
-    if (x2i_last) { const int rc = launch_x2i(); if (rc != ROD_OK) return rc; }
     if (use_bands) {
-        const size_t smem = 4 * sizeof(X2wWarpTables);
-        for (int pass = 0; pass < 2; ++pass) {  // 0: images with 8-byte aligned rows (64-bit loads), 1: the others
-            const std::vector<int>& st = pass == 0 ? plan->lowres_x2w_tile_start : plan->lowres_x2w4_tile_start;
-            const Tile* tl = pass == 0 ? plan->d_lowres_x2w_tiles : plan->d_lowres_x2w4_tiles;
-            if ((pass == 0 ? plan->n_lowres_x2w_tiles : plan->n_lowres_x2w4_tiles) == 0) continue;
-            const int t_lo = st[img_lo], t_hi = st[img_hi];
-            if (t_hi <= t_lo) continue;
-            LowresX2wParams p;
-            const cudaStream_t lst = ls.pick();
-            p.images = plan->d_images;
-            p.tiles = tl + t_lo;
-            p.n_tiles = t_hi - t_lo;
-            p.shapes = plan->d_shapes;
-            p.tab = plan->d_tab;
-            p.src = src; p.dst = dst; p.opcodes = opcodes;
-            // a fresh counter per launch (ring of 256): launches of one plan may overlap on different streams
-            p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
-            ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), lst));
-            const int ctas = (p.n_tiles + 3) / 4;
-            int per_sm = 4;  // benchmark knob: ROD_X2W_CTAS
-            const char* e_ctas = getenv("ROD_X2W_CTAS");
-            if (e_ctas && atoi(e_ctas) >= 1 && atoi(e_ctas) <= 4) per_sm = atoi(e_ctas);
-            if (pass == 0 && (((uintptr_t)src) & 7) == 0) lowres_x2w_kernel<true><<<grid_for(plan, ctas, per_sm), 128, smem, lst>>>(p);
-            else lowres_x2w_kernel<false><<<grid_for(plan, ctas, per_sm), 128, smem, lst>>>(p);
-            ROD_CUDA(cudaGetLastError());
-        }
+        // staged kernels (packed-integer: exact 2x in both axes; float taps: exact-2x width only; regular three-tap), one
+        // launch per copy-unit class.  The list's copy unit holds for offsets and pitches; the base pointers may be less
+        // aligned.
+        const uintptr_t base = (uintptr_t)src | (uintptr_t)dst;
+        const int base_unit = (base & 15) == 0 ? 0 : ((base & 7) == 0 ? 1 : 2);
+        for (int u = 0; u < 3 && rc == ROD_OK; ++u)
+            rc = band(LR_X2P16 + u, kX2pKernels[std::max(u, base_unit)], 4 * sizeof(X2pWarpSmem), kX2pCtasPerSm);
+        for (int u = 0; u < 3 && rc == ROD_OK; ++u)
+            rc = band(LR_X2F16 + u, kX2fKernels[std::max(u, base_unit)], 4 * sizeof(X2fWarpSmem), kX2fCtasPerSm);
+        for (int u = 0; u < 3 && rc == ROD_OK; ++u)
+            rc = band(LR_X2H16 + u, kX2hKernels[std::max(u, base_unit)], 4 * sizeof(X2hWarpSmem), kX2hCtasPerSm);
+        // warp-marching kernel: images with 8-byte aligned rows (64-bit loads), then the others
+        const BandKernel x2w8 = (((uintptr_t)src) & 7) == 0 ? lowres_x2w_kernel<true> : lowres_x2w_kernel<false>;
+        if (rc == ROD_OK) rc = band(LR_X2W8, x2w8, 4 * sizeof(X2wWarpTables), kX2wCtasPerSm);
+        if (rc == ROD_OK) rc = band(LR_X2W4, lowres_x2w_kernel<false>, 4 * sizeof(X2wWarpTables), kX2wCtasPerSm);
+        if (rc != ROD_OK) return rc;
     }
-    {
-        const std::vector<int>& starts = use_bands ? plan->lowres_x2_rest_tile_start : plan->lowres_x2_tile_start;
-        const Tile* tiles = use_bands ? plan->d_lowres_x2_rest_tiles : plan->d_lowres_x2_tiles;
-        const int t_lo = starts[img_lo], t_hi = starts[img_hi];
-        if (t_hi > t_lo) {
-            LowresX2Params p;
-            const cudaStream_t lst = ls.pick();
-            p.images = plan->d_images;
-            p.tiles = tiles + t_lo;
-            p.n_tiles = t_hi - t_lo;
-            p.shapes = plan->d_shapes;
-            p.tab = plan->d_tab;
-            p.src = src; p.dst = dst; p.opcodes = opcodes;
-            const size_t smem = plan->lowres_x2_smem;
-            int ctas_per_sm = (int)((220 * 1024) / (smem + 1024));
-            ctas_per_sm = ctas_per_sm < 1 ? 1 : ctas_per_sm;
-            if (plan->lowres_x2_threads == 128) {
-                ROD_CUDA(cudaFuncSetAttribute(lowres_x2_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                lowres_x2_kernel<128, 4><<<grid_for(plan, p.n_tiles, ctas_per_sm > 4 ? 4 : ctas_per_sm), 128, smem, lst>>>(p);
-            } else {
-                ROD_CUDA(cudaFuncSetAttribute(lowres_x2_kernel<256, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                lowres_x2_kernel<256, 2><<<grid_for(plan, p.n_tiles, ctas_per_sm > 2 ? 2 : ctas_per_sm), 256, smem, lst>>>(p);
-            }
-            ROD_CUDA(cudaGetLastError());
-        }
+    if (const auto [tiles, n_tiles] = plan->lowres[use_bands ? LR_X2_REST : LR_X2_STRIP].range(img_lo, img_hi); n_tiles > 0) {
+        LowresX2Params p;
+        const cudaStream_t lst = ls.pick();
+        p.images = plan->d_images;
+        p.tiles = tiles;
+        p.n_tiles = n_tiles;
+        p.shapes = plan->d_shapes;
+        p.tab = plan->d_tab;
+        p.src = src; p.dst = dst; p.opcodes = opcodes;
+        const size_t smem = plan->lowres_x2_smem;
+        int ctas_per_sm = (int)((220 * 1024) / (smem + 1024));
+        ctas_per_sm = ctas_per_sm < 1 ? 1 : ctas_per_sm;
+        ROD_CUDA(cudaFuncSetAttribute(lowres_x2_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        lowres_x2_kernel<128><<<grid_for(plan, p.n_tiles, ctas_per_sm > 4 ? 4 : ctas_per_sm), 128, smem, lst>>>(p);
+        ROD_CUDA(cudaGetLastError());
     }
     return ROD_OK;
 }
@@ -2084,19 +1956,12 @@ int launch_lowres_lists(const rod_plan* plan, const uint8_t* src, uint8_t* dst, 
 
 int launch_lowres(const rod_plan* plan, const uint8_t* src, uint8_t* dst, const uint8_t* opcodes,
                   cudaStream_t stream, int img_lo, int img_hi) {
-    auto in_range = [&](int n, const std::vector<int>& st) { return n > 0 && st[img_hi] > st[img_lo]; };
-    int n_lists = in_range(plan->n_lowres_tiles, plan->lowres_tile_start) + in_range(plan->n_lowres_x2g_tiles, plan->lowres_x2g_tile_start) +
-                  in_range(plan->n_lowres_x2w_tiles, plan->lowres_x2w_tile_start) + in_range(plan->n_lowres_x2w4_tiles, plan->lowres_x2w4_tile_start) +
-                  in_range(plan->n_lowres_x2_rest_tiles, plan->lowres_x2_rest_tile_start);
-    for (int u = 0; u < 3; ++u)
-        n_lists += in_range(plan->n_lowres_x2p_tiles[u], plan->lowres_x2p_tile_start[u]) + in_range(plan->n_lowres_x2f_tiles[u], plan->lowres_x2f_tile_start[u]) +
-                   in_range(plan->n_lowres_x2h_tiles[u], plan->lowres_x2h_tile_start[u]);
-    for (int u = 0; u < 2; ++u) n_lists += in_range(plan->n_lowres_x2i_tiles[u], plan->lowres_x2i_tile_start[u]);
-    const char* e_conc = getenv("ROD_LOWRES_CONCURRENT");
+    int n_lists = 0;  // the full strip list replaces the others when it runs
+    for (int l = 0; l < LR_NUM_LISTS; ++l) n_lists += l != LR_X2_STRIP && plan->lowres[l].range(img_lo, img_hi).second > 0;
     LrStreams ls;
     ls.s[0] = stream; ls.s[1] = ls.s[2] = nullptr;
     ls.n = 1; ls.i = 0;
-    if (n_lists < 2 || (e_conc && atoi(e_conc) == 0)) return launch_lowres_lists(plan, src, dst, opcodes, ls, img_lo, img_hi);
+    if (n_lists < 2) return launch_lowres_lists(plan, src, dst, opcodes, ls, img_lo, img_hi);
     // the fork / join of one call must not interleave with another host thread's on the same plan
     std::lock_guard<std::mutex> lock(plan->lr_mutex);
     if (plan->lr_ev_fork == nullptr) {  // created as a whole or not at all
@@ -2122,7 +1987,6 @@ int launch_lowres(const rod_plan* plan, const uint8_t* src, uint8_t* dst, const 
     for (auto& s : plan->lr_streams) ROD_CUDA(cudaStreamWaitEvent(s, plan->lr_ev_fork, 0));
     ls.s[1] = plan->lr_streams[0]; ls.s[2] = plan->lr_streams[1];
     ls.n = 3;
-    ls.lanes = env_int("ROD_LR_LANES", 0, 1, 0) != 0;
     int rc = launch_lowres_lists(plan, src, dst, opcodes, ls, img_lo, img_hi);
     for (int i = 0; i < 2; ++i) {  // the join is executed on every path
         cudaError_t e = cudaEventRecord(plan->lr_ev_join[i], plan->lr_streams[i]);

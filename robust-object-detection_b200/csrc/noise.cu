@@ -13,7 +13,6 @@
 // HBM-bound elementwise op: one work item is a span of <= 16384 consecutive bytes; each
 // thread moves 16 bytes per step with 128-bit loads/stores that bypass L1.  Spans whose
 // addresses are not 16-byte aligned (pitched rows of strided views) take a byte path.
-#include <stdlib.h>
 
 #include <mutex>
 #include <vector>
@@ -396,14 +395,13 @@ int gauss_table_for(int device, float sigma, const int32_t** out) {
 int launch_noise(const rod_plan* plan, int mode, const uint8_t* src, uint8_t* dst, const float* noise,
                  float* field_out, float sigma, uint64_t seed, uint64_t first_image, uint32_t offset,
                  const uint8_t* opcodes, int my_op, cudaStream_t stream, int img_lo, int img_hi, int generator) {
-    if (plan->n_noise_tiles == 0) return ROD_OK;
+    const auto [tiles, n_tiles] = plan->noise_tiles.range(img_lo, img_hi);
+    if (n_tiles == 0) return ROD_OK;
     if (generator < 0) generator = plan->gauss_generator;
     NoiseParams p;
     p.images = plan->d_images;
-    const int t_lo = plan->noise_tile_start[img_lo], t_hi = plan->noise_tile_start[img_hi];
-    if (t_hi <= t_lo) return ROD_OK;
-    p.tiles = plan->d_noise_tiles + t_lo;
-    p.n_tiles = t_hi - t_lo;
+    p.tiles = tiles;
+    p.n_tiles = n_tiles;
     p.src = src; p.dst = dst; p.noise = noise; p.field_out = field_out;
     p.sigma = sigma;
     p.key0 = (uint32_t)seed; p.key1 = (uint32_t)(seed >> 32);
@@ -414,9 +412,7 @@ int launch_noise(const rod_plan* plan, int mode, const uint8_t* src, uint8_t* ds
     p.table = nullptr;
     p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
     ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), stream));
-    int per_sm = 4;  // CTAs per SM the grid is sized for: 4 are resident, a longer queue evens out the tail (knob: ROD_NOISE_CTAS)
-    const char* e_ctas = getenv("ROD_NOISE_CTAS");
-    if (e_ctas && atoi(e_ctas) >= 1 && atoi(e_ctas) <= 64) per_sm = atoi(e_ctas);
+    const int per_sm = 4;  // CTAs per SM the grid is sized for: 4 are resident, a longer queue evens out the tail
     if ((mode == NOISE_PHILOX || mode == NOISE_FIELD) && (generator == ROD_GAUSS_AUTO || generator == ROD_GAUSS_TABLE_PHILOX7) &&
         sigma >= ROD_GAUSS_TABLE_MIN_SIGMA && sigma <= ROD_GAUSS_TABLE_MAX_SIGMA) {
         int rc = gauss_table_for(plan->device, sigma, &p.table);
@@ -425,11 +421,9 @@ int launch_noise(const rod_plan* plan, int mode, const uint8_t* src, uint8_t* ds
         // Work item = a whole span when there are plenty (>= 8 per resident warp), else a half / quarter span so that
         // small batches still spread over all warps.  Measured on a B200, sigma 15, 1360x765: 256 images 5.10 TB/s with
         // whole spans vs 4.87 with quarter spans (fewer atomic -> tile -> image dependency chains); 16 images 2.74 TB/s
-        // with quarter spans vs 2.38 with whole spans.  Knob: ROD_NOISE_PIECE_SHIFT = 0 | 1 | 2.
+        // with quarter spans vs 2.38 with whole spans.
         const long warps = 32L * plan->sm_count;
         p.piece_shift = p.n_tiles >= 8 * warps ? 0 : (2L * p.n_tiles >= 8 * warps ? 1 : 2);
-        const char* e_ps = getenv("ROD_NOISE_PIECE_SHIFT");
-        if (e_ps && atoi(e_ps) >= 0 && atoi(e_ps) <= 2) p.piece_shift = atoi(e_ps);
         const int ctas = grid_for(plan, ((p.n_tiles << p.piece_shift) + 31) / 32, 1);
 #define ROD_TAB_LAUNCH(M, TH, UN, R)                                                                                       \
     do {                                                                                                                   \

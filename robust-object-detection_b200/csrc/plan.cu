@@ -1,6 +1,4 @@
 // plan.cu -- batch plans: descriptor upload, tile lists, resize tables (host side of librod_b200.so).
-#include <stdlib.h>
-
 #include <map>
 #include <new>
 
@@ -49,10 +47,17 @@ static int upload(const rod_plan* plan, const std::vector<T>& v, T** dptr) {
     return ROD_OK;
 }
 
-static void tile_starts(const std::vector<Tile>& tl, int n_images, std::vector<int>& st) {
-    st.assign(n_images + 1, (int)tl.size());
-    for (int t = (int)tl.size() - 1; t >= 0; --t) st[tl[t].img] = t;
-    for (int i = n_images - 1; i >= 0; --i) st[i] = std::min(st[i], st[i + 1]);
+// Replaces the device copy of `list` with `tiles` (in image order) and indexes it by image.
+static int upload_tiles(const rod_plan* plan, const std::vector<Tile>& tiles, TileList* list) {
+    plan_free(plan, list->d);
+    list->d = nullptr;
+    list->n = 0;
+    list->start.assign(plan->n_images + 1, (int)tiles.size());
+    for (int t = (int)tiles.size() - 1; t >= 0; --t) list->start[tiles[t].img] = t;
+    for (int i = plan->n_images - 1; i >= 0; --i) list->start[i] = std::min(list->start[i], list->start[i + 1]);
+    const int rc = upload(plan, tiles, &list->d);
+    if (rc == ROD_OK) list->n = (int)tiles.size();
+    return rc;
 }
 
 int ensure_lowres_tables(rod_plan* plan, double factor) {
@@ -63,20 +68,13 @@ int ensure_lowres_tables(rod_plan* plan, double factor) {
     bool all_identity = true;
     int max_rows = 1, max_cols = 1, max_src_rows = 1;
     size_t x2_smem = 0;
-    // tuning knobs (benchmarks only): CTA size, forced strip height, shared-memory budget per CTA
-    const char* e_thr = getenv("ROD_X2_THREADS");
-    const char* e_rows = getenv("ROD_X2_STRIP");
-    const int x2_threads = (e_thr && atoi(e_thr) == 256) ? 256 : 128;
-    const int x2_force_rows = e_rows ? atoi(e_rows) : 0;
-    const size_t x2_max_smem = (x2_threads == 128) ? 54 * 1024 : 100 * 1024;
-    plan->lowres_x2_threads = x2_threads;
     for (size_t s = 0; s < plan->shapes.size(); ++s) {
         const int h = plan->shapes[s].h, w = plan->shapes[s].w;
         if (!build_lowres_shape(h, w, factor, kMaxAreaTaps, blob, &shapes[s])) return ROD_ERR_UNSUPPORTED;
         DevShape& sh = shapes[s];
         if (sh.lin_identity) continue;
         all_identity = false;
-        x2_smem = std::max(x2_smem, choose_strip_rows(&sh, blob.data(), x2_max_smem, x2_threads, x2_force_rows));
+        x2_smem = std::max(x2_smem, choose_strip_rows(&sh, blob.data()));
         if (sh.strip_rows > 0) continue;
         int rows, cols, srows;
         lowres_tile_footprint(sh, blob.data(), kLowresTH, kLowresTWB, &rows, &cols, &srows);
@@ -87,8 +85,6 @@ int ensure_lowres_tables(rod_plan* plan, double factor) {
     if (blob.empty()) blob.push_back(0);
     // warp-marching kernel: one tile = (band of rows, strip of 30 chunks); band height from the amount of work
     // (aim at >= 4 tiles per resident warp; 16 warps per SM)
-    const char* e_march = getenv("ROD_X2_MARCH");
-    const bool march = !(e_march && atoi(e_march) == 0);
     auto march_image = [&](int i) {
         const DevImage& im = plan->h_images[i];
         return shapes[im.shape_id].x2w != 0 && (im.src_pitch & 3) == 0 && (im.src_off & 3) == 0;
@@ -99,20 +95,17 @@ int ensure_lowres_tables(rod_plan* plan, double factor) {
     };
     auto n_strips = [&](int w) { return ((w + 7) / 8 + 29) / 30; };
     int band_rows = 0;
-    if (march) {
+    {
         long long strip_rows = 0;
         for (int i = 0; i < plan->n_images; ++i)
             if (march_image(i)) strip_rows += (long long)plan->h_images[i].h * n_strips(plan->h_images[i].w);
-        const char* e_band = getenv("ROD_X2_BAND");
-        band_rows = e_band ? atoi(e_band) : (int)(strip_rows / (80LL * plan->sm_count));  // ~5 tiles per resident warp (measured best on B200)
+        band_rows = (int)(strip_rows / (80LL * plan->sm_count));  // ~5 tiles per resident warp (measured best on B200)
         band_rows = std::max(24, std::min(256, band_rows & ~7));  // <= kX2wMaxBandRows (per-warp shared tables)
     }
     // packed-integer kernel (exact 2x in both axes): additionally needs 4-byte aligned destination rows (32 / 64-bit stores)
-    const char* e_packed = getenv("ROD_X2_PACKED");
-    const bool packed_on = !(e_packed && atoi(e_packed) == 0);
     auto packed_image = [&](int i) {
         const DevImage& im = plan->h_images[i];
-        return packed_on && shapes[im.shape_id].x2p != 0 && (im.dst_pitch & 3) == 0 && (im.dst_off & 3) == 0;
+        return shapes[im.shape_id].x2p != 0 && (im.dst_pitch & 3) == 0 && (im.dst_off & 3) == 0;
     };
     auto packed_class = [&](int i) {  // 0: 16-byte copy units, 1: 8-byte, 2: 4-byte
         const DevImage& im = plan->h_images[i];
@@ -123,113 +116,59 @@ int ensure_lowres_tables(rod_plan* plan, double factor) {
     };
     // float-tap staged kernel (exact-2x width, general y taps): 4-byte aligned destination rows, and a y scale small
     // enough for its ring of 8 source rows
-    const char* e_x2f = getenv("ROD_X2_FLOAT_STAGED");
-    const bool x2f_on = !(e_x2f && atoi(e_x2f) == 0);
     auto float_image = [&](int i) {
         const DevImage& im = plan->h_images[i];
         const DevShape& sh = shapes[im.shape_id];
-        return x2f_on && sh.x2w != 0 && sh.area_mode == AREA_GENERAL && sh.ay_packed && (im.dst_pitch & 3) == 0 &&
+        return sh.x2w != 0 && sh.area_mode == AREA_GENERAL && sh.ay_packed && (im.dst_pitch & 3) == 0 &&
                (im.dst_off & 3) == 0 && (sh.h <= 8 || 4LL * sh.h <= 9LL * sh.nh);
     };
-    const char* e_x2h = getenv("ROD_X2_REGULAR");
-    const bool x2h_on = !(e_x2h && atoi(e_x2h) == 0);
-    auto regular_image = [&](int i) { return x2h_on && float_image(i) && shapes[plan->h_images[i].shape_id].x2h != 0; };
+    auto regular_image = [&](int i) { return float_image(i) && shapes[plan->h_images[i].shape_id].x2h != 0; };
     // odd-width staged kernel: regular 3-tap / one-slip shapes whose y scale fits the ring of 8 source rows
-    const char* e_x2g = getenv("ROD_X2_ODD_STAGED");
-    const bool x2g_on = !(e_x2g && atoi(e_x2g) == 0);
     auto odd_image = [&](int i) {
         const DevShape& sh = shapes[plan->h_images[i].shape_id];
-        return x2g_on && sh.x2g != 0 && (sh.h <= 8 || 4LL * sh.h <= 9LL * sh.nh);
+        return sh.x2g != 0 && (sh.h <= 8 || 4LL * sh.h <= 9LL * sh.nh);
     };
-    const char* e_x2i = getenv("ROD_X2_ODD_REGULAR");
-    const bool x2i_on = !(e_x2i && atoi(e_x2i) == 0);
-    std::vector<Tile> gen_tiles, x2_tiles, x2w_tiles, x2w4_tiles, x2_rest_tiles, x2p_tiles[3], x2f_tiles[3], x2h_tiles[3], x2g_tiles, x2i_tiles[2], gen_all;
+    std::vector<Tile> lists[LR_NUM_LISTS], gen_all;
     build_strip_tiles(plan->h_images, shapes, false, kLowresTH, kLowresTWB, gen_all);
     for (const Tile& t : gen_all)
-        if (!odd_image(t.img)) gen_tiles.push_back(t);
-    build_strip_tiles(plan->h_images, shapes, true, kLowresTH, kLowresTWB, x2_tiles);
+        if (!odd_image(t.img)) lists[LR_GENERIC].push_back(t);
+    build_strip_tiles(plan->h_images, shapes, true, kLowresTH, kLowresTWB, lists[LR_X2_STRIP]);
     int band_rows_odd = 0;
     {
         long long strip_rows = 0;
         for (int i = 0; i < plan->n_images; ++i)
             if (odd_image(i)) strip_rows += (long long)plan->h_images[i].h * n_strips(plan->h_images[i].w);
-        const char* e_band = getenv("ROD_X2G_BAND_DIV");  // tiles per SM the band height aims at (benchmark knob)
-        const long long div = e_band && atoi(e_band) >= 4 ? atoi(e_band) : 60;
-        band_rows_odd = std::max(24, std::min(256, (int)(strip_rows / (div * plan->sm_count)) & ~7));
+        band_rows_odd = std::max(24, std::min(256, (int)(strip_rows / (60LL * plan->sm_count)) & ~7));  // ~60 tiles per SM
     }
     for (int i = 0; i < plan->n_images; ++i) {
         const DevShape& sh = shapes[plan->h_images[i].shape_id];
         if (odd_image(i)) {
-            std::vector<Tile>& list = (x2i_on && sh.x2i != 0) ? x2i_tiles[sh.x2i - 1] : x2g_tiles;
+            std::vector<Tile>& list = lists[sh.x2i != 0 ? LR_X2I_CARRY + sh.x2i - 1 : LR_X2G];
             for (int y = 0; y < plan->h_images[i].h; y += band_rows_odd)
                 for (int st = 0; st < n_strips(plan->h_images[i].w); ++st)
                     list.push_back(Tile{i, y, std::min(plan->h_images[i].h, y + band_rows_odd), st});
             continue;
         }
         if (sh.strip_rows <= 0) continue;
-        if (march && march_image(i)) {
+        if (march_image(i)) {
+            const int l = packed_image(i) ? LR_X2P16 + packed_class(i) : regular_image(i) ? LR_X2H16 + packed_class(i)
+                          : float_image(i) ? LR_X2F16 + packed_class(i) : al8_image(i) ? LR_X2W8 : LR_X2W4;
             for (int y = 0; y < plan->h_images[i].h; y += band_rows)
                 for (int st = 0; st < n_strips(plan->h_images[i].w); ++st)
-                    (packed_image(i) ? x2p_tiles[packed_class(i)] : regular_image(i) ? x2h_tiles[packed_class(i)] : float_image(i) ? x2f_tiles[packed_class(i)] : al8_image(i) ? x2w_tiles : x2w4_tiles).push_back(Tile{i, y, std::min(plan->h_images[i].h, y + band_rows), st});
+                    lists[l].push_back(Tile{i, y, std::min(plan->h_images[i].h, y + band_rows), st});
         } else {
-            for (int y = 0; y < plan->h_images[i].h; y += sh.strip_rows) x2_rest_tiles.push_back(Tile{i, y, 0, 0});
+            for (int y = 0; y < plan->h_images[i].h; y += sh.strip_rows) lists[LR_X2_REST].push_back(Tile{i, y, 0, 0});
         }
     }
-    void* old[] = {plan->d_shapes, plan->d_tab, plan->d_lowres_tiles, plan->d_lowres_x2_tiles, plan->d_lowres_x2w_tiles, plan->d_lowres_x2w4_tiles,
-                   plan->d_lowres_x2_rest_tiles, plan->d_lowres_x2p_tiles[0], plan->d_lowres_x2p_tiles[1], plan->d_lowres_x2p_tiles[2],
-                   plan->d_lowres_x2f_tiles[0], plan->d_lowres_x2f_tiles[1], plan->d_lowres_x2f_tiles[2], plan->d_lowres_x2g_tiles,
-                   plan->d_lowres_x2h_tiles[0], plan->d_lowres_x2h_tiles[1], plan->d_lowres_x2h_tiles[2],
-                   plan->d_lowres_x2i_tiles[0], plan->d_lowres_x2i_tiles[1]};
-    for (void* q : old) plan_free(plan, q);
-    plan->d_shapes = nullptr; plan->d_tab = nullptr; plan->d_lowres_tiles = nullptr; plan->d_lowres_x2_tiles = nullptr;
-    plan->d_lowres_x2w_tiles = nullptr; plan->d_lowres_x2w4_tiles = nullptr; plan->d_lowres_x2_rest_tiles = nullptr;
+    plan->lowres_factor = -1.0;  // tables are incomplete until every upload below succeeded
+    plan_free(plan, plan->d_shapes);
+    plan_free(plan, plan->d_tab);
+    plan->d_shapes = nullptr;
+    plan->d_tab = nullptr;
     int rc = upload(plan, shapes, &plan->d_shapes);
-    plan->d_lowres_x2g_tiles = nullptr;
-    if (rc == ROD_OK) rc = upload(plan, x2g_tiles, &plan->d_lowres_x2g_tiles);
-    for (int u = 0; u < 2; ++u) {
-        plan->d_lowres_x2i_tiles[u] = nullptr;
-        if (rc == ROD_OK) rc = upload(plan, x2i_tiles[u], &plan->d_lowres_x2i_tiles[u]);
-    }
-    for (int u = 0; u < 3; ++u) {
-        plan->d_lowres_x2p_tiles[u] = nullptr;
-        if (rc == ROD_OK) rc = upload(plan, x2p_tiles[u], &plan->d_lowres_x2p_tiles[u]);
-        plan->d_lowres_x2f_tiles[u] = nullptr;
-        if (rc == ROD_OK) rc = upload(plan, x2f_tiles[u], &plan->d_lowres_x2f_tiles[u]);
-        plan->d_lowres_x2h_tiles[u] = nullptr;
-        if (rc == ROD_OK) rc = upload(plan, x2h_tiles[u], &plan->d_lowres_x2h_tiles[u]);
-    }
     if (rc == ROD_OK) rc = upload(plan, blob, &plan->d_tab);
-    if (rc == ROD_OK) rc = upload(plan, gen_tiles, &plan->d_lowres_tiles);
-    if (rc == ROD_OK) rc = upload(plan, x2_tiles, &plan->d_lowres_x2_tiles);
-    if (rc == ROD_OK) rc = upload(plan, x2w_tiles, &plan->d_lowres_x2w_tiles);
-    if (rc == ROD_OK) rc = upload(plan, x2w4_tiles, &plan->d_lowres_x2w4_tiles);
-    if (rc == ROD_OK) rc = upload(plan, x2_rest_tiles, &plan->d_lowres_x2_rest_tiles);
+    for (int l = 0; l < LR_NUM_LISTS && rc == ROD_OK; ++l) rc = upload_tiles(plan, lists[l], &plan->lowres[l]);
     if (rc != ROD_OK) return rc;
-    plan->n_lowres_tiles = (int)gen_tiles.size();
-    plan->n_lowres_x2_tiles = (int)x2_tiles.size();
-    plan->n_lowres_x2w_tiles = (int)x2w_tiles.size();
-    plan->n_lowres_x2w4_tiles = (int)x2w4_tiles.size();
-    plan->n_lowres_x2g_tiles = (int)x2g_tiles.size();
-    tile_starts(x2g_tiles, plan->n_images, plan->lowres_x2g_tile_start);
-    for (int u = 0; u < 2; ++u) {
-        plan->n_lowres_x2i_tiles[u] = (int)x2i_tiles[u].size();
-        tile_starts(x2i_tiles[u], plan->n_images, plan->lowres_x2i_tile_start[u]);
-    }
-    for (int u = 0; u < 3; ++u) {
-        plan->n_lowres_x2p_tiles[u] = (int)x2p_tiles[u].size();
-        tile_starts(x2p_tiles[u], plan->n_images, plan->lowres_x2p_tile_start[u]);
-        plan->n_lowres_x2f_tiles[u] = (int)x2f_tiles[u].size();
-        tile_starts(x2f_tiles[u], plan->n_images, plan->lowres_x2f_tile_start[u]);
-        plan->n_lowres_x2h_tiles[u] = (int)x2h_tiles[u].size();
-        tile_starts(x2h_tiles[u], plan->n_images, plan->lowres_x2h_tile_start[u]);
-    }
-    tile_starts(x2w4_tiles, plan->n_images, plan->lowres_x2w4_tile_start);
-    plan->n_lowres_x2_rest_tiles = (int)x2_rest_tiles.size();
-    tile_starts(gen_tiles, plan->n_images, plan->lowres_tile_start);
-    tile_starts(x2_tiles, plan->n_images, plan->lowres_x2_tile_start);
-    tile_starts(x2w_tiles, plan->n_images, plan->lowres_x2w_tile_start);
-    tile_starts(x2_rest_tiles, plan->n_images, plan->lowres_x2_rest_tile_start);
-    plan->lowres_x2w_band_rows = band_rows;
     plan->lowres_x2_smem = x2_smem;
     plan->lowres_factor = factor;
     plan->lowres_all_identity = all_identity;
@@ -293,14 +232,12 @@ int ensure_letterbox_tables(rod_plan* plan, int out_h, int out_w) {
             for (int x = 0; x < out_w; x += kLbTW) tiles.push_back(Tile{i, y, x, 0});
     if (plan->d_lb) { plan_free(plan, plan->d_lb); plan->d_lb = nullptr; }
     if (plan->d_lb_tab) { plan_free(plan, plan->d_lb_tab); plan->d_lb_tab = nullptr; }
-    if (plan->d_lb_tiles) { plan_free(plan, plan->d_lb_tiles); plan->d_lb_tiles = nullptr; }
     int rc = upload(plan, lbs, &plan->d_lb);
     if (rc != ROD_OK) return rc;
     rc = upload(plan, blob, &plan->d_lb_tab);
     if (rc != ROD_OK) return rc;
-    rc = upload(plan, tiles, &plan->d_lb_tiles);
+    rc = upload_tiles(plan, tiles, &plan->lb_tiles);
     if (rc != ROD_OK) return rc;
-    plan->n_lb_tiles = (int)tiles.size();
     plan->lb_all_linear = true;
     for (const DevLetterbox& g : lbs)
         if (g.identity || g.area2) plan->lb_all_linear = false;
@@ -363,13 +300,6 @@ extern "C" int rod_plan_create(const rod_image_desc* images, int n_images, rod_p
     std::vector<Tile> nt, bt;
     build_noise_tiles(plan->h_images, kNoiseSpan, nt);
     build_blur_tiles(plan->h_images, kBlurRowsPerTile, bt);
-    auto starts = [&](const std::vector<Tile>& tl, std::vector<int>& st) {
-        st.assign(n_images + 1, (int)tl.size());
-        for (int t = (int)tl.size() - 1; t >= 0; --t) st[tl[t].img] = t;
-        for (int i = n_images - 1; i >= 0; --i) st[i] = std::min(st[i], st[i + 1]);
-    };
-    starts(nt, plan->noise_tile_start);
-    starts(bt, plan->blur_tile_start);
     for (int i = 1; i < n_images; ++i) {
         const rod_image_desc& a = images[i - 1];
         const rod_image_desc& b = images[i];
@@ -377,12 +307,10 @@ extern "C" int rod_plan_create(const rod_image_desc* images, int n_images, rod_p
             b.dst_offset < a.dst_offset + (uint64_t)a.height * a.dst_pitch - (a.dst_pitch - 3ull * a.width))
             plan->monotonic = false;
     }
-    plan->n_noise_tiles = (int)nt.size();
-    plan->n_blur_tiles = (int)bt.size();
     if (plan_alloc(plan, (void**)&plan->d_counters, kCounterRing * sizeof(unsigned int)) != cudaSuccess) { rod_plan_destroy(plan); return ROD_ERR_OOM; }
     int rc = upload(plan, plan->h_images, &plan->d_images);
-    if (rc == ROD_OK) rc = upload(plan, nt, &plan->d_noise_tiles);
-    if (rc == ROD_OK) rc = upload(plan, bt, &plan->d_blur_tiles);
+    if (rc == ROD_OK) rc = upload_tiles(plan, nt, &plan->noise_tiles);
+    if (rc == ROD_OK) rc = upload_tiles(plan, bt, &plan->blur_tiles);
     if (rc != ROD_OK) { rod_plan_destroy(plan); return rc; }
     *out_plan = plan;
     return ROD_OK;
@@ -416,13 +344,11 @@ extern "C" int rod_set_blur_kernel(rod_plan* plan, const float* kernel, int k) {
     if (plan->d_f2d_taps) { plan_free(plan, plan->d_f2d_taps); plan->d_f2d_taps = nullptr; }
     int rc = upload(plan, taps, &plan->d_f2d_taps);
     if (rc != ROD_OK) return rc;
-    if (plan->d_f2d_tiles == nullptr) {
+    if (plan->f2d_tiles.d == nullptr) {
         std::vector<Tile> tiles;
         build_grid_tiles(plan->h_images, kF2dTH, kF2dTWB, tiles);
-        rc = upload(plan, tiles, &plan->d_f2d_tiles);
+        rc = upload_tiles(plan, tiles, &plan->f2d_tiles);
         if (rc != ROD_OK) return rc;
-        plan->n_f2d_tiles = (int)tiles.size();
-        tile_starts(tiles, plan->n_images, plan->f2d_tile_start);
     }
     plan->f2d_ntaps = (int)taps.size();
     plan->f2d_k = k;
@@ -437,16 +363,11 @@ extern "C" void rod_plan_destroy(rod_plan* plan) {
     cudaDeviceSynchronize();
     if (plan->d_patch_clean) cudaFree(plan->d_patch_clean);
     if (plan->d_patch_corrupted) cudaFree(plan->d_patch_corrupted);
-    void* ptrs[] = {plan->d_images, plan->d_noise_tiles, plan->d_blur_tiles, plan->d_lowres_tiles, plan->d_lowres_x2_tiles,
-                    plan->d_lowres_x2w_tiles, plan->d_lowres_x2w4_tiles, plan->d_lowres_x2_rest_tiles, plan->d_shapes,
-                    plan->d_lowres_x2p_tiles[0], plan->d_lowres_x2p_tiles[1], plan->d_lowres_x2p_tiles[2],
-                    plan->d_lowres_x2f_tiles[0], plan->d_lowres_x2f_tiles[1], plan->d_lowres_x2f_tiles[2], plan->d_lowres_x2g_tiles,
-                    plan->d_lowres_x2h_tiles[0], plan->d_lowres_x2h_tiles[1], plan->d_lowres_x2h_tiles[2],
-                    plan->d_lowres_x2i_tiles[0], plan->d_lowres_x2i_tiles[1],
-                    plan->d_tab, plan->d_lb, plan->d_lb_tab, plan->d_lb_tiles, plan->d_scratch, plan->d_stage_src,
-                    plan->d_f2d_taps, plan->d_f2d_tiles, plan->d_counters,
-                    plan->d_stage_dst, plan->d_stage_noise, plan->d_stage_ops};
+    void* ptrs[] = {plan->d_images, plan->noise_tiles.d, plan->blur_tiles.d, plan->d_shapes, plan->d_tab, plan->d_lb,
+                    plan->d_lb_tab, plan->lb_tiles.d, plan->d_scratch, plan->d_stage_src, plan->d_f2d_taps,
+                    plan->f2d_tiles.d, plan->d_counters, plan->d_stage_dst, plan->d_stage_noise, plan->d_stage_ops};
     for (void* p : ptrs) plan_free(plan, p);
+    for (const TileList& l : plan->lowres) plan_free(plan, l.d);
     for (cudaStream_t s : plan->streams)
         if (s) cudaStreamDestroy(s);
     for (cudaStream_t s : plan->aux_streams)

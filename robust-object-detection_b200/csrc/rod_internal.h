@@ -4,6 +4,7 @@
 
 #include <atomic>
 #include <mutex>
+#include <utility>
 #include <vector>
 
 #include "../../include/rod_b200.h"
@@ -40,6 +41,32 @@ struct DevLetterbox {
     int32_t lane_group;        // fused kernel: lanes l and l + lane_group would read the same shared-memory bank (0: no such period)
 };
 
+// A tile list on the device, in image order: the tiles of image i are d[start[i], start[i + 1]).
+struct TileList {
+    Tile* d = nullptr;
+    int n = 0;
+    std::vector<int> start;
+    // first tile and tile count of images [lo, hi)
+    std::pair<const Tile*, int> range(int lo, int hi) const {
+        if (n == 0) return {d, 0};
+        return {d + start[lo], start[hi] - start[lo]};
+    }
+};
+
+// The LowRes tile lists, one per kernel and copy unit (lowres.cu launch_lowres_lists)
+enum LowresList {
+    LR_GENERIC,                       // lowres_kernel: shapes that are not exact-2x in x
+    LR_X2_STRIP,                      // lowres_x2_kernel over every exact-2x image (base pointers not 4-byte aligned)
+    LR_X2_REST,                       // lowres_x2_kernel over the exact-2x images no band kernel takes
+    LR_X2W8, LR_X2W4,                 // lowres_x2w_kernel: 8-byte aligned rows and w % 8 == 0 (64-bit loads), the others
+    LR_X2P16, LR_X2P8, LR_X2P4,       // lowres_x2p_kernel (exact 2x in both axes) by copy unit: 16, 8, 4 bytes
+    LR_X2F16, LR_X2F8, LR_X2F4,       // lowres_x2f_kernel (exact-2x width, float y taps)
+    LR_X2H16, LR_X2H8, LR_X2H4,       // lowres_x2h_kernel (... with the regular three-tap y structure)
+    LR_X2G,                           // lowres_x2g_kernel: odd widths at factor 0.5
+    LR_X2I_CARRY, LR_X2I_EVEN,        // lowres_x2i_kernel: odd widths with a regular y axis, odd h / even h
+    LR_NUM_LISTS
+};
+
 }  // namespace rod
 
 struct rod_plan {
@@ -56,47 +83,9 @@ struct rod_plan {
     uint64_t src_min_offset = 0;               // smallest src_offset (start of the span a host upload must cover)
 
     rod::DevImage* d_images = nullptr;
-    rod::Tile* d_noise_tiles = nullptr;
-    rod::Tile* d_blur_tiles = nullptr;
-    rod::Tile* d_lowres_tiles = nullptr;
-    int n_noise_tiles = 0, n_blur_tiles = 0, n_lowres_tiles = 0;
-    // tiles of image i are [start[i], start[i+1]) in each list (lists are in image order)
-    std::vector<int> noise_tile_start, blur_tile_start, lowres_tile_start, lowres_x2_tile_start;
-    rod::Tile* d_lowres_x2_tiles = nullptr;
-    int n_lowres_x2_tiles = 0;
+    rod::TileList noise_tiles, blur_tiles;
+    rod::TileList lowres[rod::LR_NUM_LISTS];  // indexed by rod::LowresList
     size_t lowres_x2_smem = 0;
-    int lowres_x2_threads = 128;  // CTA size of lowres_x2_kernel (ROD_X2_THREADS=128|256)
-    // warp-marching x2 kernel (4-byte aligned rows of eligible exact-2x shapes): band x strip tiles; the strip-kernel
-    // list restricted to the remaining exact-2x images
-    rod::Tile* d_lowres_x2w_tiles = nullptr;    // images whose rows are 8-byte aligned and w % 8 == 0 (64-bit loads)
-    rod::Tile* d_lowres_x2w4_tiles = nullptr;   // the other eligible images (32-bit loads)
-    int n_lowres_x2w4_tiles = 0;
-    std::vector<int> lowres_x2w4_tile_start;
-    rod::Tile* d_lowres_x2_rest_tiles = nullptr;
-    // exact 2x in both axes (packed-integer kernel), same band x strip tiles; three lists by the copy unit the image
-    // allows: [0] 16 bytes (w % 16 == 0, 16-byte aligned rows), [1] 8 bytes (w % 8 == 0, 8-byte aligned rows), [2] 4 bytes
-    rod::Tile* d_lowres_x2p_tiles[3] = {nullptr, nullptr, nullptr};
-    int n_lowres_x2p_tiles[3] = {0, 0, 0};
-    std::vector<int> lowres_x2p_tile_start[3];
-    // exact-2x widths with float y taps (odd heights): lowres_x2f_kernel, same tiles and unit classes
-    rod::Tile* d_lowres_x2f_tiles[3] = {nullptr, nullptr, nullptr};
-    int n_lowres_x2f_tiles[3] = {0, 0, 0};
-    std::vector<int> lowres_x2f_tile_start[3];
-    // ... of those, the shapes with the regular three-tap structure (DevShape::x2h): lowres_x2h_kernel
-    rod::Tile* d_lowres_x2h_tiles[3] = {nullptr, nullptr, nullptr};
-    int n_lowres_x2h_tiles[3] = {0, 0, 0};
-    std::vector<int> lowres_x2h_tile_start[3];
-    // odd widths at factor 0.5: lowres_x2g_kernel (any byte alignment), same band x strip tiles
-    rod::Tile* d_lowres_x2g_tiles = nullptr;
-    int n_lowres_x2g_tiles = 0;
-    std::vector<int> lowres_x2g_tile_start;
-    // ... of those, the shapes with a regular y axis (DevShape::x2i = 1: odd h, [0]; 2: even h, [1]): lowres_x2i_kernel
-    rod::Tile* d_lowres_x2i_tiles[2] = {nullptr, nullptr};
-    int n_lowres_x2i_tiles[2] = {0, 0};
-    std::vector<int> lowres_x2i_tile_start[2];
-    int n_lowres_x2w_tiles = 0, n_lowres_x2_rest_tiles = 0;
-    std::vector<int> lowres_x2w_tile_start, lowres_x2_rest_tile_start;
-    int lowres_x2w_band_rows = 0;
     // ring of work counters for dynamically scheduled kernels, one per launch: launches of one plan may be in flight
     // on several streams / from several host threads, so the slot index is taken atomically and the ring is long
     // enough (4096 launches) that a slot is never reused while its launch is still pending
@@ -119,17 +108,14 @@ struct rod_plan {
     rod::DevLetterbox* d_lb = nullptr;
     uint32_t* d_lb_tab = nullptr;
     bool lb_all_linear = false;  // every shape is a plain INTER_LINEAR letterbox (fused kernel eligible)
-    rod::Tile* d_lb_tiles = nullptr;
-    int n_lb_tiles = 0;
+    rod::TileList lb_tiles;
     uint8_t* d_scratch = nullptr;  // corrupted full-res images for the letterbox path
     uint64_t scratch_bytes = 0;
 
     // general 2-D blur kernel override (rod_set_blur_kernel): non-zero taps in row-major order
     float4* d_f2d_taps = nullptr;
     int f2d_ntaps = 0, f2d_k = 0;
-    rod::Tile* d_f2d_tiles = nullptr;
-    int n_f2d_tiles = 0;
-    std::vector<int> f2d_tile_start;
+    rod::TileList f2d_tiles;
 
     // restoration pairs (rod_restoration_pairs_f32): contiguous-patch plan + two uint8 patch buffers
     rod_plan* inner = nullptr;

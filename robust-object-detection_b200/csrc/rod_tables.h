@@ -242,10 +242,11 @@ inline bool build_lowres_shape(int h, int w, double factor, int max_taps, std::v
 }
 
 // Exact-2x shapes are processed in full-width strips (lowres_x2_kernel).  Pick the strip height that
-// fills the 256-thread CTA best: items = (strip_rows / 8) * ceil(w / 8); fewer apron rows is better too.
+// fills the 128-thread CTA best: items = (strip_rows / 8) * ceil(w / 8); fewer apron rows is better too.
 // Sets sh->strip_rows / strip_half_rows (0 = use the generic tiled kernel) and returns the shared bytes.
-inline size_t choose_strip_rows(DevShape* sh, const uint32_t* blob, size_t max_smem = 100 * 1024, int nthreads = 256,
-                                int force_rows = 0) {
+inline size_t choose_strip_rows(DevShape* sh, const uint32_t* blob) {
+    const size_t max_smem = 54 * 1024;  // 4 CTAs of 128 threads per SM (lowres_x2_kernel)
+    const int nthreads = 128;
     sh->strip_rows = 0;
     sh->strip_half_rows = 0;
     if (!sh->x2 || sh->lin_identity) return 0;
@@ -255,7 +256,6 @@ inline size_t choose_strip_rows(DevShape* sh, const uint32_t* blob, size_t max_s
     double best = -1.0;
     size_t best_smem = 0;
     for (int R = 16; R <= 64; R += 8) {
-        if (force_rows > 0 && R != force_rows) continue;
         int nj = 1;
         for (int y0 = 0; y0 < sh->h; y0 += R) {
             const int y1 = std::min(sh->h, y0 + R) - 1;

@@ -430,11 +430,13 @@ def test_ragged_mixed_resolution_batch(torch_):
 def test_lowres_marching_kernel_alignments(torch_):
     """lowres_x2w_kernel (warp-marching bands x strips): images packed at 4-byte granularity (rows that are not
     8-byte aligned take the 32-bit load path), widths with a two-pixel last chunk, pitched rows, and a source base
-    that is not 4-byte aligned (falls back to the strip kernel)."""
+    that is not 4-byte aligned (falls back to the strip kernel).  Odd heights above 1999 are the only shapes that
+    select lowres_x2f_kernel (w % 4 == 0) and lowres_x2g_kernel (odd w)."""
     from robust_object_detection_b200.batch import CorruptionPlan
     shapes = [(765, 1360), (360, 480), (100, 8), (9, 4), (2, 4), (5, 12), (64, 64), (65, 128), (131, 36), (201, 1400),
               (97, 1916), (540, 960), (33, 2000), (40, 20), (77, 1364), (1080, 1920), (1050, 1400), (41, 44),
-              (98, 1916), (6, 244), (4, 248), (10, 1204), (12, 1448)]   # rows at 4- / 8-byte phases, last strips of one (two-pixel) chunk
+              (98, 1916), (6, 244), (4, 248), (10, 1204), (12, 1448),   # rows at 4- / 8-byte phases, last strips of one (two-pixel) chunk
+              (2001, 1360), (2001, 1361)]
     imgs = [synth(4200 + i, h, w) for i, (h, w) in enumerate(shapes)]
     want = [orc.apply_lowres(im, 0.5) for im in imgs]
     for align in (4, 256):

@@ -18,4 +18,4 @@ out = []
 if "noise" in which: out.append(("noise", t(lambda: plan.noise(src, dst, None, 15.0, seed=1))))
 if "lowres" in which: out.append(("lowres", t(lambda: plan.lowres(src, dst))))
 if "blur" in which: out.append(("blur", t(lambda: plan.blur(src, dst))))
-print(" ".join(f"{k}={v:.0f}" for k, v in out), {k: v for k, v in os.environ.items() if k.startswith("ROD_")})
+print(" ".join(f"{k}={v:.0f}" for k, v in out))

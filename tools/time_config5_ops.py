@@ -24,4 +24,4 @@ for n in (16, 64):
         for _ in range(40): fn()
         e1.record(); torch.cuda.synchronize()
         res[name] = round(e0.elapsed_time(e1) / 40 * 1e3, 1)
-    print(f"config5 n={n} us:", res, {k: v for k, v in os.environ.items() if k.startswith("ROD_")})
+    print(f"config5 n={n} us:", res)
