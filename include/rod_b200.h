@@ -157,6 +157,21 @@ ROD_API int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, const 
                               const float* noise, float sigma, int k, double factor, uint64_t seed,
                               uint64_t first_image_index, uint32_t offset, void* stream);
 
+/* Faster R-CNN loader (augmentations.py:60-74 RandomCorruption inside train_frcnn_augmented.py:61-67's
+ * Compose([RandomCorruption(0.5), ToImage(), ToDtype(float32, scale=True)])) for a batch: opcodes[i] picks the corruption
+ * of image i exactly as rod_corrupt_batch_u8 does (same parameters and checks; Philox noise uses the plan's own generator),
+ * then BGR -> RGB, HWC -> CHW and fl(float(v) * fl(1/255)) per element, torchvision's to_dtype_image arithmetic.
+ * Output layout: `out` is one flat device float32 buffer (256-byte aligned, else ROD_ERR_INVALID_ARG); image i is the
+ * contiguous [3, H_i, W_i] block at float offset rod_plan_chw_offset(plan, i), in plan order, each block starting at a
+ * multiple of 64 floats (256 bytes); rod_plan_chw_offset(plan, n_images) is the buffer's size in floats.  The gaps
+ * between blocks are not written.  Clean images are read from `src` in place; corrupted ones go through the plan's
+ * scratch buffer (the dst descriptors' layout). */
+ROD_API int rod_corrupt_chw_f32(rod_plan* plan, const uint8_t* src, const uint8_t* opcodes, float* out, const float* noise,
+                        float sigma, int k, double factor, uint64_t seed, uint64_t first_image_index, uint32_t offset,
+                        void* stream);
+/* Float offset of image i's block in the output of rod_corrupt_chw_f32 (0 <= i <= n_images; 0 otherwise). */
+ROD_API uint64_t rod_plan_chw_offset(const rod_plan* plan, int i);
+
 /* SURVEY 8f rank 4 -- RestorationDataset.__getitem__ (scripts/train_restoration.py:104-129) for a batch of patches.
  * The plan's source descriptors are the crops (offset + pitch into the device-resident images; one patch size per
  * batch); flips[i] != 0 applies cv2.flip(patch, 1) first; opcodes[i] picks the corruption (1..3; 0 = none).

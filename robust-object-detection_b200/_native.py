@@ -13,7 +13,7 @@ LIB_PATH = os.path.join(_HERE, "librod_b200.so")
 
 ROD_OK, ROD_ERR_INVALID_ARG, ROD_ERR_UNSUPPORTED, ROD_ERR_CUDA, ROD_ERR_NO_DEVICE, ROD_ERR_OOM = range(6)
 OP_NONE, OP_NOISE, OP_BLUR, OP_LOWRES = 0, 1, 2, 3
-LAUNCHES_CORRUPT_BATCH, LAUNCHES_CORRUPT_LETTERBOX = 100, 101
+LAUNCHES_CORRUPT_BATCH, LAUNCHES_CORRUPT_LETTERBOX, LAUNCHES_CORRUPT_CHW = 100, 101, 102
 
 
 class ImageDesc(ctypes.Structure):
@@ -47,6 +47,8 @@ SYMBOLS = {
     "rod_lowres_u8": (_i, [_vp, _vp, _vp, _d, _vp, _vp]),
     "rod_corrupt_batch_u8": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _i, _d, _u64, _u64, _u32, _vp]),
     "rod_corrupt_letterbox_f16": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _f, _i, _d, _u64, _u64, _u32, _vp]),
+    "rod_corrupt_chw_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _i, _d, _u64, _u64, _u32, _vp]),
+    "rod_plan_chw_offset": (_u64, [_vp, _i]),
     "rod_restoration_pairs_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _d, _u64, _u64, _u32, _vp]),
     "rod_resize_linear_u8": (_i, [_vp, _i, _i, ctypes.c_int64, _vp, _i, _i, ctypes.c_int64, _vp]),
     "rod_jpeg_create": (_i, [ctypes.POINTER(ImageDesc), _i, _vp, _u64, ctypes.POINTER(_vp)]),

@@ -225,6 +225,28 @@ class CorruptionPlan:
                                                   float(factor), int(seed), int(first_image_index), int(offset),
                                                   _stream_handle(stream)), "rod_corrupt_letterbox_f16")
 
+    def chw_offsets(self) -> list:
+        """Float offsets of the images' [3,H,W] blocks in the output of corrupt_chw_f32, plus the total size in floats as
+        the last entry (rod_plan_chw_offset: blocks in plan order, each starting at a multiple of 256 bytes)."""
+        if getattr(self, "_chw_offsets", None) is None:
+            self._chw_offsets = [int(N.lib().rod_plan_chw_offset(self._h, i)) for i in range(self.n_images + 1)]
+        return self._chw_offsets
+
+    def chw_views(self, out) -> list:
+        """The [3,H,W] tensors of the images inside a flat output buffer of corrupt_chw_f32."""
+        offs = self.chw_offsets()
+        return [out[o:o + 3 * h * w].view(3, h, w) for o, (h, w) in zip(offs, self.shapes)]
+
+    def corrupt_chw_f32(self, src, opcodes, out, noise=None, sigma: float = NOISE_SIGMA, k: int = BLUR_KERNEL,
+                        factor: float = DOWNSCALE_FACTOR, seed: int = 0, first_image_index: int = 0, offset: int = 0,
+                        stream=None) -> None:
+        """Faster R-CNN loader path (RandomCorruption + ToImage + ToDtype(float32, scale=True)): the corruption of
+        corrupt() for opcodes, then BGR->RGB, HWC->CHW and float(v) * float32(1/255) into `out`, a flat CUDA float32
+        buffer of chw_offsets()[-1] elements (256-byte aligned) laid out by chw_offsets()."""
+        N.check(N.lib().rod_corrupt_chw_f32(self._h, _ptr(src), _ptr(opcodes), _ptr(out), _ptr(noise), float(sigma),
+                                            int(k), float(factor), int(seed), int(first_image_index), int(offset),
+                                            _stream_handle(stream)), "rod_corrupt_chw_f32")
+
     def restoration_pairs(self, src, flips, opcodes, corrupted_out, clean_out, noise=None, sigma: float = NOISE_SIGMA,
                           k: int = BLUR_KERNEL, factor: float = DOWNSCALE_FACTOR, seed: int = 0,
                           first_image_index: int = 0, offset: int = 0, stream=None) -> None:

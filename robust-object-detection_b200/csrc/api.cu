@@ -100,6 +100,17 @@ int run_mixed_ops(rod_plan* plan, int op_lo, const uint8_t* src, uint8_t* dst, c
     return first_rc;
 }
 
+// The plan's scratch: corrupted images at the dst descriptors, read by the letterbox and CHW kernels.
+int ensure_scratch(rod_plan* plan) {
+    if (plan->d_scratch == nullptr || plan->scratch_bytes < plan->dst_extent) {
+        if (plan->d_scratch) cudaFree(plan->d_scratch);
+        plan->d_scratch = nullptr;
+        ROD_CUDA(cudaMalloc((void**)&plan->d_scratch, plan->dst_extent + 64));
+        plan->scratch_bytes = plan->dst_extent;
+    }
+    return ROD_OK;
+}
+
 }  // namespace
 
 extern "C" const char* rod_version(void) { return "rod_b200 0.1.0 (sm_100a)"; }
@@ -140,6 +151,7 @@ extern "C" int rod_plan_launches(const rod_plan* plan, int op) {
         }
         case 100: return 4;  // rod_corrupt_batch_u8: copy + noise + blur + lowres
         case 101: return 4;  // rod_corrupt_letterbox_f16: noise + blur + lowres + letterbox (clean images are read in place)
+        case 102: return 4;  // rod_corrupt_chw_f32: noise + blur + lowres + conversion (clean images are read in place)
         default: return 0;
     }
 }
@@ -233,12 +245,8 @@ extern "C" int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, con
     } generator_scope(plan);
     int rc = ensure_letterbox_tables(plan, out_h, out_w);
     if (rc != ROD_OK) return rc;
-    if (plan->d_scratch == nullptr || plan->scratch_bytes < plan->dst_extent) {
-        if (plan->d_scratch) cudaFree(plan->d_scratch);
-        plan->d_scratch = nullptr;
-        ROD_CUDA(cudaMalloc((void**)&plan->d_scratch, plan->dst_extent + 64));
-        plan->scratch_bytes = plan->dst_extent;
-    }
+    rc = ensure_scratch(plan);
+    if (rc != ROD_OK) return rc;
     // Fused path: noise / blur / clean rows are produced inside the letterbox kernel (no full-resolution round trip);
     // only LowRes images go through the scratch.  Needs plain linear letterboxes, the angle-0 blur and Philox sigma
     // in range.
@@ -264,6 +272,26 @@ extern "C" int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, con
                        offset, (cudaStream_t)stream);
     if (rc != ROD_OK) return rc;
     return launch_letterbox(plan, plan->d_scratch, src, opcodes, out_f16, pad_value, (cudaStream_t)stream);
+}
+
+// train_frcnn_augmented.py:61-67: RandomCorruption(0.5) + ToImage + ToDtype(float32, scale=True) for a batch.
+extern "C" int rod_corrupt_chw_f32(rod_plan* plan, const uint8_t* src, const uint8_t* opcodes, float* out, const float* noise,
+                                   float sigma, int k, double factor, uint64_t seed, uint64_t first_image_index,
+                                   uint32_t offset, void* stream) {
+    if (plan == nullptr || src == nullptr || out == nullptr || opcodes == nullptr) return ROD_ERR_INVALID_ARG;
+    if (((uintptr_t)out & 255) != 0) return ROD_ERR_INVALID_ARG;  // the layout's 256-byte alignment starts at `out`
+    // the checks of rod_corrupt_batch_u8, before anything is launched
+    if (noise == nullptr && sigma > kPhiloxMaxSigma) return ROD_ERR_UNSUPPORTED;
+    if (plan->f2d_ntaps == 0 && !blur_supported(k, 0.0)) return ROD_ERR_UNSUPPORTED;
+    int rc = ensure_lowres_tables(plan, factor);
+    if (rc == ROD_OK) rc = ensure_chw_tables(plan);
+    if (rc == ROD_OK) rc = ensure_scratch(plan);
+    if (rc != ROD_OK) return rc;
+    // corrupted images go to the scratch; clean ones are read from `src` by the conversion itself
+    rc = run_mixed_ops(plan, ROD_OP_NOISE, src, plan->d_scratch, opcodes, noise, sigma, k, factor, seed, first_image_index,
+                       offset, (cudaStream_t)stream);
+    if (rc != ROD_OK) return rc;
+    return launch_chw_f32(plan, src, plan->d_scratch, opcodes, out, (cudaStream_t)stream);
 }
 
 extern "C" int rod_resize_linear_u8(const uint8_t* src, int h, int w, int64_t src_pitch, uint8_t* dst, int nh, int nw,

@@ -246,6 +246,23 @@ int ensure_letterbox_tables(rod_plan* plan, int out_h, int out_w) {
     return ROD_OK;
 }
 
+int ensure_chw_tables(rod_plan* plan) {
+    if (plan->d_chw_off != nullptr) return ROD_OK;
+    std::vector<Tile> tiles;
+    for (int i = 0; i < plan->n_images; ++i)
+        for (int y = 0; y < plan->h_images[i].h; y += kChwBandRows)
+            tiles.push_back(Tile{i, y, std::min(plan->h_images[i].h, y + kChwBandRows), 0});
+    int rc = upload_tiles(plan, tiles, &plan->chw_tiles);
+    uint64_t* off = nullptr;
+    if (rc == ROD_OK) rc = upload(plan, plan->chw_off, &off);
+    if (rc != ROD_OK) {
+        plan_free(plan, off);
+        return rc;
+    }
+    plan->d_chw_off = off;  // set last: it marks the tables complete
+    return ROD_OK;
+}
+
 }  // namespace rod
 
 using namespace rod;
@@ -297,6 +314,11 @@ extern "C" int rod_plan_create(const rod_image_desc* images, int n_images, rod_p
         plan->dst_extent = std::max<uint64_t>(plan->dst_extent, d.dst_offset + (uint64_t)(d.height - 1) * d.dst_pitch + 3ull * d.width);
     }
     plan->payload_bytes = elem;
+    // CHW float32 output layout (include/rod_b200.h rod_plan_chw_offset): blocks of 3*H*W floats rounded up to 64 floats
+    plan->chw_off.resize(n_images + 1);
+    plan->chw_off[0] = 0;
+    for (int i = 0; i < n_images; ++i)
+        plan->chw_off[i + 1] = plan->chw_off[i] + (3ull * images[i].height * images[i].width + 63) / 64 * 64;
     std::vector<Tile> nt, bt;
     build_noise_tiles(plan->h_images, kNoiseSpan, nt);
     build_blur_tiles(plan->h_images, kBlurRowsPerTile, bt);
@@ -365,7 +387,8 @@ extern "C" void rod_plan_destroy(rod_plan* plan) {
     if (plan->d_patch_corrupted) cudaFree(plan->d_patch_corrupted);
     void* ptrs[] = {plan->d_images, plan->noise_tiles.d, plan->blur_tiles.d, plan->d_shapes, plan->d_tab, plan->d_lb,
                     plan->d_lb_tab, plan->lb_tiles.d, plan->d_scratch, plan->d_stage_src, plan->d_f2d_taps,
-                    plan->f2d_tiles.d, plan->d_counters, plan->d_stage_dst, plan->d_stage_noise, plan->d_stage_ops};
+                    plan->f2d_tiles.d, plan->d_counters, plan->d_stage_dst, plan->d_stage_noise, plan->d_stage_ops,
+                    plan->chw_tiles.d, plan->d_chw_off};
     for (void* p : ptrs) plan_free(plan, p);
     for (const TileList& l : plan->lowres) plan_free(plan, l.d);
     for (cudaStream_t s : plan->streams)
@@ -385,3 +408,6 @@ extern "C" void rod_plan_destroy(rod_plan* plan) {
 
 extern "C" int rod_plan_num_images(const rod_plan* plan) { return plan ? plan->n_images : 0; }
 extern "C" uint64_t rod_plan_payload_bytes(const rod_plan* plan) { return plan ? plan->payload_bytes : 0; }
+extern "C" uint64_t rod_plan_chw_offset(const rod_plan* plan, int i) {
+    return (plan != nullptr && i >= 0 && i <= plan->n_images) ? plan->chw_off[i] : 0;
+}

@@ -25,6 +25,7 @@ constexpr int kMaxAreaTaps = 8;
 constexpr int kF2dTH = 16;         // general 2-D filter tile: rows x output bytes
 constexpr int kF2dTWB = 768;
 constexpr int kF2dMaxElems = 130;  // cv::filter2D uses DFT-based convolution from 130 kernel elements on (8U)
+constexpr int kChwBandRows = 8;    // CHW conversion: rows per work item, one per warp
 
 struct HostShape {
     int h, w;
@@ -109,8 +110,14 @@ struct rod_plan {
     uint32_t* d_lb_tab = nullptr;
     bool lb_all_linear = false;  // every shape is a plain INTER_LINEAR letterbox (fused kernel eligible)
     rod::TileList lb_tiles;
-    uint8_t* d_scratch = nullptr;  // corrupted full-res images for the letterbox path
+    uint8_t* d_scratch = nullptr;  // corrupted full-res images for the letterbox and CHW paths
     uint64_t scratch_bytes = 0;
+
+    // float32 CHW output (rod_corrupt_chw_f32): float offset of image i's [3,H,W] block, i = n: the total (rod_plan_create);
+    // its device copy and the row bands are uploaded on first use
+    std::vector<uint64_t> chw_off;
+    uint64_t* d_chw_off = nullptr;
+    rod::TileList chw_tiles;
 
     // general 2-D blur kernel override (rod_set_blur_kernel): non-zero taps in row-major order
     float4* d_f2d_taps = nullptr;
@@ -180,10 +187,13 @@ int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8
                            uint64_t first_image, uint32_t offset, bool lowres_in_kernel, cudaStream_t stream);
 int launch_letterbox(const rod_plan* plan, const uint8_t* img, const uint8_t* src, const uint8_t* opcodes, void* out_f16,
                      int pad_value, cudaStream_t stream);
+int launch_chw_f32(const rod_plan* plan, const uint8_t* src, const uint8_t* scratch, const uint8_t* opcodes, float* out,
+                   cudaStream_t stream);
 
 int gauss_table_for(int device, float sigma, const int32_t** out);  // noise.cu: device copy of the Philox-mode table
 int ensure_lowres_tables(rod_plan* plan, double factor);
 int ensure_letterbox_tables(rod_plan* plan, int out_h, int out_w);
+int ensure_chw_tables(rod_plan* plan);
 
 enum NoiseMode { NOISE_COMPAT = 0, NOISE_PHILOX = 1, NOISE_COPY = 2, NOISE_FIELD = 3 };
 }  // namespace rod

@@ -10,6 +10,7 @@ ops taking CUDA uint8 tensors"; north_star: "a thin PyTorch custom-op / C-ABI la
     rod::lowres                 rod_lowres_u8                      apply_lowres                   :41-45
     rod::corrupt_batch          rod_corrupt_batch_u8               _apply_random_corruption + gate :48-56, :93
     rod::corrupt_letterbox      rod_corrupt_letterbox_f16          hook + Ultralytics LetterBox / Format / /255
+    rod::corrupt_chw            rod_corrupt_chw_f32                RandomCorruption + ToImage + ToDtype(float32, scale=True)
 
 All ops are functional (fresh output tensor, input untouched -- the reference's ownership convention), run on the
 CURRENT CUDA stream of the input's device, have fake (meta) implementations so they trace under torch.compile /
@@ -128,6 +129,30 @@ def corrupt_letterbox(img: torch.Tensor, opcodes: torch.Tensor, out_h: int, out_
     return out
 
 
+def _chw_strides(h: int, w: int):
+    """Strides of the [N,3,H,W] float32 result of rod::corrupt_chw: image blocks start at multiples of 64 floats
+    (include/rod_b200.h rod_plan_chw_offset), so the batch stride is 3*H*W rounded up to 64."""
+    return ((3 * h * w + 63) // 64 * 64, h * w, w, 1)
+
+
+@torch.library.custom_op("rod::corrupt_chw", mutates_args=(), device_types="cuda")
+def corrupt_chw(img: torch.Tensor, opcodes: torch.Tensor, sigma: float, k: int, factor: float, seed: int,
+                first_image_index: int) -> torch.Tensor:
+    """Faster R-CNN loader path: the corruption of rod::corrupt_batch, then BGR->RGB, HWC->CHW and float32 scaling as
+    torchvision's ToDtype(float32, scale=True) -> float32 [N,3,H,W] (batch stride rounded up to 64 floats)."""
+    x, n, h, w = _check(img)
+    if not opcodes.is_cuda or opcodes.dtype != torch.uint8 or opcodes.numel() != n:
+        raise ValueError("opcodes must be a CUDA uint8 tensor with one entry per image")
+    strides = _chw_strides(h, w)
+    out = torch.empty_strided((n, 3, h, w), strides, dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        plan = _plan(n, h, w, x.device)
+        plan.set_blur_kernel(None)
+        plan.corrupt_chw_f32(x, opcodes.contiguous(), out, None, float(sigma), int(k), float(factor), int(seed),
+                             int(first_image_index))
+    return out
+
+
 @noise.register_fake
 def _(img, sigma, seed, first_image_index, field=None):
     return torch.empty_like(img.contiguous())
@@ -152,3 +177,10 @@ def _(img, opcodes, sigma, k, factor, seed, first_image_index):
 def _(img, opcodes, out_h, out_w, pad_value, sigma, k, factor, seed, first_image_index):
     n = 1 if img.dim() == 3 else img.shape[0]
     return img.new_empty((n, 3, out_h, out_w), dtype=torch.float16)
+
+
+@corrupt_chw.register_fake
+def _(img, opcodes, sigma, k, factor, seed, first_image_index):
+    n = 1 if img.dim() == 3 else img.shape[0]
+    h, w = img.shape[-3], img.shape[-2]
+    return img.new_empty_strided((n, 3, h, w), _chw_strides(h, w), dtype=torch.float32)

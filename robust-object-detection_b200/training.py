@@ -382,3 +382,209 @@ class RestorationPairBatcher:
             dec.append((y, x, flip, op))
         self.last_decisions = dec
         return self._pairs(plan, crops.reshape(-1), dec, fields)
+
+
+class DetectionCorruptionBatcher:
+    """Batched device path of the torchvision Faster R-CNN loader (train_frcnn_augmented.py:61-67,131-134): per item
+    `PIL.Image.open(p).convert("RGB")` -> RandomCorruption(p) (augmentations.py:60-74) -> ToImage() ->
+    ToDtype(torch.float32, scale=True), then `.to(device)` in the loop.  Here one call takes a whole batch and returns
+    CUDA float32 [3,H,W] RGB tensors (views into one flat buffer, rod_corrupt_chw_f32):
+
+        batcher = DetectionCorruptionBatcher(p=0.5)               # noise="compat": the reference's tensors, bit for bit
+        images = batcher(paths)                                  # or bytes objects, PIL images, HWC RGB uint8 arrays
+        loader = DataLoader(dataset_without_transforms, batch_size=2, shuffle=True, num_workers=0,
+                            collate_fn=batcher.collate)          # (images, targets) with the images already on the GPU
+
+    Decisions: `random` is consumed as the per-item gate would (skip iff random() > p, then random.choice), for the whole
+    batch first; in compat mode the fields of the noise images are then drawn from NumPy's global legacy stream in image
+    order (np.random.normal(0, 15, (H, W, 3)).astype(float32) for the BGR array: augmentations.legacy_normal_f32).  The two
+    streams are independent, so this equals the reference's per-item interleaving.  noise="philox" generates the field in
+    the kernel instead (the plan's generator, keyed by (seed, running image index)).  The drawn op-codes are left in
+    .last_ops.
+
+    Files: JPEGs the device decoder takes are decoded on the GPU (PIL and cv2.imdecode give the same pixels for them);
+    every other file -- EXIF-rotated (PIL does not apply the orientation; OpenCV would), progressive, CMYK, PNG, corrupt
+    entropy data -- is read with `Image.open(...).convert("RGB")` like the reference's dataset, so PIL's own errors and
+    settings (ImageFile.LOAD_TRUNCATED_IMAGES) apply.  The batcher uses CUDA in the calling process: with a DataLoader, keep
+    num_workers=0 (the reference's setting) so that collate runs in the main process.
+    """
+
+    def __init__(self, p: float = 0.5, noise: str = "compat", seed: int = 0, io_threads: int = 16,
+                 max_cached_plans: int = 16):
+        import torch
+        from concurrent.futures import ThreadPoolExecutor
+        if noise not in ("compat", "philox"):
+            raise ValueError("noise must be 'compat' or 'philox'")
+        self._torch = torch
+        self.p, self.noise, self.seed = float(p), noise, int(seed)
+        self._plans: dict = {}
+        self._max_plans = max_cached_plans
+        self._io_threads = max(1, int(io_threads))
+        self._pool = ThreadPoolExecutor(self._io_threads)
+        self._copy_stream = torch.cuda.Stream()
+        self._slots: List[dict] = [{}, {}]
+        self.images_seen = 0
+        self.last_ops: Optional[np.ndarray] = None
+
+    # ------------------------------------------------------------------ internals
+    def _plan(self, shapes) -> CorruptionPlan:
+        key = tuple(shapes)
+        plan = self._plans.get(key)
+        if plan is None:
+            if len(self._plans) >= self._max_plans:
+                self._plans.pop(next(iter(self._plans)))
+            plan = self._plans[key] = CorruptionPlan.ragged(shapes)
+        return plan
+
+    @staticmethod
+    def _read_pil(data) -> np.ndarray:
+        import io
+        from PIL import Image
+        with Image.open(io.BytesIO(data)) as im:
+            return np.asarray(im.convert("RGB"))
+
+    @classmethod
+    def _load(cls, item):
+        """I/O thread: (file bytes, (h, w)) for a JPEG the device decoder takes, else (HWC RGB uint8 array, (h, w))."""
+        if isinstance(item, np.ndarray):
+            if item.dtype != np.uint8 or item.ndim != 3 or item.shape[2] != 3:
+                raise ValueError("expected HWC RGB uint8 arrays")
+            return item, (int(item.shape[0]), int(item.shape[1]))
+        if not isinstance(item, (bytes, bytearray, memoryview)) and hasattr(item, "convert"):  # a PIL image
+            arr = np.asarray(item if item.mode == "RGB" else item.convert("RGB"))
+            return arr, (int(arr.shape[0]), int(arr.shape[1]))
+        from .jpeg import probe
+        data = item if isinstance(item, (bytes, bytearray, memoryview)) else open(item, "rb").read()
+        shape = probe(data)
+        if shape is not None:
+            return data, shape
+        arr = cls._read_pil(data)
+        return arr, (int(arr.shape[0]), int(arr.shape[1]))
+
+    def _stage(self, slot: dict, items: Sequence, futs) -> None:
+        """Read / decode / pack one batch into the slot's buffers on the copy stream and draw its decisions."""
+        torch = self._torch
+        from .augmentations import NOISE_SIGMA, legacy_normal_f32
+        from .jpeg import JpegDecoder
+        loaded = [f.result() for f in futs]
+        shapes = [sh for _, sh in loaded]
+        plan = self._plan(shapes)
+        n = len(items)
+        elems = [3 * h * w for h, w in shapes]
+        elem_base = np.concatenate([[0], np.cumsum(elems)]).astype(np.int64)
+        grow = False
+        for name, dtype, size in (("src", torch.uint8, plan.src_bytes), ("noise", torch.float32, int(elem_base[-1])),
+                                  ("ops", torch.uint8, max(n, 64))):
+            if slot.get(name + "_cap", 0) < size:
+                cap = max(size, 2 * slot.get(name + "_cap", 0))
+                slot[name + "_host"] = torch.empty(cap, dtype=dtype).pin_memory()
+                slot[name + "_dev"] = torch.empty(cap, dtype=dtype, device="cuda")
+                slot[name + "_cap"] = cap
+                grow = True
+        if grow:  # a fresh block's previous use may still be pending on the compute stream
+            self._copy_stream.wait_stream(torch.cuda.current_stream())
+        ev = slot.get("free")
+        if ev is not None:
+            ev.synchronize()  # the compute that last read this slot's buffers has finished
+        dev, hbuf = slot["src_dev"], slot["src_host"].numpy()
+        offs = plan.src_offsets
+        host_idx = [i for i, (d, _) in enumerate(loaded) if isinstance(d, np.ndarray)]
+        enc = [i for i, (d, _) in enumerate(loaded) if not isinstance(d, np.ndarray)]
+        with torch.cuda.stream(self._copy_stream):
+            if enc:
+                dec = JpegDecoder([loaded[i][0] for i in enc], [offs[i] for i in enc], host_threads=self._io_threads)
+                dec.decode(dev, stream=self._copy_stream)
+                for i, st in zip(enc, dec.status(stream=self._copy_stream)):
+                    if st != 0:  # not decodable here after all, or corrupt entropy data: PIL's reading is the reference's
+                        arr = self._read_pil(loaded[i][0])
+                        if (int(arr.shape[0]), int(arr.shape[1])) != shapes[i]:
+                            raise IOError("image size differs between the file header and its decoded pixels")
+                        loaded[i] = (arr, shapes[i])
+                        host_idx.append(i)
+                host_idx.sort()
+
+            def pack(i):  # RGB -> BGR into the pinned buffer (NumPy releases the GIL for the copy)
+                (h, w), off = shapes[i], offs[i]
+                hbuf[off:off + 3 * h * w].reshape(h, w, 3)[...] = loaded[i][0][:, :, ::-1]
+
+            list(self._pool.map(pack, host_idx))
+            # one copy per run of consecutive host-sourced images
+            k = 0
+            while k < len(host_idx):
+                j = k
+                while j + 1 < len(host_idx) and host_idx[j + 1] == host_idx[j] + 1:
+                    j += 1
+                lo = offs[host_idx[k]]
+                hi = offs[host_idx[j]] + elems[host_idx[j]]
+                dev[lo:hi].copy_(slot["src_host"][lo:hi], non_blocking=True)
+                k = j + 1
+            ops = draw_decisions(n, gate="pil", p=self.p)
+            noise = None
+            if self.noise == "compat" and (ops == 1).any():
+                nh, nd = slot["noise_host"], slot["noise_dev"]
+                for i in np.flatnonzero(ops == 1):  # only the noise images' spans are drawn and uploaded
+                    lo, hi = int(elem_base[i]), int(elem_base[i + 1])
+                    legacy_normal_f32(NOISE_SIGMA, shapes[i] + (3,), out=nh.numpy()[lo:hi])
+                    nd[lo:hi].copy_(nh[lo:hi], non_blocking=True)
+                noise = nd
+            slot["ops_host"][:n] = torch.from_numpy(ops)
+            slot["ops_dev"][:n].copy_(slot["ops_host"][:n], non_blocking=True)
+            ready = torch.cuda.Event()
+            ready.record(self._copy_stream)
+        slot.update(plan=plan, n=n, ready=ready, ops=ops, noise=noise, first_index=self.images_seen)
+        self.images_seen += n
+
+    def _compute(self, slot: dict) -> List:
+        torch = self._torch
+        from .augmentations import NOISE_SIGMA
+        cur = torch.cuda.current_stream()
+        cur.wait_event(slot["ready"])
+        plan = slot["plan"]
+        out = torch.empty(plan.chw_offsets()[-1], dtype=torch.float32, device="cuda")
+        plan.corrupt_chw_f32(slot["src_dev"], slot["ops_dev"], out, noise=slot["noise"], sigma=float(NOISE_SIGMA),
+                             seed=self.seed, first_image_index=slot["first_index"])
+        free = torch.cuda.Event()
+        free.record(cur)
+        slot["free"] = free
+        self.last_ops = slot["ops"]
+        return plan.chw_views(out)
+
+    def _submit(self, items):
+        return [self._pool.submit(self._load, it) for it in items]
+
+    # ------------------------------------------------------------------ public
+    def __call__(self, items: Sequence) -> List:
+        """One batch -> list of CUDA float32 [3,H,W] RGB tensors in [0, 1] (the drawn op-codes in .last_ops)."""
+        items = list(items)
+        slot = self._slots[0]
+        self._stage(slot, items, self._submit(items))
+        return self._compute(slot)
+
+    def run(self, batches: Iterable[Sequence]) -> Iterator[List]:
+        """Pipelined: while batch i is corrupted and converted on the current stream, batch i+1 is read, packed and
+        uploaded on a copy stream."""
+        it = iter(batches)
+        try:
+            cur = list(next(it))
+        except StopIteration:
+            return
+        k = 0
+        self._stage(self._slots[0], cur, self._submit(cur))
+        while True:
+            out = self._compute(self._slots[k & 1])  # enqueued first: the GPU works while the next batch is staged
+            try:
+                nxt = list(next(it))
+            except StopIteration:
+                nxt = None
+            if nxt is not None:
+                self._stage(self._slots[(k + 1) & 1], nxt, self._submit(nxt))
+            yield out
+            if nxt is None:
+                return
+            k += 1
+
+    def collate(self, batch: Sequence[Tuple[object, object]]):
+        """collate_fn for DataLoader(num_workers=0) over a dataset of (PIL image, target) built without transforms:
+        returns (tuple of CUDA float32 [3,H,W] tensors, tuple of targets) like the reference's tuple(zip(*batch))."""
+        images, targets = zip(*batch)
+        return tuple(self(list(images))), tuple(targets)
