@@ -248,10 +248,10 @@ extern "C" int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, con
     rc = ensure_scratch(plan);
     if (rc != ROD_OK) return rc;
     // Fused path: noise / blur / clean rows are produced inside the letterbox kernel (no full-resolution round trip);
-    // only LowRes images go through the scratch.  Needs plain linear letterboxes, the angle-0 blur and Philox sigma
-    // in range.
-    const bool fused = plan->lb_all_linear && plan->f2d_ntaps == 0 && blur_supported(k, 0.0) && k >= 3 &&
-                       (noise != nullptr || sigma <= kPhiloxMaxSigma);
+    // only LowRes images go through the scratch.  Needs an even output width (two columns per lane, half2 stores), plain
+    // linear letterboxes, the angle-0 blur and Philox sigma in range.
+    const bool fused = (out_w & 1) == 0 && plan->lb_all_linear && plan->f2d_ntaps == 0 && blur_supported(k, 0.0) &&
+                       k >= 3 && (noise != nullptr || sigma <= kPhiloxMaxSigma);
     if (fused) {
         rc = ensure_lowres_tables(plan, factor);
         if (rc != ROD_OK) return rc;

@@ -4,10 +4,9 @@
 // Not part of /root/reference (it lives in Ultralytics 8.3.x, which the reference's
 // train_*_augmented.py scripts call through model.train(...)); the resize arithmetic is the same
 // 8-bit fixed-point INTER_LINEAR of SURVEY 8a/a5, the rest is pad(114) + channel swap +
-// half(float(u8) / 255.f).  One thread produces two horizontally adjacent output pixels
-// (3 channels each) and writes one half2 per colour plane.
+// half(float(u8) / 255.f).  In letterbox_kernel one thread produces one output pixel and writes
+// it as three scalar halves, one per colour plane.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "rod_internal.h"
 
@@ -145,9 +144,7 @@ struct FusedLbParams {
     const DevShape* shapes;  // lowres tables (plan->d_shapes / d_tab), used when lowres_in_kernel
     const uint32_t* ltab;
     int lowres_in_kernel;    // 1: LowRes rows are produced in shared memory too (every LowRes-able shape is exact-2x)
-    unsigned int* counter;   // zeroed before the launch: next tile to hand out
     int buf_bytes;           // bytes of one row buffer (16-byte multiple)
-    int xtab_bytes;          // bytes of the per-CTA x table (16-byte multiple)
 };
 
 constexpr int kFusedLeft = 64;  // bytes in front of pixel 0 in every row buffer (halo of up to 15 pixels + window)
@@ -326,144 +323,18 @@ __device__ __forceinline__ void load6_smem(const uint8_t* buf, int o, uint32_t& 
     hi = __funnelshift_r(w1, w2, sh);
 }
 
-template <int NW>  // warps per CTA = output rows per tile
-__global__ void __launch_bounds__(32 * NW, 16 / NW) fused_letterbox_kernel(FusedLbParams p) {
-    extern __shared__ __align__(16) uint8_t smem[];
-    __half* lut = reinterpret_cast<__half*>(smem);  // 256 x half(v / 255)
-    for (int v = threadIdx.x; v < 256; v += 32 * NW) lut[v] = __float2half_rn(__fdiv_rn((float)v, 255.0f));
-    __syncthreads();
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // per-CTA copy of the x tables of the current shape: {3 * s0 (byte offset of the left tap), a0 | a1 << 16, right-border
-    // flag} per output column, read through the short scoreboard
-    uint2* xtab = reinterpret_cast<uint2*>(smem + 512);
-    int cached_shape = -1;
-    // three identical row buffers per warp: [kFusedLeft | row | 64]
-    uint8_t* X0 = smem + 512 + (size_t)p.xtab_bytes + (size_t)warp * (3 * p.buf_bytes) + kFusedLeft;
-    uint8_t* X1 = X0 + p.buf_bytes;
-    uint8_t* X2 = X1 + p.buf_bytes;
-    const size_t plane = (size_t)p.out_h * p.out_w;
-    const __half padh = lut[p.pad];
-    const int groups = (p.out_h + NW - 1) / NW;
-    // tiles (NW output rows of one image) are handed out dynamically: their cost differs by an order of magnitude
-    // (padding rows, clean rows, noise / blur / LowRes rows)
-    int* s_tile = reinterpret_cast<int*>(smem + 512 + p.xtab_bytes - 16);
-    for (;;) {
-        __syncthreads();
-        if (threadIdx.x == 0) *s_tile = (int)atomicAdd(p.counter, 1u);
-        __syncthreads();
-        const int ti = *s_tile;
-        if (ti >= p.n_images * groups) break;
-        const int img = ti / groups;
-        const int Y = (ti - img * groups) * NW + warp;
-        const DevImage im = p.images[img];
-        const DevLetterbox g = p.lb[im.shape_id];
-        if (im.shape_id != cached_shape) {  // CTA-uniform: every warp walks the same tile sequence
-            __syncthreads();
-            const int32_t* lx_s0 = reinterpret_cast<const int32_t*>(p.tab + g.lx_s0);
-            for (int X = threadIdx.x; X < p.out_w; X += 32 * NW) {
-                const int cx = X - g.left;
-                uint2 e = make_uint2(0xFFFFFFFFu, 0u);  // padding column
-                if (cx >= 0 && cx < g.new_w) {
-                    const int s0 = lx_s0[cx];
-                    e = make_uint2((uint32_t)(3 * s0) | ((s0 + 1 > g.w - 1) ? 0x80000000u : 0u), p.tab[g.lx_a + cx]);
-                }
-                xtab[X] = e;
-            }
-            cached_shape = im.shape_id;
-            __syncthreads();
-        }
-        if (Y >= p.out_h) continue;
-        __half* orow = p.out + (size_t)img * 3 * plane + (size_t)Y * p.out_w;
-        const int cy = Y - g.top;
-        if (cy < 0 || cy >= g.new_h) {
-            for (int X = lane; X < p.out_w; X += 32) { orow[X] = padh; orow[plane + X] = padh; orow[2 * plane + X] = padh; }
-            continue;
-        }
-        const int op = p.opcodes[img];
-        const bool lowres_here = (op == ROD_OP_LOWRES) && p.lowres_in_kernel != 0 && p.shapes[im.shape_id].lin_identity == 0;
-        const bool pre = (op == ROD_OP_LOWRES) && p.lowres_in_kernel == 0;
-        const uint8_t* base = pre ? p.scratch + im.dst_off : p.src + im.src_off;
-        const int64_t pitch = pre ? im.dst_pitch : im.src_pitch;
-        const uint32_t ys = p.tab[g.ly_s + cy], yb = p.tab[g.ly_b + cy];
-        const int r0 = (int)(ys & 0xFFFFu), r1 = (int)(ys >> 16);
-        const int n = 3 * im.w;
-        const bool two = (r1 != r0);
-        const bool blur = (op == ROD_OP_BLUR);
-        if (lowres_here) {
-            // rows r0, r1 of lowres(image): the (at most three) low-res rows they blend live two at a time in X2
-            const DevShape sh = p.shapes[im.shape_id];
-            const int p_pitch = (3 * sh.nw + 24 + 15) & ~15;
-            const uint32_t ya = p.ltab[sh.ly_s + r0];
-            const int a0 = (int)(ya & 0xFFFFu), a1 = (int)(ya >> 16);
-            fused_lowres_prow(im, sh, p.ltab, base, a0, X2 + (a0 & 1) * p_pitch, lane);
-            if (a1 != a0) fused_lowres_prow(im, sh, p.ltab, base, a1, X2 + (a1 & 1) * p_pitch, lane);
-            __syncwarp();
-            fused_lowres_fullrow(im, sh, p.ltab, r0, X2, p_pitch, X0, lane);
-            __syncwarp();
-            if (two) {
-                const uint32_t yb2 = p.ltab[sh.ly_s + r1];
-                const int b0 = (int)(yb2 & 0xFFFFu), b1 = (int)(yb2 >> 16);
-                if (b0 != a0 && b0 != a1) fused_lowres_prow(im, sh, p.ltab, base, b0, X2 + (b0 & 1) * p_pitch, lane);
-                if (b1 != a0 && b1 != a1 && b1 != b0) fused_lowres_prow(im, sh, p.ltab, base, b1, X2 + (b1 & 1) * p_pitch, lane);
-                __syncwarp();
-                fused_lowres_fullrow(im, sh, p.ltab, r1, X2, p_pitch, X1, lane);
-            }
-        } else {
-        // both source rows are requested before anything waits (blur filters out of place: X1 -> X0, X2 -> X1)
-        fused_stage_row(base + (int64_t)r0 * pitch, n, blur ? X1 : X0, lane);
-        if (two) fused_stage_row(base + (int64_t)r1 * pitch, n, blur ? X2 : X1, lane);
-        asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
-        __syncwarp();
-        if (op == ROD_OP_NOISE) {
-            fused_noise_row(p, im, img, r0, X0, lane);
-            if (two) fused_noise_row(p, im, img, r1, X1, lane);
-        } else if (blur) {
-            fused_blur_row(p, im, X1, X0, lane);
-            __syncwarp();
-            if (two) fused_blur_row(p, im, X2, X1, lane);
-        }
-        }
-        const uint8_t* bufA = X0;
-        const uint8_t* rowB = two ? X1 : X0;
-        __syncwarp();
-#pragma unroll 2
-        for (int X = lane; X < p.out_w; X += 32) {
-            const uint2 xe = xtab[X];
-            __half h0 = padh, h1 = padh, h2 = padh;
-            if (xe.x != 0xFFFFFFFFu) {
-                const int o3 = (int)(xe.x & 0x7FFFFFFFu);
-                const uint32_t a = xe.y;
-                uint32_t lo0, hi0, lo1, hi1;
-                load6_smem(bufA, o3, lo0, hi0);
-                load6_smem(rowB, o3, lo1, hi1);
-                if (xe.x & 0x80000000u) {  // right border: both taps are the last pixel
-                    hi0 = __byte_perm(lo0, 0u, 0x4421); lo0 = __byte_perm(lo0, 0u, 0x0210);
-                    hi1 = __byte_perm(lo1, 0u, 0x4421); lo1 = __byte_perm(lo1, 0u, 0x0210);
-                }
-                const uint32_t g0[3] = {__byte_perm(lo0, hi0, 0x4430), __byte_perm(lo0, hi0, 0x4441), __byte_perm(lo0, hi0, 0x4452)};
-                const uint32_t g1[3] = {__byte_perm(lo1, hi1, 0x4430), __byte_perm(lo1, hi1, 0x4441), __byte_perm(lo1, hi1, 0x4452)};
-                uint32_t v[3];
-#pragma unroll
-                for (int c = 0; c < 3; ++c) v[c] = linear_v(dot2_lo(a, g0[c], 0u) >> 4, dot2_lo(a, g1[c], 0u) >> 4, yb);
-                h2 = lut[v[0]]; h1 = lut[v[1]]; h0 = lut[v[2]];  // BGR -> RGB
-            }
-            orow[X] = h0; orow[plane + X] = h1; orow[2 * plane + X] = h2;
-        }
-        __syncwarp();  // the row buffers are rewritten by this warp's next row
-    }
-}
-
 // =====================================================================================
-// Version 2 of the fused training path (even out_w): the same row producers, but
-//   * every WARP works on single output rows on its own (no block barrier, no per-CTA table).  Rows are ordered by op class
-//     (noise, LowRes, blur, clean), centre-out and image-minor, and dealt round-robin to the resident warps: the expensive
-//     rows of all images run first, spread evenly, and the cheap padding rows fill the tail;
+// The fused kernel.  It needs an even out_w (rod_corrupt_letterbox_f16 sends odd widths to the unfused path):
+//   * every WARP works on single output rows on its own (no block barrier).  Rows are ordered by op class (noise, LowRes,
+//     blur, clean), centre-out and image-minor, and dealt round-robin to the resident warps: the expensive rows of all
+//     images run first, spread evenly, and the cheap padding rows fill the tail;
 //   * the resampling loop makes two adjacent output columns per lane and step: x taps from a per-shape table in global
 //     memory (one 16-byte load through L1), the horizontal stage as dp2a onto the 2^23 float grid, the vertical stage as the
-//     three round-toward-zero FMAs of the resize kernels, half(v / 255) as one more FMA (== the 256-entry table of
-//     version 1 for every byte value) and a packed half2 conversion; three 4-byte stores per step;
+//     three round-toward-zero FMAs of the resize kernels, half(v / 255) as one more FMA and a packed half2 conversion;
+//     three 4-byte stores per step (~50 instructions per output column);
 //   * padding rows leave as 16-byte stores.
-// Version 1 spent 55 % of its instructions in the resampling loop (~95 per output column; here ~50).
+// half(fl(v * fl(1/255))) must equal the 256-entry half(float(v) / 255.f) table of letterbox_kernel for every byte value
+// v (it does, checked exhaustively): the unfused fallback has to produce the same bytes.
 // =====================================================================================
 __device__ __forceinline__ void fused_column(const uint8_t* bufA, const uint8_t* rowB, uint32_t o3, uint32_t a, const X2Row& rc,
                                              float c255, float nc255, float out[3]) {
@@ -653,34 +524,20 @@ int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8
     p.keys = philox_round_keys(p.key0, p.key1);
     p.k = k;
     p.buf_bytes = kFusedLeft + ((3 * plan->max_w + 15) & ~15) + 128;  // also holds two low-res rows (3 * max_w / 2 + 39 each)
-    p.xtab_bytes = ((p.out_w * 8 + 15) & ~15) + 16;  // + the broadcast slot of the dynamic tile index
-    // 4 rows per tile: more, smaller tiles balance the expensive noise / blur / LowRes rows (measured 6 % faster than 8 at
-    // batch 64, equal at batch 16)
+    // 4 warps per CTA: smaller CTAs balance the expensive noise / blur / LowRes rows (measured 6 % faster than 8 at batch 64,
+    // equal at batch 16).  Measured on a B200 (1360x765 sources, seed-42 mix): batch 64 152 us, batch 16 43.5 us.
+    // (Tried and dropped: keeping the NEXT row's source rows in flight during the resampling loop -- four row buffers per
+    // warp, 12 warps per SM: 171 us at batch 64.  The loop is bound by its shared-memory reads, not by the source-row
+    // latency: at scale 2.125 the six-byte windows of every fifth column pair fall into the same bank.)
     constexpr int nw = 4;
-    // version 2 (row per warp, two columns per lane) whenever out_w is even.  Measured on a B200 (1360x765 sources, seed-42
-    // mix): batch 64 152 us (version 1: 161 us), batch 16 43.5 us (43.1 us).  Knob ROD_FUSED_V2 = 0 forces version 1.
-    // (Tried and dropped: a version 3 that keeps the NEXT row's source rows in flight during the resampling loop -- four row
-    // buffers per warp, 12 warps per SM: 171 us at batch 64.  The loop is bound by its shared-memory reads, not by the
-    // source-row latency: at scale 2.125 the six-byte windows of every fifth column pair fall into the same bank.)
-    const char* e_v2 = getenv("ROD_FUSED_V2");
-    const bool v2 = (p.out_w & 1) == 0 && !(e_v2 && atoi(e_v2) == 0);
-    const size_t smem = v2 ? (size_t)(2 * kFusedMaxSorted + 32) + (size_t)nw * (size_t)(3 * p.buf_bytes) : 512 + (size_t)p.xtab_bytes + (size_t)nw * (size_t)(3 * p.buf_bytes);
+    const size_t smem = (size_t)(2 * kFusedMaxSorted + 32) + (size_t)nw * (size_t)(3 * p.buf_bytes);
     if (smem > 227 * 1024) return ROD_ERR_UNSUPPORTED;
     int per_sm = (int)((227 * 1024) / (smem + 1024));
     per_sm = per_sm < 1 ? 1 : per_sm;
-    p.counter = nullptr;
-    if (v2) {   // one output row per warp, dealt round-robin (no work counter: one launch, nothing else on the stream)
-        const int ctas = (plan->n_images * p.out_h + nw - 1) / nw;
-        ROD_CUDA(cudaFuncSetAttribute(fused_letterbox2_kernel<nw>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        fused_letterbox2_kernel<nw><<<grid_for(plan, ctas, per_sm), 32 * nw, smem, stream>>>(p);
-        ROD_CUDA(cudaGetLastError());
-        return ROD_OK;
-    }
-    p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
-    ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), stream));
-    const int tiles = plan->n_images * ((p.out_h + nw - 1) / nw);
-    ROD_CUDA(cudaFuncSetAttribute(fused_letterbox_kernel<nw>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fused_letterbox_kernel<nw><<<grid_for(plan, tiles, per_sm), 32 * nw, smem, stream>>>(p);
+    // one output row per warp, dealt round-robin (no work counter: one launch, nothing else on the stream)
+    const int ctas = (plan->n_images * p.out_h + nw - 1) / nw;
+    ROD_CUDA(cudaFuncSetAttribute(fused_letterbox2_kernel<nw>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fused_letterbox2_kernel<nw><<<grid_for(plan, ctas, per_sm), 32 * nw, smem, stream>>>(p);
     ROD_CUDA(cudaGetLastError());
     return ROD_OK;
 }

@@ -830,9 +830,9 @@ def test_full_size_config4_testset_by_replication_and_sharding(torch_):
             assert torch_.equal(sdst[:sp.dst_offsets[-1]], full[op][b0:b0 + sp.dst_offsets[-1]]), (rank, op)
 
 
-@pytest.mark.parametrize("fused_version", ["1", "2"])
-def test_letterbox_fused_training_path(torch_, monkeypatch, fused_version):
-    monkeypatch.setenv("ROD_FUSED_V2", "0" if fused_version == "1" else "1")   # 1: block-per-four-rows kernel, 2: row-per-warp kernel (default)
+@pytest.mark.parametrize("ow", [640, 639])
+def test_letterbox_fused_training_path(torch_, ow):
+    # the (640, 640) source is an identity letterbox at 640 x 640 and 639 is odd: both widths take the unfused path
     from robust_object_detection_b200.batch import CorruptionPlan
     shapes = [(765, 1360)] * 5 + [(720, 1280), (360, 480), (640, 640), (1079, 1917)]
     plan = CorruptionPlan.ragged(shapes)
@@ -840,20 +840,20 @@ def test_letterbox_fused_training_path(torch_, monkeypatch, fused_version):
     src = torch_.from_numpy(plan.pack(imgs)).cuda()
     ops_host = np.array([0, 2, 3, 2, 0, 3, 2, 0, 3], dtype=np.uint8)
     ops = torch_.from_numpy(ops_host).cuda()
-    out = torch_.empty((len(shapes), 3, 640, 640), dtype=torch_.float16, device="cuda")
-    plan.corrupt_letterbox(src, ops, out, 640, 640, 114, seed=1)
+    out = torch_.empty((len(shapes), 3, 640, ow), dtype=torch_.float16, device="cuda")
+    plan.corrupt_letterbox(src, ops, out, 640, ow, 114, seed=1)
     got = out.cpu().numpy()
     for i, img in enumerate(imgs):
-        want = orc.letterbox_norm_f16(orc.apply_op(img, int(ops_host[i])), 640, 640, 114)
+        want = orc.letterbox_norm_f16(orc.apply_op(img, int(ops_host[i])), 640, ow, 114)
         assert np.array_equal(got[i], want), (i, shapes[i])
 
 
-@pytest.mark.parametrize("fused_version", ["1", "2"])
-def test_fused_letterbox_kernel_paths(torch_, monkeypatch, fused_version):
-    monkeypatch.setenv("ROD_FUSED_V2", "0" if fused_version == "1" else "1")   # 1: block-per-four-rows kernel, 2: row-per-warp kernel (default)
-    """fused_letterbox_kernel (every shape a plain linear letterbox): 16-byte-aligned rows (cp.async staging), odd widths
+@pytest.mark.parametrize("ow", [320, 319])
+def test_fused_letterbox_kernel_paths(torch_, ow):
+    """fused_letterbox2_kernel (every shape a plain linear letterbox): 16-byte-aligned rows (cp.async staging), odd widths
     (32-bit / byte staging, Philox groups straddling rows), supplied noise field, another blur size, and a pitched
-    source; all against the oracle, bit-exact except Philox noise (statistical mode)."""
+    source; all against the oracle, bit-exact except Philox noise (statistical mode).  An odd output width runs the same
+    cases on the unfused path."""
     from robust_object_detection_b200.batch import CorruptionPlan
     shapes = [(765, 1360), (765, 1360), (540, 960), (333, 517), (401, 1001), (1079, 1917), (360, 480), (765, 1360)]
     ops_host = np.array([1, 2, 3, 2, 1, 0, 1, 0], dtype=np.uint8)
@@ -861,28 +861,28 @@ def test_fused_letterbox_kernel_paths(torch_, monkeypatch, fused_version):
     plan = CorruptionPlan.ragged(shapes)
     src = torch_.from_numpy(plan.pack(imgs)).cuda()
     ops = torch_.from_numpy(ops_host).cuda()
-    out = torch_.empty((len(shapes), 3, 320, 320), dtype=torch_.float16, device="cuda")
+    out = torch_.empty((len(shapes), 3, 320, ow), dtype=torch_.float16, device="cuda")
     # (a) compat noise (supplied field), k = 9
     np.random.seed(33)
     fields = [orc.draw_noise_field(im.shape, 15) for im in imgs]
     nz = torch_.from_numpy(np.concatenate([f.reshape(-1) for f in fields])).cuda()
-    plan.corrupt_letterbox(src, ops, out, 320, 320, 114, noise=nz)
+    plan.corrupt_letterbox(src, ops, out, 320, ow, 114, noise=nz)
     got = out.cpu().numpy()
     for i, img in enumerate(imgs):
         op = int(ops_host[i])
         cor = orc.add_noise_field(img, fields[i]) if op == 1 else orc.apply_op(img, op)
-        assert np.array_equal(got[i], orc.letterbox_norm_f16(cor, 320, 320, 114)), (i, shapes[i], op)
+        assert np.array_equal(got[i], orc.letterbox_norm_f16(cor, 320, ow, 114)), (i, shapes[i], op)
     # (b) Philox noise keyed by a global index offset, blur k = 5
-    plan.corrupt_letterbox(src, ops, out, 320, 320, 114, k=5, seed=77, first_image_index=1000)
+    plan.corrupt_letterbox(src, ops, out, 320, ow, 114, k=5, seed=77, first_image_index=1000)
     got = out.cpu().numpy()
     for i, img in enumerate(imgs):
         op = int(ops_host[i])
         if op == 1:
-            want = orc.letterbox_norm_f16(orc.add_philox_noise(img, orc.philox_noise_field(img.size, 15.0, 77, 1000 + i, generator="boxmuller")), 320, 320, 114)
+            want = orc.letterbox_norm_f16(orc.add_philox_noise(img, orc.philox_noise_field(img.size, 15.0, 77, 1000 + i, generator="boxmuller")), 320, ow, 114)
             assert np.mean(got[i] != want) < 2e-3, (i, shapes[i])
         else:
             cor = orc.apply_motion_blur(img, 5, 0) if op == 2 else orc.apply_op(img, op)
-            assert np.array_equal(got[i], orc.letterbox_norm_f16(cor, 320, 320, 114)), (i, shapes[i], op)
+            assert np.array_equal(got[i], orc.letterbox_norm_f16(cor, 320, ow, 114)), (i, shapes[i], op)
     # (c) pitched source rows
     sp = [3 * w + 12 for h, w in shapes]
     so = np.concatenate([[0], np.cumsum([(h * q + 255) // 256 * 256 for (h, w), q in zip(shapes, sp)])])
@@ -892,18 +892,18 @@ def test_fused_letterbox_kernel_paths(torch_, monkeypatch, fused_version):
         h, w, _ = img.shape
         hsrc[o:o + h * q].reshape(h, q)[:, :3 * w] = img.reshape(h, 3 * w)
     ops2 = torch_.from_numpy(np.array([2, 0, 3, 2, 0, 2, 3, 0], dtype=np.uint8)).cuda()
-    planp.corrupt_letterbox(torch_.from_numpy(hsrc).cuda(), ops2, out, 320, 320, 114)
+    planp.corrupt_letterbox(torch_.from_numpy(hsrc).cuda(), ops2, out, 320, ow, 114)
     got = out.cpu().numpy()
     for i, img in enumerate(imgs):
-        want = orc.letterbox_norm_f16(orc.apply_op(img, int(ops2[i].item())), 320, 320, 114)
+        want = orc.letterbox_norm_f16(orc.apply_op(img, int(ops2[i].item())), 320, ow, 114)
         assert np.array_equal(got[i], want), (i, shapes[i])
 
 
-@pytest.mark.parametrize("fused_version", ["1", "2"])
-def test_fused_letterbox_lowres_in_kernel(torch_, monkeypatch, fused_version):
-    monkeypatch.setenv("ROD_FUSED_V2", "0" if fused_version == "1" else "1")   # 1: block-per-four-rows kernel, 2: row-per-warp kernel (default)
-    """Every shape exact-2x (w % 4 == 0): the LowRes rows are produced inside fused_letterbox_kernel too (no scratch);
-    odd and even heights, a width with a two-pixel last chunk, several output sizes."""
+@pytest.mark.parametrize("oh, ow", [(640, 640), (320, 416), (96, 96), (96, 97)])
+def test_fused_letterbox_lowres_in_kernel(torch_, oh, ow):
+    """Every shape exact-2x (w % 4 == 0): the LowRes rows are produced inside fused_letterbox2_kernel too (no scratch);
+    odd and even heights, a width with a two-pixel last chunk, several output sizes; an odd output width takes the
+    unfused path."""
     from robust_object_detection_b200.batch import CorruptionPlan
     shapes = [(765, 1360), (540, 960), (360, 480), (1080, 1920), (1050, 1400), (97, 1916), (131, 36), (765, 1360)]
     ops_host = np.array([3, 3, 3, 3, 3, 3, 3, 2], dtype=np.uint8)
@@ -912,12 +912,11 @@ def test_fused_letterbox_lowres_in_kernel(torch_, monkeypatch, fused_version):
     src = torch_.from_numpy(plan.pack(imgs)).cuda()
     ops = torch_.from_numpy(ops_host).cuda()
     want_cor = [orc.apply_op(im, int(o)) for im, o in zip(imgs, ops_host)]
-    for oh, ow in ((640, 640), (320, 416), (96, 96)):
-        out = torch_.empty((len(shapes), 3, oh, ow), dtype=torch_.float16, device="cuda")
-        plan.corrupt_letterbox(src, ops, out, oh, ow, 114)
-        got = out.cpu().numpy()
-        for i in range(len(shapes)):
-            assert np.array_equal(got[i], orc.letterbox_norm_f16(want_cor[i], oh, ow, 114)), (i, shapes[i], oh, ow)
+    out = torch_.empty((len(shapes), 3, oh, ow), dtype=torch_.float16, device="cuda")
+    plan.corrupt_letterbox(src, ops, out, oh, ow, 114)
+    got = out.cpu().numpy()
+    for i in range(len(shapes)):
+        assert np.array_equal(got[i], orc.letterbox_norm_f16(want_cor[i], oh, ow, 114)), (i, shapes[i], oh, ow)
 
 
 def test_apply_host_chunked_pipeline(torch_):
