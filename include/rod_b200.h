@@ -114,13 +114,25 @@ ROD_API int rod_noise_prewarm(int device, float sigma);
 /* The 256 entries of that table (int32, host pointer): for tests and for restating the stream. */
 ROD_API int rod_gauss_table_i32(float sigma, int32_t* out256);
 
-/* The HOST side of compat mode: the field `np.random.normal(0, sigma, shape).astype(np.float32)` of augmentations.py:31,
- * regenerated bit for bit from NumPy's legacy generator state (MT19937 + polar Gaussian) with the per-pair work spread
- * over `threads` host threads (0 = all).  key[624], *pos, *has_gauss, *cached are np.random.get_state()[1:5] on entry
- * and the state NumPy itself would have after the call on return (feed them to np.random.set_state), so later draws
- * continue on the same stream.  Pure host code (no GPU work): the reference's own bottleneck, 104 of 137 ms per frame. */
+/* The HOST generator of compat mode: the field `np.random.normal(0, sigma, shape).astype(np.float32)` of
+ * augmentations.py:31, regenerated bit for bit from NumPy's legacy generator state (MT19937 + polar Gaussian) with the
+ * per-pair work spread over `threads` host threads (0 = all).  key[624], *pos, *has_gauss, *cached are
+ * np.random.get_state()[1:5] on entry and the state NumPy itself would have after the call on return (feed them to
+ * np.random.set_state), so later draws continue on the same stream.  Pure host code (no GPU work).  It is the reference
+ * the device generator below is tested against, and the field source of the host-buffer paths (rod_apply_host). */
 ROD_API int rod_numpy_legacy_normal_f32(uint32_t* key, int32_t* pos, int32_t* has_gauss, double* cached, double sigma,
                                 uint64_t n, float* out, int threads);
+/* The same stream drawn on the GPU (csrc/legacy_rng.cu): the values go into n_seg device segments in order, segment s
+ * getting seg_counts[s] consecutive floats at out + seg_offsets[s] (segments sorted and disjoint, else
+ * ROD_ERR_INVALID_ARG; floats between them are not written), so the fields of several images are one draw.  The state
+ * arguments are those of rod_numpy_legacy_normal_f32; sigma must be finite and >= 0.  Returns once the state after the
+ * call is known: one host wait on `stream` per round (one round unless the call exceeds 256 x 128 blocks of 624 words,
+ * about 2.6 fields of 1360x765x3).  The few values whose float32 could depend on the last ulps of the device log() are
+ * recomputed on the host with libm log() and written by a kernel queued on `stream`; *host_fixups (may be NULL) gets
+ * their number.  A total count of 0 changes no state. */
+ROD_API int rod_numpy_legacy_normal_f32_device(uint32_t* key, int32_t* pos, int32_t* has_gauss, double* cached,
+                                double sigma, const uint64_t* seg_offsets, const uint64_t* seg_counts, int n_seg,
+                                float* out, int* host_fixups, void* stream);
 
 /* a2+a3: apply_motion_blur(img, k, angle_deg) (augmentations.py:21-38) for angle_deg == 0:
  * horizontal k-tap box, BORDER_REFLECT_101, out = (2S + k) / (2k).  k odd, 1 <= k <= 31;

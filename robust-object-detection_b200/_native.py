@@ -44,6 +44,9 @@ SYMBOLS = {
     "rod_gauss_table_i32": (_i, [ctypes.c_float, ctypes.POINTER(ctypes.c_int32)]),
     "rod_numpy_legacy_normal_f32": (_i, [_vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32),
                                          ctypes.POINTER(ctypes.c_double), _d, _u64, _vp, _i]),
+    "rod_numpy_legacy_normal_f32_device": (_i, [_vp, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32),
+                                                ctypes.POINTER(ctypes.c_double), _d, _vp, _vp, _i, _vp,
+                                                ctypes.POINTER(_i), _vp]),
     "rod_lowres_u8": (_i, [_vp, _vp, _vp, _d, _vp, _vp]),
     "rod_corrupt_batch_u8": (_i, [_vp, _vp, _vp, _vp, _vp, _f, _i, _d, _u64, _u64, _u32, _vp]),
     "rod_corrupt_letterbox_f16": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _f, _i, _d, _u64, _u64, _u32, _vp]),

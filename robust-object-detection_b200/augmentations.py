@@ -164,26 +164,76 @@ def _pinned_field(n: int) -> np.ndarray:
     return buf
 
 
+def _legacy_state(sigma: float):
+    """NumPy's global legacy state as (key, pos, has_gauss, cached) for the native generators, or None when the draw must
+    be NumPy's own: a state that is not MT19937, or a sigma that is negative (NumPy raises) or NaN."""
+    import ctypes
+    state = np.random.get_state(legacy=True)
+    if state[0] != "MT19937" or not (float(sigma) >= 0.0):
+        return None
+    return (np.array(state[1], dtype=np.uint32, copy=True), ctypes.c_int32(int(state[2])), ctypes.c_int32(int(state[3])),
+            ctypes.c_double(float(state[4])))
+
+
+def _set_legacy_state(st) -> None:
+    key, pos, has, cached = st
+    np.random.set_state(("MT19937", key, pos.value, has.value, cached.value))
+
+
 def legacy_normal_f32(sigma: float, shape, out: np.ndarray = None) -> np.ndarray:
     """np.random.normal(0, sigma, shape).astype(np.float32) -- the draw of augmentations.py:31 -- bit for bit, consuming
     and advancing NumPy's GLOBAL legacy generator exactly like that call, but with the per-sample log / sqrt / divide of
     the polar method spread over all host threads (csrc/np_legacy_rng.cpp; the MT19937 word stream itself stays
     sequential).  The reference spends 104 of its 137 ms per 1360x765 frame in this draw."""
-    n = int(np.prod(shape))
-    state = np.random.get_state(legacy=True)
-    if state[0] != "MT19937" or not (float(sigma) >= 0.0):
-        return np.random.normal(0, sigma, shape).astype(np.float32)  # (raises ValueError for sigma < 0, like the reference)
     import ctypes
-    key = np.array(state[1], dtype=np.uint32, copy=True)
-    pos, has, cached = ctypes.c_int32(int(state[2])), ctypes.c_int32(int(state[3])), ctypes.c_double(float(state[4]))
+    n = int(np.prod(shape))
+    st = _legacy_state(sigma)
+    if st is None:
+        return np.random.normal(0, sigma, shape).astype(np.float32)  # (raises ValueError for sigma < 0, like the reference)
     if out is None:
         out = np.empty(n, dtype=np.float32)
     elif out.dtype != np.float32 or out.size != n or not out.flags.c_contiguous:
         raise ValueError("out must be a C-contiguous float32 array of prod(shape) elements")
+    key, pos, has, cached = st
     N.check(N.lib().rod_numpy_legacy_normal_f32(key.ctypes.data, ctypes.byref(pos), ctypes.byref(has), ctypes.byref(cached),
                                                 float(sigma), n, out.ctypes.data, 0), "rod_numpy_legacy_normal_f32")
-    np.random.set_state(("MT19937", key, pos.value, has.value, cached.value))
+    _set_legacy_state(st)
     return out.reshape(shape)
+
+
+def legacy_normal_f32_device(sigma: float, out, spans) -> int:
+    """The same stream as legacy_normal_f32, drawn on the GPU (csrc/legacy_rng.cu) straight into device memory: `out` is
+    a CUDA float32 tensor, `spans` a list of (offset, count) element ranges of it, sorted and disjoint.  The values of
+    np.random.normal(0, sigma, total).astype(np.float32) fill the spans in order -- one draw per image, back to back, is
+    the same stream as one draw per span -- and NumPy's global state ends where that call would leave it.  The draw is
+    queued on the current stream; the call returns once the state is known.  Returns the number of values that were
+    recomputed on the host (those whose float32 could depend on the last ulps of the device log())."""
+    import ctypes
+
+    import torch
+    if not (isinstance(out, torch.Tensor) and out.is_cuda and out.dtype == torch.float32 and out.is_contiguous()):
+        raise ValueError("out must be a contiguous CUDA float32 tensor")
+    offs = np.array([int(o) for o, _ in spans], dtype=np.uint64)
+    counts = np.array([int(c) for _, c in spans], dtype=np.uint64)
+    if any(int(o) < 0 or int(c) < 0 or int(o) + int(c) > out.numel() for o, c in spans):
+        raise ValueError("a span lies outside `out`")
+    st = _legacy_state(sigma) if float(sigma) != float("inf") else None
+    if st is None:  # NumPy's own draw (raises for sigma < 0 before any state changes)
+        vals = torch.from_numpy(np.random.normal(0, sigma, int(counts.sum())).astype(np.float32))
+        k = 0
+        for o, c in zip(offs.tolist(), counts.tolist()):
+            out[o:o + c].copy_(vals[k:k + c])
+            k += c
+        return 0
+    key, pos, has, cached = st
+    fix = ctypes.c_int(0)
+    with torch.cuda.device(out.device):
+        N.check(N.lib().rod_numpy_legacy_normal_f32_device(
+            key.ctypes.data, ctypes.byref(pos), ctypes.byref(has), ctypes.byref(cached), float(sigma), offs.ctypes.data,
+            counts.ctypes.data, len(spans), out.data_ptr(), ctypes.byref(fix), torch.cuda.current_stream().cuda_stream or None),
+            "rod_numpy_legacy_normal_f32_device")
+    _set_legacy_state(st)
+    return fix.value
 
 
 def apply_noise(img_bgr: np.ndarray, sigma: float) -> np.ndarray:

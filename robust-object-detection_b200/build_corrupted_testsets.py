@@ -16,8 +16,9 @@ byte-identical to cv2.imwrite's (tested).  `ENCODER = "host"` keeps cv2.imwrite 
 pinned staging, chunked H2D / kernel / D2H); other file types than .jpg / .jpeg always take that route.
 
 RNG: Test_Noise draws each image's field from NumPy's global legacy generator in glob order after np.random.seed(SEED)
--- the same stream as the reference's np.random.normal calls, regenerated bit for bit by csrc/np_legacy_rng.cpp with the
-per-sample math on all host threads -- so the noisy files are byte-identical too.
+-- the same stream as the reference's np.random.normal calls, regenerated bit for bit: on the GPU, one draw per batch
+(csrc/legacy_rng.cu) with the device encoder; on the host (csrc/np_legacy_rng.cpp, per-sample math on all host threads)
+with `ENCODER = "host"` -- so the noisy files are byte-identical too.
 `NOISE_MODE = "philox"` generates the field on the GPU instead (statistically equivalent, not byte-identical).
 
 Several GPUs (BASELINE configs[3], SURVEY 8e): started under `torchrun --nproc-per-node N` (RANK / WORLD_SIZE / LOCAL_RANK
@@ -38,7 +39,7 @@ import numpy as np
 
 from . import _native as N
 from .augmentations import apply_lowres, apply_motion_blur, apply_noise  # noqa: F401  (same names as the reference)
-from .augmentations import legacy_normal_f32
+from .augmentations import legacy_normal_f32, legacy_normal_f32_device
 from .augmentations import _motion_blur_kernel as motion_blur_kernel  # noqa: F401
 from .batch import CorruptionPlan
 from .sharding import shard_by_bytes
@@ -59,7 +60,7 @@ DOWNSCALE_FACTOR = 0.5
 NOISE_MODE = "compat"      # "compat": host np.random stream (byte-identical) | "philox": in-kernel RNG
 PHILOX_SEED = SEED
 BATCH_BYTES = 512 << 20    # decoded source bytes per GPU batch
-NOISE_BATCH_BYTES = 128 << 20   # ... of a compat-noise batch (its float32 field is 4x that, page-locked)
+NOISE_BATCH_BYTES = 128 << 20   # ... of a compat-noise batch on the host-encoder path (its float32 field is 4x that, page-locked)
 IO_THREADS = 16
 DECODER = "gpu"            # "gpu": device JPEG decoder for .jpg / .jpeg sources (same pixels as cv2.imread; needs ENCODER = "gpu") | "host": cv2.imread
 ENCODER = "gpu"            # "gpu": device JPEG encoder for .jpg / .jpeg outputs (same bytes as cv2.imwrite) | "host": cv2.imwrite
@@ -247,15 +248,11 @@ def _corrupt_encode(variant: str, r: "_DeviceRun", run: "_TreeRun"):
         pix = torch.empty(plan.dst_bytes, dtype=torch.uint8, device="cuda")
         if variant == "Test_Noise":
             field = None
-            if NOISE_MODE == "compat":   # the draws of augmentations.py:31, one per image, in order
-                total = sum(3 * h * w for h, w in plan.shapes)
-                noise = run.pinned("noise", 4 * total).view(np.float32)
-                o = 0
-                for h, w in plan.shapes:
-                    legacy_normal_f32(NOISE_SIGMA, (h, w, 3), out=noise[o:o + 3 * h * w])
-                    o += 3 * h * w
+            if NOISE_MODE == "compat":   # the draws of augmentations.py:31, one per image, in order: one device draw
                 # (indexed by the plan's packed element index -- images back to back -- as rod_noise_u8 expects)
-                field = run.pinned_tensor("noise", 4 * total).view(torch.float32).cuda(non_blocking=True)
+                total = sum(3 * h * w for h, w in plan.shapes)
+                field = torch.empty(total, dtype=torch.float32, device="cuda")
+                legacy_normal_f32_device(NOISE_SIGMA, field, [(0, total)])
             plan.noise(src_dev, pix, field, float(NOISE_SIGMA), seed=PHILOX_SEED, first_image_index=r.pos)
         elif variant == "Test_Blur":
             if float(BLUR_ANGLE_DEG) != 0.0:
@@ -353,9 +350,12 @@ def _process_images(src_img_dir: Path, dst_img_dir: Path, variant: str, run: "_T
     lo, hi = _shard_of(paths, variant)
     paths = paths[lo:hi]
 
-    # compat noise carries a float32 field of 4 bytes per pixel byte through page-locked memory: smaller batches there
-    cap = min(BATCH_BYTES, NOISE_BATCH_BYTES) if (variant == "Test_Noise" and NOISE_MODE == "compat") else BATCH_BYTES
     device = ENCODER == "gpu"
+    # the host-encoder path stages compat noise as a float32 field of 4 bytes per pixel byte in page-locked memory:
+    # smaller batches there.  The device path draws the field on the GPU, so its batches are those of the other variants
+    # (and so hit the device cache of the tree's decoded batches).
+    host_field = variant == "Test_Noise" and NOISE_MODE == "compat" and not device
+    cap = min(BATCH_BYTES, NOISE_BATCH_BYTES) if host_field else BATCH_BYTES
 
     def submit_loads(i):
         """read / decode ahead until the batch is full (cv2 and file reads release the GIL); a batch that is still on the

@@ -269,7 +269,7 @@ class RestorationPairBatcher:
         corrupted, clean = pairs(frames)        # float32 [B,3,P,P] RGB in [0,1], on the GPU
 
     noise="compat" draws each noise patch's field from NumPy's global legacy stream (bit-identical to the reference under
-    the same seeds: augmentations.legacy_normal_f32); noise="philox" generates it in the kernel, keyed by (seed, running
+    the same seeds: augmentations.legacy_normal_f32_device, one draw per batch on the GPU); noise="philox" generates it in the kernel, keyed by (seed, running
     sample index)."""
 
     def __init__(self, patch_size: int = 256, is_train: bool = True, noise: str = "compat", seed: int = 0):
@@ -283,7 +283,6 @@ class RestorationPairBatcher:
         self.last_decisions: List[tuple] = []
 
     def __call__(self, frames: Sequence[np.ndarray]):
-        from .augmentations import NOISE_SIGMA, legacy_normal_f32
         from .batch import draw_restoration_decisions, resize_linear_u8
         torch, P, n = self._torch, self.size, len(frames)
         if n not in self._plans:  # crops are staged back to back: one plan per batch size
@@ -292,7 +291,7 @@ class RestorationPairBatcher:
                               torch.empty(n * 3 * P * P, dtype=torch.uint8).pin_memory())
         plan, hbuf = self._plans[n]
         crops = hbuf.numpy().reshape(n, P, P, 3)
-        dec, fields = [], []
+        dec = []
         for i, im in enumerate(frames):
             if im.dtype != np.uint8 or im.ndim != 3 or im.shape[2] != 3:
                 raise ValueError("expected HWC uint8 BGR frames")
@@ -300,28 +299,24 @@ class RestorationPairBatcher:
                 im = resize_linear_u8(im, max(int(im.shape[0]), P), max(int(im.shape[1]), P))
             y, x, flip, op = draw_restoration_decisions(int(im.shape[0]), int(im.shape[1]), P, self.is_train)
             crops[i] = im[y:y + P, x:x + P]
-            if op == 1 and self.noise == "compat":  # the draw of apply_noise on the (flipped) patch, in sample order
-                fields.append(legacy_normal_f32(NOISE_SIGMA, (P, P, 3)).reshape(-1))
-            elif self.noise == "compat":
-                fields.append(None)
             dec.append((y, x, flip, op))
         self.last_decisions = dec
         src = hbuf.cuda()  # (synchronous for the host: the pinned crop buffer is rewritten by the next call)
-        return self._pairs(plan, src, dec, fields)
+        return self._pairs(plan, src, dec)
 
-    def _pairs(self, plan, src, dec, fields):
-        """src: the n crops back to back on the device; dec: (y, x, flip, op) per sample; fields: compat noise fields"""
-        from .augmentations import NOISE_SIGMA
+    def _pairs(self, plan, src, dec):
+        """src: the n crops back to back on the device; dec: (y, x, flip, op) per sample.  Compat mode draws the noise
+        samples' fields here, in sample order, in one device draw (the decisions consume only `random`, so drawing them
+        after all decisions is the reference's np.random stream)."""
+        from .augmentations import NOISE_SIGMA, legacy_normal_f32_device
         torch, P, n = self._torch, self.size, len(dec)
         flips = torch.tensor([int(d[2]) for d in dec], dtype=torch.uint8).cuda()
         ops = torch.tensor([d[3] for d in dec], dtype=torch.uint8).cuda()
         nz = None
-        if self.noise == "compat" and any(f is not None for f in fields):
-            host = np.zeros((n, 3 * P * P), dtype=np.float32)
-            for i, f in enumerate(fields):
-                if f is not None:
-                    host[i] = f
-            nz = torch.from_numpy(host.reshape(-1)).cuda()
+        noisy = [i for i, d in enumerate(dec) if d[3] == 1]
+        if self.noise == "compat" and noisy:
+            nz = torch.empty(n * 3 * P * P, dtype=torch.float32, device="cuda")
+            legacy_normal_f32_device(NOISE_SIGMA, nz, [(i * 3 * P * P, 3 * P * P) for i in noisy])
         corrupted = torch.empty((n, 3, P, P), dtype=torch.float32, device="cuda")
         clean = torch.empty_like(corrupted)
         plan.restoration_pairs(src, flips, ops, corrupted, clean, noise=nz, sigma=float(NOISE_SIGMA), seed=self.seed,
@@ -336,7 +331,6 @@ class RestorationPairBatcher:
         `random` / `np.random` state."""
         from concurrent.futures import ThreadPoolExecutor
         from . import _native as N
-        from .augmentations import NOISE_SIGMA, legacy_normal_f32
         from .batch import _ptr, _stream_handle, draw_restoration_decisions
         from .jpeg import JpegDecoder
         torch, P, n = self._torch, self.size, len(items)
@@ -365,7 +359,7 @@ class RestorationPairBatcher:
             self._plans[n] = (CorruptionPlan([(P, P)] * n, offs, [0] * n), torch.empty(n * 3 * P * P, dtype=torch.uint8).pin_memory())
         plan = self._plans[n][0]
         crops = torch.empty((n, P, P, 3), dtype=torch.uint8, device="cuda")
-        dec, fields = [], []
+        dec = []
         for i, (h, w) in enumerate(shapes):
             frame = dev[fplan.src_offsets[i]:fplan.src_offsets[i] + 3 * h * w].view(h, w, 3)
             if h < P or w < P:  # the reference enlarges such a frame first (train_restoration.py:79-81)
@@ -375,13 +369,9 @@ class RestorationPairBatcher:
                 frame, h, w = big, nh, nw
             y, x, flip, op = draw_restoration_decisions(h, w, P, self.is_train)
             crops[i].copy_(frame[y:y + P, x:x + P])
-            if op == 1 and self.noise == "compat":
-                fields.append(legacy_normal_f32(NOISE_SIGMA, (P, P, 3)).reshape(-1))
-            elif self.noise == "compat":
-                fields.append(None)
             dec.append((y, x, flip, op))
         self.last_decisions = dec
-        return self._pairs(plan, crops.reshape(-1), dec, fields)
+        return self._pairs(plan, crops.reshape(-1), dec)
 
 
 class DetectionCorruptionBatcher:
@@ -397,7 +387,8 @@ class DetectionCorruptionBatcher:
 
     Decisions: `random` is consumed as the per-item gate would (skip iff random() > p, then random.choice), for the whole
     batch first; in compat mode the fields of the noise images are then drawn from NumPy's global legacy stream in image
-    order (np.random.normal(0, 15, (H, W, 3)).astype(float32) for the BGR array: augmentations.legacy_normal_f32).  The two
+    order (np.random.normal(0, 15, (H, W, 3)).astype(float32) for the BGR array), in one device draw per batch
+    (augmentations.legacy_normal_f32_device).  The two
     streams are independent, so this equals the reference's per-item interleaving.  noise="philox" generates the field in
     the kernel instead (the plan's generator, keyed by (seed, running image index)).  The drawn op-codes are left in
     .last_ops.
@@ -464,7 +455,7 @@ class DetectionCorruptionBatcher:
     def _stage(self, slot: dict, items: Sequence, futs) -> None:
         """Read / decode / pack one batch into the slot's buffers on the copy stream and draw its decisions."""
         torch = self._torch
-        from .augmentations import NOISE_SIGMA, legacy_normal_f32
+        from .augmentations import NOISE_SIGMA, legacy_normal_f32_device
         from .jpeg import JpegDecoder
         loaded = [f.result() for f in futs]
         shapes = [sh for _, sh in loaded]
@@ -477,7 +468,8 @@ class DetectionCorruptionBatcher:
                                   ("ops", torch.uint8, max(n, 64))):
             if slot.get(name + "_cap", 0) < size:
                 cap = max(size, 2 * slot.get(name + "_cap", 0))
-                slot[name + "_host"] = torch.empty(cap, dtype=dtype).pin_memory()
+                if name != "noise":  # (the compat field is drawn on the device)
+                    slot[name + "_host"] = torch.empty(cap, dtype=dtype).pin_memory()
                 slot[name + "_dev"] = torch.empty(cap, dtype=dtype, device="cuda")
                 slot[name + "_cap"] = cap
                 grow = True
@@ -507,7 +499,14 @@ class DetectionCorruptionBatcher:
                 (h, w), off = shapes[i], offs[i]
                 hbuf[off:off + 3 * h * w].reshape(h, w, 3)[...] = loaded[i][0][:, :, ::-1]
 
-            list(self._pool.map(pack, host_idx))
+            packing = [self._pool.submit(pack, i) for i in host_idx]
+            ops = draw_decisions(n, gate="pil", p=self.p)
+            noise = None
+            if self.noise == "compat" and (ops == 1).any():  # the noise images' fields in image order: one device draw
+                noise = slot["noise_dev"]
+                legacy_normal_f32_device(NOISE_SIGMA, noise, [(int(elem_base[i]), elems[i]) for i in np.flatnonzero(ops == 1)])
+            for f in packing:
+                f.result()
             # one copy per run of consecutive host-sourced images
             k = 0
             while k < len(host_idx):
@@ -518,15 +517,6 @@ class DetectionCorruptionBatcher:
                 hi = offs[host_idx[j]] + elems[host_idx[j]]
                 dev[lo:hi].copy_(slot["src_host"][lo:hi], non_blocking=True)
                 k = j + 1
-            ops = draw_decisions(n, gate="pil", p=self.p)
-            noise = None
-            if self.noise == "compat" and (ops == 1).any():
-                nh, nd = slot["noise_host"], slot["noise_dev"]
-                for i in np.flatnonzero(ops == 1):  # only the noise images' spans are drawn and uploaded
-                    lo, hi = int(elem_base[i]), int(elem_base[i + 1])
-                    legacy_normal_f32(NOISE_SIGMA, shapes[i] + (3,), out=nh.numpy()[lo:hi])
-                    nd[lo:hi].copy_(nh[lo:hi], non_blocking=True)
-                noise = nd
             slot["ops_host"][:n] = torch.from_numpy(ops)
             slot["ops_dev"][:n].copy_(slot["ops_host"][:n], non_blocking=True)
             ready = torch.cuda.Event()
