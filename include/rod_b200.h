@@ -72,7 +72,11 @@ ROD_API void rod_plan_destroy(rod_plan* plan);
 ROD_API int  rod_plan_num_images(const rod_plan* plan);
 /* Sum over images of 3*H*W: bytes one full-resolution pass reads (and writes). */
 ROD_API uint64_t rod_plan_payload_bytes(const rod_plan* plan);
-/* Number of kernels one call of the given op launches (for launch accounting). */
+/* Number of kernels one call of the given op launches (for launch accounting; the counter memsets and the copies of
+ * the host entry points are not counted).  ROD_OP_LOWRES: 1 until the first LowRes call built the resize tables, then
+ * one per non-empty tile list.  That is exact when the source base pointer of the call is 4-byte aligned and, if the
+ * plan has images for the staged exact-2x kernels, so is the destination base.  Otherwise one strip-kernel launch
+ * replaces all the exact-2x band and strip launches, and the call launches fewer kernels than this count. */
 ROD_API int  rod_plan_launches(const rod_plan* plan, int op);
 
 /* a1: apply_noise (augmentations.py:30-33).

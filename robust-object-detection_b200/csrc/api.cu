@@ -144,7 +144,8 @@ extern "C" int rod_plan_launches(const rod_plan* plan, int op) {
         case ROD_OP_NONE: case ROD_OP_NOISE: case ROD_OP_BLUR: return 1;
         case ROD_OP_LOWRES: {  // one launch per non-empty tile list (known once the resize tables exist)
             if (plan->d_shapes == nullptr) return 1;
-            // except the full strip list: it runs only when the base pointers are not 4-byte aligned, in place of the others
+            // except the full strip list: it runs only when the source base (or, with staged lists, the destination base)
+            // is not 4-byte aligned, in place of the band lists and X2_REST; such a call launches fewer kernels
             int n = 0;
             for (int l = 0; l < LR_NUM_LISTS; ++l) n += l != LR_X2_STRIP && plan->lowres[l].n > 0;
             return n > 0 ? n : 1;

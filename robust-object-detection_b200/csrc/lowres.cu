@@ -1,16 +1,41 @@
 // lowres.cu -- a4+a5: fused INTER_AREA downscale + 8-bit INTER_LINEAR upscale (sm_100a).
 //
 // Reference: scripts/augmentations.py:41-45 (apply_lowres): cv2.resize(img,(nw,nh),INTER_AREA) followed by
-// cv2.resize(small,(w,h),INTER_LINEAR).  The low-resolution intermediate never exists in HBM.  Three kernels:
-//   lowres_x2w_kernel  exact-2x widths with w % 4 == 0 and 4-byte aligned rows (every VisDrone frame size): warp-marching,
-//                      the low-res rows live in registers (see the banner above the kernel)
-//   lowres_x2_kernel   exact-2x widths whose rows are not 4-byte aligned: full-width strips, low-res rows in shared memory
-//   lowres_kernel      any other shape (odd widths, other factors): tiles of kLowresTH rows x kLowresTWB output BYTES
-//                      (cut in byte columns: every stage is per byte, channel = byte % 3)
+// cv2.resize(small,(w,h),INTER_LINEAR).  The low-resolution intermediate never exists in HBM.
+//
+// Every image goes to one tile list (ensure_lowres_tables in plan.cu); a call launches one kernel per non-empty list
+// (launch_lowres_lists below).  Shapes are at factor 0.5 unless noted; "rows aligned to n" means the image's pitch and
+// offset are multiples of n.  tests/test_kernel_paths.py asserts this table.
+//   kernel                       list          layouts that select it
+//   lowres_x2i_kernel<true>      X2I_CARRY     odd w = 2 nw + 1 with three x taps, regular y axis, odd h
+//   lowres_x2i_kernel<false>     X2I_EVEN      ... even h
+//   lowres_x2g_kernel            X2G           odd w with three x taps, other y axes (no alignment requirement)
+//   lowres_x2p_kernel<16|8|4>    X2P16|8|4     exact 2x in both axes, w % 4 == 0; source and destination rows aligned to 4;
+//                                              copy unit 16 / 8 / 4: w and every pitch and offset a multiple of it
+//   lowres_x2h_kernel<16|8|4>    X2H16|8|4     exact-2x width, w % 4 == 0, odd h whose low-res row j reads source rows
+//                                              2j..2j+2 (h up to ~2000); alignment and copy unit as X2P
+//   lowres_x2f_kernel<16|8|4>    X2F16|8|4     exact-2x width, w % 4 == 0, other packed y axes (odd h from ~2001); as X2P
+//   lowres_x2w_kernel<true>      X2W8          the X2P / X2H / X2F shapes whose source rows are aligned to 8 (w % 8 == 0)
+//                                              but whose destination rows are not aligned to 4 (odd pitch, offset 2 mod 4)
+//   lowres_x2w_kernel<false>     X2W4          ... source rows aligned to 4 only; and X2W8 when the source base is not
+//                                              8-aligned
+//   lowres_x2_kernel<128>        X2_REST       other exact-2x widths (w % 4 != 0 or a FASTN y axis), and the X2P / X2H /
+//                                              X2F shapes whose source rows are not aligned to 4
+//                                X2_STRIP      every exact-2x image, in place of all of the above but X2I / X2G, when the
+//                                              source base is not 4-aligned, or the destination base is not 4-aligned
+//                                              while an X2P / X2H / X2F list is not empty
+//   lowres_kernel                GENERIC       anything else (other factors, widths that are not 2 nw or 2 nw + 1)
+// The base pointers may also be less aligned than a staged list's copy unit: the list then runs the kernel of the unit
+// that src | dst allows (lowres_x2p_kernel<8> for X2P16 at a base 8 mod 16).
+//
+// lowres_kernel: tiles of kLowresTH rows x kLowresTWB output BYTES (cut in byte columns: every stage is per byte,
+// channel = byte % 3)
 //     phase B1/B2: separable INTER_AREA in OpenCV's operation order (resizeArea_ / resizeAreaFast_), horizontal pass
 //                  per source row into a float buffer, then the y taps -> low-res tile P (u8, shared)
 //     phase C1   : horizontal fixed-point pass  hx = (P[s0]*a0 + P[s1]*a1) >> 4   (u16, shared)
 //     phase C2   : vertical pass + pack; each thread owns 8 byte columns and marches down 8 rows
+// lowres_x2_kernel: full-width strips, low-res rows in shared memory.  The band kernels (x2w, x2p, x2h, x2f, x2g, x2i):
+// a warp owns a band of rows x a strip of 30 chunks of 8 output pixels (see the banner above lowres_x2w_kernel).
 
 #include <algorithm>
 #include <mutex>

@@ -428,10 +428,12 @@ def test_ragged_mixed_resolution_batch(torch_):
 
 
 def test_lowres_marching_kernel_alignments(torch_):
-    """lowres_x2w_kernel (warp-marching bands x strips): images packed at 4-byte granularity (rows that are not
-    8-byte aligned take the 32-bit load path), widths with a two-pixel last chunk, pitched rows, and a source base
-    that is not 4-byte aligned (falls back to the strip kernel).  Odd heights above 1999 are the only shapes that
-    select lowres_x2f_kernel (w % 4 == 0) and lowres_x2g_kernel (odd w)."""
+    """The band kernels on rows at 4- and 8-byte phases: images packed at 4-byte granularity (their destination rows
+    stay 4-byte aligned, so the exact-2x images go to lowres_x2p_kernel / lowres_x2h_kernel with 8- or 4-byte copy
+    units, not to lowres_x2w_kernel), widths with a two-pixel last chunk, pitched rows, and a source base that is not
+    4-byte aligned (the strip kernel lowres_x2_kernel takes every exact-2x image).  (2001, 1360) selects
+    lowres_x2f_kernel and (2001, 1361) lowres_x2g_kernel.  tests/test_kernel_paths.py traces which kernel each layout
+    reaches, lowres_x2w_kernel included."""
     from robust_object_detection_b200.batch import CorruptionPlan
     shapes = [(765, 1360), (360, 480), (100, 8), (9, 4), (2, 4), (5, 12), (64, 64), (65, 128), (131, 36), (201, 1400),
               (97, 1916), (540, 960), (33, 2000), (40, 20), (77, 1364), (1080, 1920), (1050, 1400), (41, 44),
