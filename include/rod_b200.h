@@ -76,7 +76,12 @@ ROD_API uint64_t rod_plan_payload_bytes(const rod_plan* plan);
  * the host entry points are not counted).  ROD_OP_LOWRES: 1 until the first LowRes call built the resize tables, then
  * one per non-empty tile list.  That is exact when the source base pointer of the call is 4-byte aligned and, if the
  * plan has images for the staged exact-2x kernels, so is the destination base.  Otherwise one strip-kernel launch
- * replaces all the exact-2x band and strip launches, and the call launches fewer kernels than this count. */
+ * replaces all the exact-2x band and strip launches, and the call launches fewer kernels than this count.
+ * The combined entry points have codes of their own: 100 = rod_corrupt_batch_u8 (copy, noise, blur, then the LowRes
+ * lists), 101 = rod_corrupt_letterbox_f16 on its unfused path (noise, blur, LowRes lists, letterbox) and 102 =
+ * rod_corrupt_chw_f32 (noise, blur, LowRes lists, conversion); each is 3 + the ROD_OP_LOWRES count, with the same
+ * base-pointer caveat.  rod_corrupt_letterbox_f16 on its fused path launches 1 kernel, plus the ROD_OP_LOWRES count
+ * when the LowRes images do not run inside that kernel. */
 ROD_API int  rod_plan_launches(const rod_plan* plan, int op);
 
 /* a1: apply_noise (augmentations.py:30-33).
@@ -167,7 +172,9 @@ ROD_API int rod_corrupt_batch_u8(rod_plan* plan, const uint8_t* src, uint8_t* ds
 /* Training path (BASELINE config 5): corruption fused with the detector-input formatting
  * of Ultralytics' LetterBox + Format + preprocess_batch: INTER_LINEAR resize-to-fit of the
  * CORRUPTED pixels, constant pad, BGR->RGB, HWC->CHW, half(float(u8)/255).  `out` is a
- * device fp16 array [n_images, 3, out_h, out_w]. */
+ * device fp16 array [n_images, 3, out_h, out_w].  Any 2-byte aligned `out` is accepted; the fused kernel stores pairs
+ * of halves, so it runs only when `out` is 4-byte aligned (and out_w is even), otherwise the unfused path computes the
+ * same bytes. */
 ROD_API int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, const uint8_t* opcodes,
                               void* out_f16, int out_h, int out_w, int pad_value,
                               const float* noise, float sigma, int k, double factor, uint64_t seed,

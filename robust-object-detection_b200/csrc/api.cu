@@ -150,9 +150,11 @@ extern "C" int rod_plan_launches(const rod_plan* plan, int op) {
             for (int l = 0; l < LR_NUM_LISTS; ++l) n += l != LR_X2_STRIP && plan->lowres[l].n > 0;
             return n > 0 ? n : 1;
         }
-        case 100: return 4;  // rod_corrupt_batch_u8: copy + noise + blur + lowres
-        case 101: return 4;  // rod_corrupt_letterbox_f16: noise + blur + lowres + letterbox (clean images are read in place)
-        case 102: return 4;  // rod_corrupt_chw_f32: noise + blur + lowres + conversion (clean images are read in place)
+        // the combined entry points (not op-codes): three single-launch stages plus the LowRes lists
+        case 100:  // rod_corrupt_batch_u8: copy, noise, blur, LowRes
+        case 101:  // rod_corrupt_letterbox_f16, unfused path: noise, blur, LowRes, letterbox (clean images read in place)
+        case 102:  // rod_corrupt_chw_f32: noise, blur, LowRes, conversion (clean images read in place)
+            return 3 + rod_plan_launches(plan, ROD_OP_LOWRES);
         default: return 0;
     }
 }
@@ -249,10 +251,12 @@ extern "C" int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, con
     rc = ensure_scratch(plan);
     if (rc != ROD_OK) return rc;
     // Fused path: noise / blur / clean rows are produced inside the letterbox kernel (no full-resolution round trip);
-    // only LowRes images go through the scratch.  Needs an even output width (two columns per lane, half2 stores), plain
-    // linear letterboxes, the angle-0 blur and Philox sigma in range.
-    const bool fused = (out_w & 1) == 0 && plan->lb_all_linear && plan->f2d_ntaps == 0 && blur_supported(k, 0.0) &&
-                       k >= 3 && (noise != nullptr || sigma <= kPhiloxMaxSigma);
+    // only LowRes images go through the scratch.  Needs an even output width and a 4-byte aligned output base (two
+    // columns per lane, half2 stores), plain linear letterboxes, the angle-0 blur, Philox sigma in range and rows narrow
+    // enough for the per-warp shared-memory buffers.
+    const bool fused = (out_w & 1) == 0 && (((uintptr_t)out_f16) & 3) == 0 && plan->lb_all_linear &&
+                       plan->f2d_ntaps == 0 && blur_supported(k, 0.0) && k >= 3 &&
+                       (noise != nullptr || sigma <= kPhiloxMaxSigma) && fused_letterbox_smem(plan) <= kFusedMaxSmem;
     if (fused) {
         rc = ensure_lowres_tables(plan, factor);
         if (rc != ROD_OK) return rc;
@@ -264,9 +268,8 @@ extern "C" int rod_corrupt_letterbox_f16(rod_plan* plan, const uint8_t* src, con
                         opcodes, (cudaStream_t)stream, 0, plan->n_images);
             if (rc != ROD_OK) return rc;
         }
-        rc = launch_fused_letterbox(plan, src, plan->d_scratch, opcodes, noise, out_f16, pad_value, sigma, k, seed,
-                                    first_image_index, offset, in_kernel, (cudaStream_t)stream);
-        if (rc != ROD_ERR_UNSUPPORTED) return rc;  // rows too wide for the per-warp buffers: unfused path below
+        return launch_fused_letterbox(plan, src, plan->d_scratch, opcodes, noise, out_f16, pad_value, sigma, k, seed,
+                                      first_image_index, offset, in_kernel, (cudaStream_t)stream);
     }
     // images that stay clean are read from `src` by the letterbox kernel itself: no copy into the scratch
     rc = run_mixed_ops(plan, ROD_OP_NOISE, src, plan->d_scratch, opcodes, noise, sigma, k, factor, seed, first_image_index,

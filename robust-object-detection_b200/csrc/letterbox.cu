@@ -510,6 +510,20 @@ __global__ void __launch_bounds__(32 * NW, 16 / NW) fused_letterbox2_kernel(Fuse
     }
 }
 
+// 4 warps per CTA: smaller CTAs balance the expensive noise / blur / LowRes rows (measured 6 % faster than 8 at batch 64,
+// equal at batch 16).  Measured on a B200 (1360x765 sources, seed-42 mix): batch 64 152 us, batch 16 43.5 us.
+// (Tried and dropped: keeping the NEXT row's source rows in flight during the resampling loop -- four row buffers per
+// warp, 12 warps per SM: 171 us at batch 64.  The loop is bound by its shared-memory reads, not by the source-row
+// latency: at scale 2.125 the six-byte windows of every fifth column pair fall into the same bank.)
+constexpr int kFusedWarps = 4;
+
+// bytes of one row buffer: also holds two low-res rows (3 * max_w / 2 + 39 each)
+static int fused_buf_bytes(const rod_plan* plan) { return kFusedLeft + ((3 * plan->max_w + 15) & ~15) + 128; }
+
+size_t fused_letterbox_smem(const rod_plan* plan) {
+    return (size_t)(2 * kFusedMaxSorted + 32) + (size_t)kFusedWarps * (size_t)(3 * fused_buf_bytes(plan));
+}
+
 int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8_t* scratch, const uint8_t* opcodes,
                            const float* noise, void* out_f16, int pad_value, float sigma, int k, uint64_t seed,
                            uint64_t first_image, uint32_t offset, bool lowres_in_kernel, cudaStream_t stream) {
@@ -523,15 +537,10 @@ int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8
     p.key0 = (uint32_t)seed; p.key1 = (uint32_t)(seed >> 32); p.offset = offset; p.first_image = first_image;
     p.keys = philox_round_keys(p.key0, p.key1);
     p.k = k;
-    p.buf_bytes = kFusedLeft + ((3 * plan->max_w + 15) & ~15) + 128;  // also holds two low-res rows (3 * max_w / 2 + 39 each)
-    // 4 warps per CTA: smaller CTAs balance the expensive noise / blur / LowRes rows (measured 6 % faster than 8 at batch 64,
-    // equal at batch 16).  Measured on a B200 (1360x765 sources, seed-42 mix): batch 64 152 us, batch 16 43.5 us.
-    // (Tried and dropped: keeping the NEXT row's source rows in flight during the resampling loop -- four row buffers per
-    // warp, 12 warps per SM: 171 us at batch 64.  The loop is bound by its shared-memory reads, not by the source-row
-    // latency: at scale 2.125 the six-byte windows of every fifth column pair fall into the same bank.)
-    constexpr int nw = 4;
-    const size_t smem = (size_t)(2 * kFusedMaxSorted + 32) + (size_t)nw * (size_t)(3 * p.buf_bytes);
-    if (smem > 227 * 1024) return ROD_ERR_UNSUPPORTED;
+    p.buf_bytes = fused_buf_bytes(plan);
+    constexpr int nw = kFusedWarps;
+    const size_t smem = fused_letterbox_smem(plan);
+    if (smem > kFusedMaxSmem) return ROD_ERR_UNSUPPORTED;
     int per_sm = (int)((227 * 1024) / (smem + 1024));
     per_sm = per_sm < 1 ? 1 : per_sm;
     // one output row per warp, dealt round-robin (no work counter: one launch, nothing else on the stream)

@@ -26,6 +26,7 @@ constexpr int kF2dTH = 16;         // general 2-D filter tile: rows x output byt
 constexpr int kF2dTWB = 768;
 constexpr int kF2dMaxElems = 130;  // cv::filter2D uses DFT-based convolution from 130 kernel elements on (8U)
 constexpr int kChwBandRows = 8;    // CHW conversion: rows per work item, one per warp
+constexpr size_t kFusedMaxSmem = 227 * 1024;  // fused letterbox: dynamic shared memory one CTA may use
 
 struct HostShape {
     int h, w;
@@ -182,6 +183,9 @@ int launch_resize_linear(const uint8_t* src, int h, int w, int64_t src_pitch, ui
                          cudaStream_t stream);
 int launch_format_pairs(const rod_plan* inner, const uint8_t* clean, const uint8_t* corrupted, float* clean_out,
                         float* corrupted_out, cudaStream_t stream);
+// dynamic shared memory of the fused letterbox kernel for this plan (row buffers sized by its widest image); the fused
+// path is taken only when it is at most kFusedMaxSmem
+size_t fused_letterbox_smem(const rod_plan* plan);
 int launch_fused_letterbox(const rod_plan* plan, const uint8_t* src, const uint8_t* scratch, const uint8_t* opcodes,
                            const float* noise, void* out_f16, int pad_value, float sigma, int k, uint64_t seed,
                            uint64_t first_image, uint32_t offset, bool lowres_in_kernel, cudaStream_t stream);

@@ -81,9 +81,9 @@ def kernel_name(raw: str) -> str:
     return base.split("::")[-1] + lt + args
 
 
-def test_kernel_list_matches_library():
-    """KERNELS holds every entry point of noise.cu, blur.cu, filter2d.cu and lowres.cu in the built library, and
-    nothing else: a kernel added or removed there must be added to or removed from the matrix below."""
+def library_kernels(sources):
+    """{source file: sorted kernel names (as in KERNELS)} of the entry points the built library holds for each of
+    `sources` (cuobjdump -symbols, demangled with cu++filt)."""
     if not os.path.exists(LIB):
         import __graft_entry__ as g
         g.build()
@@ -94,21 +94,30 @@ def test_kernel_list_matches_library():
         m = re.match(r"\s*identifier\s*=\s*(\S+)", line)
         if m:
             ident = os.path.basename(m.group(1))
-        elif "STO_ENTRY" in line and ident in KERNELS:
+        elif "STO_ENTRY" in line and ident in sources:
             entries[ident].append(line.split()[-1])
-    for ident, want in KERNELS.items():
+    out = {}
+    for ident in sources:
         assert entries[ident], f"no entry symbols of {ident} in {LIB}"
         names = subprocess.check_output([os.path.join(bindir, "cu++filt")], input="\n".join(entries[ident]) + "\n",
                                         text=True).split("\n")
-        got = sorted(kernel_name(n) for n in names if n.strip())
+        out[ident] = sorted(kernel_name(n) for n in names if n.strip())
+    return out
+
+
+def test_kernel_list_matches_library():
+    """KERNELS holds every entry point of noise.cu, blur.cu, filter2d.cu and lowres.cu in the built library, and
+    nothing else: a kernel added or removed there must be added to or removed from the matrix below."""
+    for ident, got in library_kernels(KERNELS).items():
+        want = KERNELS[ident]
         assert got == sorted(want), (ident, sorted(set(got) ^ set(want)))
     assert len(ALL_KERNELS) == 27
 
 
 # ------------------------------------------------------------------ launch trace
-def launched(fn):
-    """Runs fn() under torch.profiler (CUDA activity only) and returns the kernels it launched (names as in KERNELS,
-    with multiplicity); copies and memsets are left out."""
+def trace(fn):
+    """Runs fn() under torch.profiler (CUDA activity only) and returns the kernels it launched (names as in KERNELS)
+    in the order they started; copies and memsets are left out."""
     import torch
     from torch.profiler import ProfilerActivity, profile
     torch.cuda.synchronize()
@@ -121,8 +130,13 @@ def launched(fn):
             continue
         if e.name.startswith(("Memcpy", "Memset")) or "(" not in e.name:   # kernels carry their parameter list
             continue
-        names.append(kernel_name(e.name))
-    return collections.Counter(names)
+        names.append((e.time_range.start, kernel_name(e.name)))
+    return [n for _, n in sorted(names, key=lambda t: t[0])]
+
+
+def launched(fn):
+    """The kernels fn() launched (names as in KERNELS, with multiplicity)."""
+    return collections.Counter(trace(fn))
 
 
 # ------------------------------------------------------------------ layouts
@@ -274,11 +288,12 @@ def lowres_list(fam, w, so, sp, do, dp):
     return (fam, 0 if w % 16 == 0 and a % 16 == 0 else (1 if w % 8 == 0 and a % 8 == 0 else 2))
 
 
-def expected_lowres(b: Batch, factor=0.5):
-    """(Counter of the kernels one LowRes call of batch b launches, whether the strip kernel replaced the band lists)."""
+def expected_lowres(b: Batch, factor=0.5, family=FAMILY):
+    """(Counter of the kernels one LowRes call of batch b launches, whether the strip kernel replaced the band lists).
+    b needs shapes, so / sp / do / dp and src / dst with data_ptr(); `family` classifies every shape."""
     if factor != 0.5:
         return collections.Counter({"lowres_kernel": 1}), False
-    lists = {lowres_list(FAMILY[(h, w)], w, so, sp, do, dp)
+    lists = {lowres_list(family[(h, w)], w, so, sp, do, dp)
              for (h, w), so, sp, do, dp in zip(b.shapes, b.so, b.sp, b.do, b.dp)}
     sbase, dbase = b.src.data_ptr(), b.dst.data_ptr()
     staged = [l for l in lists if isinstance(l, tuple)]
