@@ -237,11 +237,18 @@ ROD_API int rod_jpeg_download(rod_jpeg_encoder* enc, uint8_t* host_out, uint32_t
  * one scan (restart markers are fine), no EXIF rotation, either Y Cb Cr with the luma sampled 2x2 (4:2:0, what OpenCV's own
  * encoder writes), 2x1 (4:2:2) or 1x1 (4:4:4) against 1x1 chroma, or greyscale; subsampled files need width >= 5.  Every
  * other file is REPORTED (status >= 10), never approximated: the caller reads it with the host codec.
+ * The _ex forms also take PROGRESSIVE files (SOF2, same frame layouts, Huffman coded, table slots 0..3, restart markers
+ * fine) when `formats` has ROD_JPEGDEC_PROGRESSIVE: every scan is checked as libjpeg-turbo's jdphuff.c does, and a file
+ * whose scans leave a coefficient bit unknown (libjpeg would block-smooth it) or redefine a quantisation table in use is
+ * reported as 12; one without EOI behind its last scan as 13.  A complete progressive file decodes to the pixels of its
+ * baseline twin.  The plain forms are the _ex forms with ROD_JPEGDEC_BASELINE.
  *   rod_jpegdec_probe        host only: ROD_OK + (height, width) when the device decoder takes the file, else
  *                            ROD_ERR_UNSUPPORTED
+ *   rod_jpegdec_probe_ex     the same for the formats in `formats` (a progressive file is walked to its EOI)
  *   rod_jpegdec_create       host work for a batch (markers, tables, scans without byte stuffing into page-locked memory,
  *                            on `host_threads` threads); image i will be written at pixels + dst_offsets[i] with row pitch
  *                            dst_pitches[i] bytes (NULL or 0: 3 * width)
+ *   rod_jpegdec_create_ex    the same for the formats in `formats`; baseline and progressive files mix in one batch
  *   rod_jpegdec_host_status  the verdict of create per image (0: decodable; 11: not a JPEG; 12: unsupported layout;
  *                            13: scan does not end in EOI) and the sizes of the decodable ones
  *   rod_jpegdec_decode       upload + Huffman decoding + IDCT + upsampling / colour conversion on `stream`; returns when the
@@ -249,9 +256,14 @@ ROD_API int rod_jpeg_download(rod_jpeg_encoder* enc, uint8_t* host_out, uint32_t
  *   rod_jpegdec_status       waits for `stream`; per image 0: decoded; 1 / 2: corrupt / truncated entropy data (pixels
  *                            undefined); >= 10: as above */
 typedef struct rod_jpeg_decoder rod_jpeg_decoder;
+#define ROD_JPEGDEC_BASELINE 1
+#define ROD_JPEGDEC_PROGRESSIVE 2
 ROD_API int rod_jpegdec_probe(const uint8_t* file, uint64_t n, int* height, int* width);
+ROD_API int rod_jpegdec_probe_ex(const uint8_t* file, uint64_t n, int formats, int* height, int* width);
 ROD_API int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* lens, int n_images, const uint64_t* dst_offsets,
                        const int64_t* dst_pitches, int host_threads, rod_jpeg_decoder** out_dec);
+ROD_API int rod_jpegdec_create_ex(const uint8_t* const* files, const uint64_t* lens, int n_images, const uint64_t* dst_offsets,
+                          const int64_t* dst_pitches, int host_threads, int formats, rod_jpeg_decoder** out_dec);
 ROD_API void rod_jpegdec_destroy(rod_jpeg_decoder* dec);   /* its device / page-locked buffers go to caches for the next decoder */
 ROD_API void rod_jpegdec_trim(void);                          /* frees the page-locked cache (the device cache: rod_jpeg_trim) */
 ROD_API int rod_jpegdec_host_status(const rod_jpeg_decoder* dec, int32_t* status, int32_t* heights, int32_t* widths);

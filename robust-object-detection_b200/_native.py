@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(_HERE, "librod_b200.so")
 ROD_OK, ROD_ERR_INVALID_ARG, ROD_ERR_UNSUPPORTED, ROD_ERR_CUDA, ROD_ERR_NO_DEVICE, ROD_ERR_OOM = range(6)
 OP_NONE, OP_NOISE, OP_BLUR, OP_LOWRES = 0, 1, 2, 3
 LAUNCHES_CORRUPT_BATCH, LAUNCHES_CORRUPT_LETTERBOX, LAUNCHES_CORRUPT_CHW = 100, 101, 102
+JPEGDEC_BASELINE, JPEGDEC_PROGRESSIVE = 1, 2
 
 
 class ImageDesc(ctypes.Structure):
@@ -63,7 +64,9 @@ SYMBOLS = {
     "rod_jpeg_stream_lengths": (_vp, [_vp]),
     "rod_jpeg_download": (_i, [_vp, _vp, _vp, _vp]),
     "rod_jpegdec_probe": (_i, [_vp, _u64, ctypes.POINTER(_i), ctypes.POINTER(_i)]),
+    "rod_jpegdec_probe_ex": (_i, [_vp, _u64, _i, ctypes.POINTER(_i), ctypes.POINTER(_i)]),
     "rod_jpegdec_create": (_i, [_vp, _vp, _i, _vp, _vp, _i, ctypes.POINTER(_vp)]),
+    "rod_jpegdec_create_ex": (_i, [_vp, _vp, _i, _vp, _vp, _i, _i, ctypes.POINTER(_vp)]),
     "rod_jpegdec_destroy": (None, [_vp]),
     "rod_jpegdec_trim": (None, []),
     "rod_jpegdec_host_status": (_i, [_vp, _vp, _vp, _vp]),

@@ -16,11 +16,22 @@
 //             jpegdec_write_kernel   decodes from the now exact start states and stores the coefficients (int16, natural
 //                                    order, per-component block rasters; DC as the difference)
 //             jpegdec_dc_kernel      DC prediction = prefix sum of the differences per component in MCU order
+//           progressive files: the scans in dependency levels (rod_jpegdec_host.h scan_levels), one launch per level
+//             jpegdec_prog_kernel    one thread per (image, scan, restart interval) of the level, sequentially through the
+//                                    interval (rod_jpegdec.h decode_prog_segment: DC predictions and EOBRUN resolved in
+//                                    place, refinements read the coefficients of the earlier levels); the Huffman tables
+//                                    of the batch's scans are read through L1; refinement scans only decode (history
+//                                    from jpegdec_mask_kernel's per-block masks, results as masks per block)
+//             jpegdec_mask_kernel    before a level with AC refinement scans: one thread per coefficient block, its
+//                                    nonzero coefficients as a 64-bit mask over zigzag positions
+//             jpegdec_apply_kernel   after a level with refinement scans: one thread per block of each, the corrections
+//                                    and new coefficients applied
 //           jpegdec_idct_kernel      one thread per 8x8 block: dequantisation + islow IDCT in registers -> Y / Cb / Cr planes
 //           jpegdec_color_kernel     one thread per four output pixels: fancy chroma upsampling + YCbCr -> BGR, written
 //                                    straight into the caller's HWC batch (the layout of a rod_plan)
-// Files of another layout (progressive, EXIF rotation, CMYK, 4:1:1 ...) are reported per image; the caller
-// decodes those with the host codec.  No CPU decoding in here.
+// Baseline and progressive files share one coefficient buffer and one IDCT / colour pass.  Files of another layout
+// (progressive unless the caller asked for it, EXIF rotation, CMYK, 4:1:1 ...) are reported per image; the caller decodes
+// those with the host codec.  No CPU decoding in here.
 #include <algorithm>
 #include <map>
 #include <string>
@@ -52,6 +63,11 @@ struct JpegDecParams {
     uint32_t* first_block;         // [subsequence] global block index its first symbol belongs to
     unsigned int* changed;         // one flag per sync launch
     int n_images;
+    const ScanRec* scans;          // progressive files: their scans, restart intervals (grouped by level) and tables
+    const ScanSeg* psegs;
+    const HuffTab* huff;
+    uint64_t* nzmask;              // [coefficient block] zigzag_nz_mask before a level with AC refinement scans
+    RefineOut* refine;             // refinement scans' results (ScanRec::out_block), applied after their level
 };
 
 constexpr int kHuffThreads = 128;
@@ -170,6 +186,46 @@ __global__ void __launch_bounds__(kHuffThreads) jpegdec_write_kernel(JpegDecPara
                       s == 0 ? span_state(bit0, 0, 0, 0) : state_start(p.end_state[gs - 1]), bit0 + (s + 1) * kSubBits,
                       p.coef + im.coef_off, sg.first_block + local, sg.first_block + sg.n_blocks, &err);
     if (err) atomicMax(p.status + sg.image, 1);
+}
+
+// One thread per restart interval of a progressive scan, `lanes` threads per warp (the intervals are serial work with
+// divergent control flow: a warp of its own for each while the level has few of them).  Segments [seg0, seg0 + n).
+__global__ void __launch_bounds__(128) jpegdec_prog_kernel(JpegDecParams p, uint32_t seg0, uint32_t n, uint32_t lanes) {
+    __shared__ uint8_t nat[64];
+    if (threadIdx.x < 64) nat[threadIdx.x] = (uint8_t)rod::jpeg::natural_order(threadIdx.x);
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31u;
+    if (lane >= lanes) return;
+    const uint32_t j = ((blockIdx.x * 128u + threadIdx.x) >> 5) * lanes + lane;
+    if (j >= n) return;
+    const ScanSeg sg = p.psegs[seg0 + j];
+    const ScanRec sc = p.scans[sg.scan];
+    if (p.status[sc.image] != 0) return;   // an earlier level found the image's data corrupt
+    const ImageRec im = p.images[sc.image];
+    const int rc = decode_prog_segment(im, sc, sg, p.huff, nat, p.streams, p.coef + im.coef_off, p.nzmask + im.coef_off / 64,
+                                       sc.Ah != 0 ? p.refine + sc.out_block : nullptr);
+    if (rc) atomicMax(p.status + sc.image, rc);
+}
+
+__global__ void __launch_bounds__(256) jpegdec_mask_kernel(JpegDecParams p, uint32_t n_blocks) {
+    __shared__ uint8_t nat[64];
+    if (threadIdx.x < 64) nat[threadIdx.x] = (uint8_t)rod::jpeg::natural_order(threadIdx.x);
+    __syncthreads();
+    const uint32_t b = blockIdx.x * 256u + threadIdx.x;
+    if (b < n_blocks) p.nzmask[b] = zigzag_nz_mask(p.coef + 64ull * b, nat);
+}
+
+// grid (blocks of the level's largest refinement scan / 256, refinement scans of the level: scans[])
+__global__ void __launch_bounds__(256) jpegdec_apply_kernel(JpegDecParams p, const uint32_t* scans) {
+    __shared__ uint8_t nat[64];
+    if (threadIdx.x < 64) nat[threadIdx.x] = (uint8_t)rod::jpeg::natural_order(threadIdx.x);
+    __syncthreads();
+    const ScanRec sc = p.scans[scans[blockIdx.y]];
+    if (p.status[sc.image] != 0) return;
+    const ImageRec im = p.images[sc.image];
+    const uint32_t j = blockIdx.x * 256u + threadIdx.x;
+    if (j >= scan_units(im, sc) * scan_blocks_per_unit(im, sc)) return;
+    apply_refinement(scan_block(p.coef + im.coef_off, im, sc, j), sc, p.refine[sc.out_block + j], nat);
 }
 
 // DC prediction (jdhuff.c: last_dc_val[ci] += diff): inclusive prefix sum of the stored differences of one component, in
@@ -365,6 +421,15 @@ struct rod_jpeg_decoder {
     std::vector<uint32_t> h_block_start, h_quad_start, h_sub_start;
     std::vector<uint2> h_ctas;
     std::vector<SegRec> h_segs;
+    std::vector<ScanRec> h_scans;        // progressive files
+    std::vector<ScanSeg> h_psegs;        // ... their restart intervals, level by level
+    std::vector<uint32_t> h_level_start; // [levels + 1] into h_psegs
+    std::vector<HuffTab> h_huff;         // ... the Huffman tables of their scans (equal tables shared)
+    std::vector<uint32_t> h_refine_scans, h_refine_start;   // ... their refinement scans by level: [levels + 1] into the list
+    std::vector<uint32_t> h_refine_max;  // ... blocks of the level's largest refinement scan
+    std::vector<char> h_level_ac_refine; // ... the level has an AC refinement scan (it needs the history masks)
+    size_t refine_blocks = 0;
+    int n_sm = 148;
     uint8_t* h_streams = nullptr;        // page-locked
     size_t stream_bytes = 0, coef_elems = 0, plane_bytes = 0;
     ImageRec* d_images = nullptr;
@@ -374,6 +439,12 @@ struct rod_jpeg_decoder {
     uint32_t* d_sub_start = nullptr;
     uint2* d_ctas = nullptr;
     SegRec* d_segs = nullptr;
+    ScanRec* d_scans = nullptr;
+    ScanSeg* d_psegs = nullptr;
+    HuffTab* d_huff = nullptr;
+    uint32_t* d_refine_scans = nullptr;
+    uint64_t* d_nzmask = nullptr;
+    RefineOut* d_refine = nullptr;
     unsigned int* d_changed = nullptr;
     uint64_t* d_end_state = nullptr;
     uint64_t* d_used_start = nullptr;
@@ -389,15 +460,20 @@ struct rod_jpeg_decoder {
     uint8_t* d_planes = nullptr;
 };
 
-extern "C" int rod_jpegdec_probe(const uint8_t* file, uint64_t n, int* height, int* width) {
-    if (file == nullptr || height == nullptr || width == nullptr) return ROD_ERR_INVALID_ARG;
+extern "C" int rod_jpegdec_probe_ex(const uint8_t* file, uint64_t n, int formats, int* height, int* width) {
+    if (file == nullptr || height == nullptr || width == nullptr || formats < 1 || formats > (kBaseline | kProgressive))
+        return ROD_ERR_INVALID_ARG;
     FileInfo info;
     std::vector<TableSet> ts(1);
-    const ParseStatus st = parse_file(file, (size_t)n, &info, &ts[0]);
-    if (st != PARSE_OK) return ROD_ERR_UNSUPPORTED;
+    const ParseStatus st = parse_file(file, (size_t)n, &info, &ts[0], formats);   // (a progressive file: every scan checked)
+    if (st != PARSE_OK || (info.progressive ? !(formats & kProgressive) : !(formats & kBaseline))) return ROD_ERR_UNSUPPORTED;
     *height = info.height;
     *width = info.width;
     return ROD_OK;
+}
+
+extern "C" int rod_jpegdec_probe(const uint8_t* file, uint64_t n, int* height, int* width) {
+    return rod_jpegdec_probe_ex(file, n, kBaseline, height, width);
 }
 
 extern "C" void rod_jpegdec_destroy(rod_jpeg_decoder* d) {
@@ -410,13 +486,17 @@ extern "C" void rod_jpegdec_destroy(rod_jpeg_decoder* d) {
     block_cache_free(d->device, d->d_end_state, d->n_sub * sizeof(uint64_t));
     block_cache_free(d->device, d->d_used_start, d->n_sub * sizeof(uint64_t));
     block_cache_free(d->device, d->d_first_block, d->n_sub * sizeof(uint32_t));
+    block_cache_free(d->device, d->d_nzmask, d->coef_elems / 64 * sizeof(uint64_t));
+    block_cache_free(d->device, d->d_refine, d->refine_blocks * sizeof(RefineOut));
     host_cache_free(d->h_streams, d->stream_bytes);
     delete d;
 }
 
-extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* lens, int n_images, const uint64_t* dst_offsets,
-                                  const int64_t* dst_pitches, int host_threads, rod_jpeg_decoder** out_dec) {
-    if (files == nullptr || lens == nullptr || dst_offsets == nullptr || n_images < 1 || out_dec == nullptr) return ROD_ERR_INVALID_ARG;
+extern "C" int rod_jpegdec_create_ex(const uint8_t* const* files, const uint64_t* lens, int n_images, const uint64_t* dst_offsets,
+                                     const int64_t* dst_pitches, int host_threads, int formats, rod_jpeg_decoder** out_dec) {
+    if (files == nullptr || lens == nullptr || dst_offsets == nullptr || n_images < 1 || out_dec == nullptr || formats < 1 ||
+        formats > (kBaseline | kProgressive))
+        return ROD_ERR_INVALID_ARG;
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return ROD_ERR_NO_DEVICE; }
     rod_jpeg_decoder* d = new (std::nothrow) rod_jpeg_decoder();
@@ -425,7 +505,7 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
     d->n_images = n_images;
     d->h_images.assign(n_images, ImageRec{});
     d->h_status.assign(n_images, 0);
-    // stream slots: a file's unstuffed scan is never longer than the file
+    // stream slots: a file's unstuffed scans are never longer than the file
     std::vector<uint64_t> slot(n_images + 1, 0);
     for (int i = 0; i < n_images; ++i) slot[i + 1] = slot[i] + ((lens[i] + 32 + 15) & ~(uint64_t)15);
     d->stream_bytes = (size_t)slot[n_images] + 64;
@@ -436,12 +516,32 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
     }
     std::vector<TableSet> per_image(n_images);
     std::vector<std::vector<SegRec>> per_image_segs(n_images);
+    std::vector<FileInfo> per_image_prog(n_images);   // progressive files: scans and tables
+    std::vector<std::vector<ScanSeg>> per_image_psegs(n_images);
     auto work = [&](int lo, int hi) {
         for (int i = lo; i < hi; ++i) {
             ImageRec& im = d->h_images[i];
             FileInfo info;
-            const ParseStatus st = files[i] ? parse_file(files[i], (size_t)lens[i], &info, &per_image[i]) : PARSE_NOT_JPEG;
+            ParseStatus st = files[i] ? parse_file(files[i], (size_t)lens[i], &info, &per_image[i], formats, d->h_streams + slot[i])
+                                      : PARSE_NOT_JPEG;
+            if (st == PARSE_OK && !(formats & (info.progressive ? kProgressive : kBaseline))) st = PARSE_UNSUPPORTED;
             if (st != PARSE_OK) { d->h_status[i] = 10 + (int)st; continue; }
+            if (info.progressive) {
+                ImageRec r{};
+                r.h = info.height; r.w = info.width;
+                r.hs = (uint8_t)info.hs; r.vs = (uint8_t)info.vs; r.ncomp = (uint8_t)info.ncomp;
+                r.stream_bytes = (uint32_t)info.stream_bytes;
+                r.stream_off = slot[i];
+                r.dst_off = dst_offsets[i];
+                r.dst_pitch = (dst_pitches && dst_pitches[i]) ? dst_pitches[i] : 3LL * info.width;
+                bool ok = true;
+                for (size_t s = 0; s < info.scans.size() && ok; ++s)   // (scan: index within the file until the batch is laid out)
+                    ok = make_scan_segments(r, info.scans[s], (uint32_t)s, slot[i], &per_image_psegs[i]);
+                if (!ok) { d->h_status[i] = 13; continue; }
+                per_image_prog[i] = std::move(info);
+                im = r;
+                continue;
+            }
             std::vector<uint32_t> rst;
             const size_t sb = unstuff_scan(files[i], (size_t)lens[i], info.scan_begin, d->h_streams + slot[i], &rst);
             if (sb == (size_t)-1) { d->h_status[i] = 13; continue; }
@@ -469,7 +569,9 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
         for (auto& t : th) t.join();
     }
     // shared table sets, buffer layout
-    std::map<std::string, int> seen;
+    std::map<std::string, int> seen, seen_huff;
+    std::vector<std::vector<ScanSeg>> by_level;
+    std::vector<std::vector<uint32_t>> refine_by_level;
     d->h_block_start.assign(n_images + 1, 0);
     d->h_quad_start.assign(n_images + 1, 0);
     d->h_sub_start.assign(1, 0);
@@ -492,6 +594,49 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
             d->plane_bytes += nblocks * 64;
             blocks += nblocks;
             quads += (uint64_t)im.h * (uint64_t)((im.w + 3) >> 2);
+            if (per_image_prog[i].progressive) {   // scans, tables, restart intervals by level
+                FileInfo& pf = per_image_prog[i];
+                std::vector<int32_t> tab(pf.huff.size());
+                for (size_t t = 0; t < pf.huff.size(); ++t) {
+                    std::string hk(reinterpret_cast<const char*>(&pf.huff[t]), sizeof(HuffTab));
+                    auto ht = seen_huff.find(hk);
+                    if (ht == seen_huff.end()) {
+                        ht = seen_huff.emplace(std::move(hk), (int)d->h_huff.size()).first;
+                        d->h_huff.push_back(pf.huff[t]);
+                    }
+                    tab[t] = ht->second;
+                }
+                std::vector<int> level;
+                const int n_levels = scan_levels(pf.scans, &level);
+                if ((int)by_level.size() < n_levels) by_level.resize(n_levels);
+                if (refine_by_level.size() < (size_t)n_levels) {
+                    refine_by_level.resize(n_levels);
+                    d->h_refine_max.resize(n_levels, 0);
+                    d->h_level_ac_refine.resize(n_levels, 0);
+                }
+                const uint32_t scan0 = (uint32_t)d->h_scans.size();
+                for (size_t s = 0; s < pf.scans.size(); ++s) {
+                    const ScanInfo& si = pf.scans[s];
+                    ScanRec r = si.rec;
+                    r.image = (uint32_t)i;
+                    for (int j = 0; j < 3; ++j) r.dc_tab[j] = si.dc_slot[j] >= 0 ? tab[si.dc_slot[j]] : -1;
+                    r.ac_tab = si.ac_slot >= 0 ? tab[si.ac_slot] : -1;
+                    if (r.Ah != 0) {   // a refinement scan: room for its results, applied after its level
+                        const uint32_t nb = scan_units(im, r) * scan_blocks_per_unit(im, r);
+                        r.out_block = (uint32_t)d->refine_blocks;
+                        d->refine_blocks += nb;
+                        refine_by_level[level[s]].push_back(scan0 + (uint32_t)s);
+                        d->h_refine_max[level[s]] = std::max(d->h_refine_max[level[s]], nb);
+                        if (r.Ss != 0) d->h_level_ac_refine[level[s]] = 1;
+                    }
+                    d->h_scans.push_back(r);
+                }
+                for (ScanSeg sg : per_image_psegs[i]) {
+                    const int lv = level[sg.scan];
+                    sg.scan += scan0;
+                    by_level[lv].push_back(sg);
+                }
+            }
             for (const SegRec& sg : per_image_segs[i]) {
                 const uint32_t bits = 8u * (sg.stream_bytes - sg.byte0);
                 const uint32_t n_sub = bits ? (bits + kSubBits - 1) / kSubBits : 1u;
@@ -506,16 +651,34 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
         d->h_quad_start[i + 1] = (uint32_t)quads;
     }
     d->n_sub = (size_t)subs;
+    d->h_level_start.assign(1, 0);
+    for (std::vector<ScanSeg>& lv : by_level) {   // the longest intervals first: they start in the first wave of the launch
+        std::stable_sort(lv.begin(), lv.end(), [](const ScanSeg& a, const ScanSeg& b) { return a.stream_bytes > b.stream_bytes; });
+        d->h_psegs.insert(d->h_psegs.end(), lv.begin(), lv.end());
+        d->h_level_start.push_back((uint32_t)d->h_psegs.size());
+    }
+    d->h_refine_start.assign(1, 0);
+    for (const std::vector<uint32_t>& lv : refine_by_level) {
+        d->h_refine_scans.insert(d->h_refine_scans.end(), lv.begin(), lv.end());
+        d->h_refine_start.push_back((uint32_t)d->h_refine_scans.size());
+    }
+    if (d->refine_blocks >= (1ull << 32)) { rod_jpegdec_destroy(d); return ROD_ERR_UNSUPPORTED; }
+    if (!d->h_psegs.empty() && cudaDeviceGetAttribute(&d->n_sm, cudaDevAttrMultiProcessorCount, d->device) != cudaSuccess) {
+        rod_jpegdec_destroy(d);
+        return cuda_fail(cudaGetLastError());
+    }
     if (blocks >= (1ull << 32) || quads >= (1ull << 32) || subs >= (1ull << 32)) { rod_jpegdec_destroy(d); return ROD_ERR_UNSUPPORTED; }
     if (d->h_tables.empty()) d->h_tables.push_back(TableSet{});
     cudaError_t err = cudaSuccess;
     auto calloc_ = [&](void** p, size_t n) { if (err == cudaSuccess) err = block_cache_alloc(d->device, p, n ? n : 16); };
     // descriptor arrays: one cached block (cudaMalloc / cudaFree per decoder would synchronise the device every batch)
-    size_t sizes[9] = {sizeof(ImageRec) * n_images, sizeof(TableSet) * d->h_tables.size(), sizeof(uint32_t) * (n_images + 1),
-                       sizeof(uint32_t) * (n_images + 1), sizeof(int32_t) * n_images, sizeof(uint32_t) * d->h_sub_start.size(),
-                       sizeof(SegRec) * d->h_segs.size(), sizeof(uint2) * d->h_ctas.size(), sizeof(unsigned int) * 4};
-    size_t offs[9];
-    for (int q = 0; q < 9; ++q) { offs[q] = d->small_bytes; d->small_bytes += (sizes[q] + 255) & ~(size_t)255; }
+    size_t sizes[13] = {sizeof(ImageRec) * n_images, sizeof(TableSet) * d->h_tables.size(), sizeof(uint32_t) * (n_images + 1),
+                        sizeof(uint32_t) * (n_images + 1), sizeof(int32_t) * n_images, sizeof(uint32_t) * d->h_sub_start.size(),
+                        sizeof(SegRec) * d->h_segs.size(), sizeof(uint2) * d->h_ctas.size(), sizeof(unsigned int) * 4,
+                        sizeof(ScanRec) * d->h_scans.size(), sizeof(ScanSeg) * d->h_psegs.size(), sizeof(HuffTab) * d->h_huff.size(),
+                        sizeof(uint32_t) * d->h_refine_scans.size()};
+    size_t offs[13];
+    for (int q = 0; q < 13; ++q) { offs[q] = d->small_bytes; d->small_bytes += (sizes[q] + 255) & ~(size_t)255; }
     calloc_((void**)&d->d_small, d->small_bytes);
     if (err == cudaSuccess) {
         d->d_images = reinterpret_cast<ImageRec*>(d->d_small + offs[0]);
@@ -527,6 +690,10 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
         d->d_segs = reinterpret_cast<SegRec*>(d->d_small + offs[6]);
         d->d_ctas = reinterpret_cast<uint2*>(d->d_small + offs[7]);
         d->d_changed = reinterpret_cast<unsigned int*>(d->d_small + offs[8]);
+        d->d_scans = reinterpret_cast<ScanRec*>(d->d_small + offs[9]);
+        d->d_psegs = reinterpret_cast<ScanSeg*>(d->d_small + offs[10]);
+        d->d_huff = reinterpret_cast<HuffTab*>(d->d_small + offs[11]);
+        d->d_refine_scans = reinterpret_cast<uint32_t*>(d->d_small + offs[12]);
     }
     calloc_((void**)&d->d_end_state, d->n_sub * sizeof(uint64_t));
     calloc_((void**)&d->d_used_start, d->n_sub * sizeof(uint64_t));
@@ -534,12 +701,21 @@ extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* l
     calloc_((void**)&d->d_streams, d->stream_bytes);
     calloc_((void**)&d->d_coef, d->coef_elems * sizeof(int16_t));
     calloc_((void**)&d->d_planes, d->plane_bytes);
+    if (d->refine_blocks) {
+        calloc_((void**)&d->d_nzmask, d->coef_elems / 64 * sizeof(uint64_t));
+        calloc_((void**)&d->d_refine, d->refine_blocks * sizeof(RefineOut));
+    }
     if (err != cudaSuccess) {
         rod_jpegdec_destroy(d);
         return cuda_fail(err);
     }
     *out_dec = d;
     return ROD_OK;
+}
+
+extern "C" int rod_jpegdec_create(const uint8_t* const* files, const uint64_t* lens, int n_images, const uint64_t* dst_offsets,
+                                  const int64_t* dst_pitches, int host_threads, rod_jpeg_decoder** out_dec) {
+    return rod_jpegdec_create_ex(files, lens, n_images, dst_offsets, dst_pitches, host_threads, kBaseline, out_dec);
 }
 
 extern "C" int rod_jpegdec_host_status(const rod_jpeg_decoder* d, int32_t* status, int32_t* heights, int32_t* widths) {
@@ -566,9 +742,17 @@ extern "C" int rod_jpegdec_decode(rod_jpeg_decoder* d, uint8_t* pixels, void* st
         ROD_CUDA(cudaMemcpyAsync(d->d_segs, d->h_segs.data(), sizeof(SegRec) * d->h_segs.size(), cudaMemcpyHostToDevice, st));
     if (!d->h_ctas.empty())
         ROD_CUDA(cudaMemcpyAsync(d->d_ctas, d->h_ctas.data(), sizeof(uint2) * d->h_ctas.size(), cudaMemcpyHostToDevice, st));
+    if (!d->h_psegs.empty()) {
+        ROD_CUDA(cudaMemcpyAsync(d->d_scans, d->h_scans.data(), sizeof(ScanRec) * d->h_scans.size(), cudaMemcpyHostToDevice, st));
+        ROD_CUDA(cudaMemcpyAsync(d->d_psegs, d->h_psegs.data(), sizeof(ScanSeg) * d->h_psegs.size(), cudaMemcpyHostToDevice, st));
+        ROD_CUDA(cudaMemcpyAsync(d->d_huff, d->h_huff.data(), sizeof(HuffTab) * d->h_huff.size(), cudaMemcpyHostToDevice, st));
+        if (!d->h_refine_scans.empty())
+            ROD_CUDA(cudaMemcpyAsync(d->d_refine_scans, d->h_refine_scans.data(), sizeof(uint32_t) * d->h_refine_scans.size(),
+                                     cudaMemcpyHostToDevice, st));
+    }
     ROD_CUDA(cudaMemcpyAsync(d->d_streams, d->h_streams, d->stream_bytes, cudaMemcpyHostToDevice, st));
     d->in_flight = true;
-    if (d->coef_elems == 0 || d->h_ctas.empty()) return ROD_OK;
+    if (d->coef_elems == 0 || (d->h_ctas.empty() && d->h_psegs.empty())) return ROD_OK;
     ROD_CUDA(cudaMemsetAsync(d->d_coef, 0, d->coef_elems * sizeof(int16_t), st));
     JpegDecParams p;
     p.images = d->d_images; p.tables = d->d_tables; p.streams = d->d_streams; p.coef = d->d_coef; p.planes = d->d_planes;
@@ -577,22 +761,43 @@ extern "C" int rod_jpegdec_decode(rod_jpeg_decoder* d, uint8_t* pixels, void* st
     p.sub_start = d->d_sub_start; p.ctas = d->d_ctas; p.end_state = d->d_end_state; p.used_start = d->d_used_start;
     p.first_block = d->d_first_block; p.changed = d->d_changed;
     p.n_images = n;
-    const unsigned n_ctas = (unsigned)d->h_ctas.size();
-    jpegdec_guess_kernel<<<n_ctas, kHuffThreads, 0, st>>>(p);
-    // synchronisation rounds, four launches per host round trip, until a launch changes no end state
-    d->sync_rounds = 0;
-    for (;;) {
-        unsigned int flags[4];
-        ROD_CUDA(cudaMemsetAsync(d->d_changed, 0, sizeof(flags), st));
-        for (int q = 0; q < 4; ++q) jpegdec_sync_kernel<<<n_ctas, kHuffThreads, 0, st>>>(p, q);
-        ROD_CUDA(cudaMemcpyAsync(flags, d->d_changed, sizeof(flags), cudaMemcpyDeviceToHost, st));
-        ROD_CUDA(cudaStreamSynchronize(st));
-        d->sync_rounds += 4;
-        if (!(flags[0] && flags[1] && flags[2] && flags[3])) break;
+    p.scans = d->d_scans; p.psegs = d->d_psegs; p.huff = d->d_huff; p.nzmask = d->d_nzmask; p.refine = d->d_refine;
+    if (!d->h_psegs.empty()) {   // progressive scans, level by level
+        const uint32_t n_sm = (uint32_t)d->n_sm;
+        for (size_t lv = 0; lv + 1 < d->h_level_start.size(); ++lv) {
+            if (d->h_level_ac_refine[lv]) {
+                const uint32_t nb = (uint32_t)(d->coef_elems / 64);
+                jpegdec_mask_kernel<<<(nb + 255) / 256, 256, 0, st>>>(p, nb);
+            }
+            const uint32_t s0 = d->h_level_start[lv], ns = d->h_level_start[lv + 1] - s0;
+            // a warp per interval while every SM gets at most 32 warps of them, more lanes per warp beyond
+            const uint32_t lanes = std::min<uint32_t>(32u, (ns + 32u * n_sm - 1) / (32u * n_sm));
+            const uint32_t warps = (ns + lanes - 1) / lanes;
+            jpegdec_prog_kernel<<<(warps + 3) / 4, 128, 0, st>>>(p, s0, ns, lanes);
+            for (uint32_t r0 = d->h_refine_start[lv]; r0 < d->h_refine_start[lv + 1]; r0 += 65535) {   // (grid.y <= 65535)
+                const uint32_t nr = std::min<uint32_t>(d->h_refine_start[lv + 1] - r0, 65535u);
+                jpegdec_apply_kernel<<<dim3((d->h_refine_max[lv] + 255) / 256, nr), 256, 0, st>>>(p, d->d_refine_scans + r0);
+            }
+        }
     }
-    jpegdec_scan_kernel<<<p.n_segs, 256, 0, st>>>(p);
-    jpegdec_write_kernel<<<n_ctas, kHuffThreads, 0, st>>>(p);
-    jpegdec_dc_kernel<<<dim3(p.n_segs, 3), 256, 0, st>>>(p);
+    const unsigned n_ctas = (unsigned)d->h_ctas.size();
+    d->sync_rounds = 0;
+    if (n_ctas > 0) {   // baseline scans
+        jpegdec_guess_kernel<<<n_ctas, kHuffThreads, 0, st>>>(p);
+        // synchronisation rounds, four launches per host round trip, until a launch changes no end state
+        for (;;) {
+            unsigned int flags[4];
+            ROD_CUDA(cudaMemsetAsync(d->d_changed, 0, sizeof(flags), st));
+            for (int q = 0; q < 4; ++q) jpegdec_sync_kernel<<<n_ctas, kHuffThreads, 0, st>>>(p, q);
+            ROD_CUDA(cudaMemcpyAsync(flags, d->d_changed, sizeof(flags), cudaMemcpyDeviceToHost, st));
+            ROD_CUDA(cudaStreamSynchronize(st));
+            d->sync_rounds += 4;
+            if (!(flags[0] && flags[1] && flags[2] && flags[3])) break;
+        }
+        jpegdec_scan_kernel<<<p.n_segs, 256, 0, st>>>(p);
+        jpegdec_write_kernel<<<n_ctas, kHuffThreads, 0, st>>>(p);
+        jpegdec_dc_kernel<<<dim3(p.n_segs, 3), 256, 0, st>>>(p);
+    }
     uint32_t max_blocks = 0, max_quads = 0;
     for (int i = 0; i < n; ++i) {
         max_blocks = std::max(max_blocks, d->h_block_start[i + 1] - d->h_block_start[i]);

@@ -11,8 +11,9 @@
 //   jdcolor.c  ycc_rgb_convert       16-bit fixed-point YCbCr -> RGB (written out as BGR)
 //              h2v1_fancy_upsample   4:2:2 files: the same filter along the row only, roundings 1 / 2
 // Supported layouts: baseline sequential (SOF0), 8 bit, one scan (with or without restart markers), either Y Cb Cr with the luma
-// sampled 2x2 (4:2:0, what OpenCV itself writes), 2x1 (4:2:2) or 1x1 (4:4:4) against 1x1 chroma, or greyscale.  Anything
-// else is reported as unsupported by the parser and the caller keeps the host codec for that file.
+// sampled 2x2 (4:2:0, what OpenCV itself writes), 2x1 (4:2:2) or 1x1 (4:4:4) against 1x1 chroma, or greyscale; and, when
+// the caller asks for them, progressive (SOF2) files of the same layouts (jdphuff.c, below).  Anything else is reported as
+// unsupported by the parser and the caller keeps the host codec for that file.
 // The same functions are compiled into tests/emu (CPU check against cv2.imdecode) and into jpegdec.cu.
 #pragma once
 #include <stdint.h>
@@ -292,6 +293,292 @@ RJ_HD uint64_t decode_span(const Layout& L, uint32_t stream_bytes, const TableSe
         }
     }
     return span_state(br.pos(), nblk, k, b);
+}
+
+// ---- progressive files (SOF2): the four MCU decoders of jdphuff.c ------------------------------------------------------
+// A progressive file codes the same quantised coefficients as its baseline twin in several scans: DC scans (Ss = Se = 0,
+// one or more components, interleaved in MCUs when more than one) and AC scans (one component, band Ss..Se); a first scan
+// (Ah = 0) codes the coefficients shifted right by Al, a refinement scan (Ah = Al + 1) one more bit of each.  Once every
+// coefficient has been refined down to Al = 0 (the parser reports every other file) the coefficients are the baseline
+// twin's, and so are the pixels (no block smoothing: libjpeg-turbo only smooths while coefficient bits are unknown).
+// The scans are decoded into the same per-component block rasters as a baseline scan; the IDCT and colour stages are shared.
+struct ScanRec {
+    uint32_t image;
+    uint8_t ncomp;               // components in the scan: 1 (non-interleaved: the component's own block raster) .. 3
+    uint8_t comp[3];             // their indices 0 .. 2, in frame order
+    uint8_t Ss, Se, Ah, Al;
+    uint32_t out_block;          // refinement scans: first block of their results in the refinement output (RefineOut)
+    int32_t dc_tab[3];           // index into the batch's HuffTab array per scan component (DC first scans), else -1
+    int32_t ac_tab;              // AC scans, else -1
+};
+
+// One restart interval of a progressive scan (a scan without restart markers: one).  Bytes as in SegRec; a UNIT is an MCU
+// of an interleaved scan and a block of a non-interleaved one.  EOBRUN and the DC predictions start from 0 in every one.
+struct ScanSeg {
+    uint64_t stream_off;
+    uint32_t scan;
+    uint32_t byte0;
+    uint32_t stream_bytes;
+    uint32_t first_unit;
+    uint32_t n_units;
+    uint32_t pad;
+};
+
+// What a refinement scan found for one block, kept apart from the coefficients so that the serial Huffman pass only
+// decodes and a parallel pass applies it (apply_refinement): bit k = zigzag position k.
+struct RefineOut {
+    uint64_t corr;               // correction bit 1 (DC refinement: bit 0)
+    uint64_t newpos;             // a new coefficient of magnitude 1 << Al
+    uint64_t newneg;             // ... and it is negative
+};
+
+RJ_HD int ctz64(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    return __ffsll((long long)x) - 1;
+#else
+    return __builtin_ctzll(x);
+#endif
+}
+RJ_HD int popc64(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    return __popcll(x);
+#else
+    return __builtin_popcountll(x);
+#endif
+}
+RJ_HD uint64_t bits_from(int k) { return k >= 64 ? 0ull : ~0ull << k; }     // positions >= k
+RJ_HD uint64_t bits_below(int k) { return k >= 64 ? ~0ull : (1ull << k) - 1; }   // positions < k
+
+// blocks across / down of component comp in a non-interleaved scan: ceil(component size / 8) (jdinput.c), not padded to MCUs
+RJ_HD int comp_blocks_w(const ImageRec& im, int comp) { return comp == 0 ? (im.w + 7) / 8 : ((im.w + im.hs - 1) / im.hs + 7) / 8; }
+RJ_HD int comp_blocks_h(const ImageRec& im, int comp) { return comp == 0 ? (im.h + 7) / 8 : ((im.h + im.vs - 1) / im.vs + 7) / 8; }
+RJ_HD uint32_t scan_units(const ImageRec& im, const ScanRec& sc) {
+    return sc.ncomp > 1 ? (uint32_t)layout_of(im).mcus : (uint32_t)comp_blocks_w(im, sc.comp[0]) * (uint32_t)comp_blocks_h(im, sc.comp[0]);
+}
+RJ_HD uint32_t scan_blocks_per_unit(const ImageRec& im, const ScanRec& sc) {
+    if (sc.ncomp == 1) return 1;
+    uint32_t n = 0;
+    for (int ci = 0; ci < sc.ncomp; ++ci) n += sc.comp[ci] == 0 ? (uint32_t)im.hs * im.vs : 1u;
+    return n;
+}
+// block (by, bx) of component comp in an image's coefficient area (the rasters of block_of: luma hs * mcu_w blocks wide,
+// chroma mcu_w).  Blocks a non-interleaved scan does not reach (right of / below ceil(size / 8)) keep zeros; they only
+// feed plane samples at x >= w / y >= h (luma) or >= the real chroma size, which the colour stage never reads.
+RJ_HD int16_t* comp_block(int16_t* coef, const Layout& L, int comp, uint32_t by, uint32_t bx) {
+    if (comp == 0) return coef + 64L * ((long)by * (L.hs * L.mcu_w) + bx);
+    return coef + 64L * (L.nl * L.mcus + (long)(comp - 1) * L.mcus + (long)by * L.mcu_w + bx);
+}
+// block j of a scan in coding order (unit j / blocks per unit; in an MCU the components' blocks in scan order)
+RJ_HD int16_t* scan_block(int16_t* coef, const ImageRec& im, const ScanRec& sc, uint32_t j) {
+    const Layout L = layout_of(im);
+    if (sc.ncomp == 1) {
+        const uint32_t bw = (uint32_t)comp_blocks_w(im, sc.comp[0]), by = j / bw;
+        return comp_block(coef, L, sc.comp[0], by, j - by * bw);
+    }
+    const uint32_t bpu = scan_blocks_per_unit(im, sc), u = j / bpu;
+    uint32_t b = j - u * bpu;
+    const uint32_t my = u / (uint32_t)L.mcu_w, mx = u - my * (uint32_t)L.mcu_w;
+    for (int ci = 0; ci < sc.ncomp; ++ci) {
+        const int comp = sc.comp[ci];
+        const uint32_t n = comp == 0 ? (uint32_t)(L.hs * L.vs) : 1u;
+        if (b < n) {
+            const uint32_t v = b / (uint32_t)(comp == 0 ? L.hs : 1), h = b - v * (uint32_t)(comp == 0 ? L.hs : 1);
+            return comp == 0 ? comp_block(coef, L, 0, L.vs * my + v, L.hs * mx + h) : comp_block(coef, L, comp, my, mx);
+        }
+        b -= n;
+    }
+    return nullptr;
+}
+
+// the nonzero coefficients of a block as a mask over zigzag positions (what an AC refinement scan needs of the history)
+RJ_HD uint64_t zigzag_nz_mask(const int16_t* blk, const uint8_t* nat) {
+    uint64_t nat_mask = 0;
+    for (int q = 0; q < 8; ++q) {   // eight 16-byte loads on the device (blocks are 128-byte aligned)
+#if defined(__CUDA_ARCH__)
+        const uint4 x = reinterpret_cast<const uint4*>(blk)[q];
+        const uint32_t w[4] = {x.x, x.y, x.z, x.w};
+#else
+        uint32_t w[4];
+        for (int j = 0; j < 4; ++j) w[j] = (uint16_t)blk[8 * q + 2 * j] | ((uint32_t)(uint16_t)blk[8 * q + 2 * j + 1] << 16);
+#endif
+        for (int j = 0; j < 4; ++j) {
+            if (w[j] & 0xFFFFu) nat_mask |= 1ull << (8 * q + 2 * j);
+            if (w[j] >> 16) nat_mask |= 1ull << (8 * q + 2 * j + 1);
+        }
+    }
+    uint64_t m = 0;
+    for (int k = 0; k < 64; ++k) m |= ((nat_mask >> nat[k]) & 1ull) << k;
+    return m;
+}
+
+// jdphuff.c decode_mcu_AC_refine's correction bits: one per position of `positions` (ascending); returns the positions
+// whose bit is 1
+RJ_HD uint64_t read_corrections(BitReader& br, uint64_t positions) {
+    uint64_t out = 0;
+    while (positions) {
+        br.refill();
+        const int c = popc64(positions) < 32 ? popc64(positions) : 32;
+        const uint32_t bits = br.peek(c);
+        br.skip(c);
+        for (int i = c - 1; i >= 0; --i) {
+            const int pos = ctz64(positions);
+            positions &= positions - 1;
+            out |= (uint64_t)((bits >> i) & 1u) << pos;
+        }
+    }
+    return out;
+}
+
+// One block of a progressive scan (jdphuff.c decode_mcu_DC_first / _AC_first / _DC_refine / _AC_refine); ci: the block's
+// index in the scan's component list, *last_dc: that component's DC prediction.  First scans write the coefficients;
+// refinement scans write *out (nz: the block's nonzero coefficients before the scan, zigzag_nz_mask).  Returns false on
+// a corrupt stream.
+RJ_HD bool decode_prog_block(BitReader& br, const ScanRec& sc, const HuffTab* tabs, const uint8_t* nat, int ci, int* last_dc,
+                             uint32_t* eobrun, int16_t* blk, uint64_t nz, RefineOut* out) {
+    const int Ss = sc.Ss, Se = sc.Se, Al = sc.Al;
+    if (Ss == 0) {
+        br.refill();
+        if (sc.Ah == 0) {   // DC first: difference to the component's prediction, stored shifted left by Al
+            const int s = decode_symbol(br, tabs[sc.dc_tab[ci]]);
+            if (s < 0 || s > 16) return false;
+            int diff = 0;
+            if (s) {
+                br.refill();
+                diff = extend(br.peek(s), s);
+                br.skip(s);
+            }
+            *last_dc += diff;
+            blk[0] = (int16_t)(int)((uint32_t)*last_dc << Al);
+        } else {            // DC refinement: one bit
+            out->corr = br.peek(1);
+            br.skip(1);
+        }
+        return true;
+    }
+    const HuffTab& ac = tabs[sc.ac_tab];
+    if (sc.Ah == 0) {       // AC first: run-length / size symbols with end-of-band runs across blocks
+        if (*eobrun > 0) { --*eobrun; return true; }
+        for (int k = Ss; k <= Se; ++k) {
+            br.refill();
+            const int sym = decode_symbol(br, ac);
+            if (sym < 0) return false;
+            const int r = sym >> 4, s = sym & 15;
+            if (s) {
+                k += r;
+                if (k > Se) return false;
+                const int v = extend(br.peek(s), s);
+                br.skip(s);
+                blk[nat[k]] = (int16_t)(int)((uint32_t)v << Al);
+            } else if (r == 15) {
+                k += 15;
+            } else {
+                *eobrun = 1u << r;
+                if (r) { *eobrun += br.peek(r); br.skip(r); }
+                --*eobrun;
+                break;
+            }
+        }
+        return true;
+    }
+    // AC refinement on masks: a symbol's run of r zeros ends at the (r + 1)-th position of the band that is zero in the
+    // history; every nonzero position passed on the way takes one correction bit (libjpeg walks them one at a time)
+    const uint64_t band = bits_from(Ss) & bits_below(Se + 1);
+    uint64_t corr = 0, newpos = 0, newneg = 0;
+    int k = Ss;
+    if (*eobrun == 0) {
+        while (k <= Se) {
+            br.refill();
+            const int sym = decode_symbol(br, ac);
+            if (sym < 0) return false;
+            const int r = sym >> 4, s = sym & 15;
+            bool neg = false;
+            if (s) {
+                if (s != 1) return false;
+                neg = br.peek(1) == 0;
+                br.skip(1);
+            } else if (r != 15) {
+                *eobrun = 1u << r;
+                if (r) { br.refill(); *eobrun += br.peek(r); br.skip(r); }
+                break;
+            }
+            uint64_t zeros = ~nz & band & bits_from(k);
+            for (int i = 0; i < r && zeros; ++i) zeros &= zeros - 1;
+            const int t = zeros ? ctz64(zeros) : Se + 1;   // the new coefficient's position (ZRL: the 16th zero)
+            corr |= read_corrections(br, nz & band & bits_from(k) & bits_below(t));
+            if (s) {
+                if (t > Se) return false;
+                newpos |= 1ull << t;
+                if (neg) newneg |= 1ull << t;
+            }
+            k = t + 1;
+        }
+    }
+    if (*eobrun > 0) {      // inside an end-of-band run: only the correction bits of the remaining nonzero coefficients
+        corr |= read_corrections(br, nz & band & bits_from(k));
+        --*eobrun;
+    }
+    out->corr = corr;
+    out->newpos = newpos;
+    out->newneg = newneg;
+    return true;
+}
+
+// What decode_prog_block found for block blk of refinement scan sc, applied (the parallel pass after a level).
+RJ_HD void apply_refinement(int16_t* blk, const ScanRec& sc, const RefineOut& o, const uint8_t* nat) {
+    const int p1 = 1 << sc.Al, m1 = (int)(~0u << sc.Al);
+    if (sc.Ss == 0) {
+        if (o.corr) blk[0] = (int16_t)(blk[0] | p1);
+        return;
+    }
+    for (uint64_t c = o.corr; c; c &= c - 1) {
+        const int z = nat[ctz64(c)], v = blk[z];
+        if ((v & p1) == 0) blk[z] = (int16_t)(v + (v >= 0 ? p1 : m1));
+    }
+    for (uint64_t n = o.newpos; n; n &= n - 1) {
+        const int k = ctz64(n);
+        blk[nat[k]] = (int16_t)(((o.newneg >> k) & 1u) ? m1 : p1);
+    }
+}
+
+// One restart interval of a progressive scan, sequentially.  coef: the image's coefficient area; refinement scans read
+// nz (the image's blocks' zigzag_nz_mask, same block order as coef) and write out (the scan's RefineOut, in coding
+// order).  Returns 0, or 1 (corrupt code), 2 (ran past the end of the segment).
+RJ_HD int decode_prog_segment(const ImageRec& im, const ScanRec& sc, const ScanSeg& sg, const HuffTab* tabs, const uint8_t* nat,
+                              const uint8_t* streams, int16_t* coef, const uint64_t* nz, RefineOut* out) {
+    const Layout L = layout_of(im);
+    BitReader br;
+    br.init_at(streams + sg.stream_off, sg.stream_bytes, 8u * sg.byte0);
+    int dc0 = 0, dc1 = 0, dc2 = 0;   // the DC predictions of the scan's components (scalars: no local-memory array)
+    uint32_t eobrun = 0;
+    const bool ac_refine = sc.Ah != 0 && sc.Ss != 0;
+    uint32_t j = sg.first_unit * scan_blocks_per_unit(im, sc);   // block index in coding order
+    if (sc.ncomp == 1) {
+        const int comp = sc.comp[0];
+        const uint32_t bw = (uint32_t)comp_blocks_w(im, comp);
+        for (uint32_t u = sg.first_unit; u < sg.first_unit + sg.n_units; ++u, ++j) {
+            const uint32_t by = u / bw;
+            int16_t* blk = comp_block(coef, L, comp, by, u - by * bw);
+            if (!decode_prog_block(br, sc, tabs, nat, 0, &dc0, &eobrun, blk, ac_refine ? nz[(blk - coef) >> 6] : 0ull,
+                                   out ? out + j : nullptr))
+                return 1;
+        }
+    } else {   // interleaved: DC scans only (the parser checks), no history needed
+        for (uint32_t u = sg.first_unit; u < sg.first_unit + sg.n_units; ++u) {
+            const uint32_t my = u / (uint32_t)L.mcu_w, mx = u - my * (uint32_t)L.mcu_w;
+            for (int ci = 0; ci < sc.ncomp; ++ci) {
+                const int comp = sc.comp[ci];
+                const int bh = comp == 0 ? L.vs : 1, bwid = comp == 0 ? L.hs : 1;
+                int pred = ci == 0 ? dc0 : (ci == 1 ? dc1 : dc2);
+                for (int v = 0; v < bh; ++v)
+                    for (int h = 0; h < bwid; ++h, ++j)
+                        if (!decode_prog_block(br, sc, tabs, nat, ci, &pred, &eobrun,
+                                               comp_block(coef, L, comp, bh * my + v, bwid * mx + h), 0ull,
+                                               out ? out + j : nullptr)) return 1;
+                if (ci == 0) dc0 = pred; else if (ci == 1) dc1 = pred; else dc2 = pred;
+            }
+        }
+    }
+    return br.bits_used() > 8ull * sg.stream_bytes ? 2 : 0;
 }
 
 // jidctint.c jpeg_idct_islow: 64 quantised coefficients (natural order) x quantisation table -> 64 samples 0..255.

@@ -1,5 +1,5 @@
 """Device-side JPEG encoding whose files equal cv2.imwrite's byte for byte, and device-side JPEG decoding whose pixels
-equal cv2.imread's (SURVEY 8f rank 1).
+equal cv2.imread's (SURVEY 8f rank 1): baseline files, and with progressive=True progressive ones.
 
 `cv2.imwrite(str(dst_img_dir / img_path.name), out)` (scripts/build_corrupted_testsets.py:124, :164) is the last step of
 the test-set build; with the corruption on the GPU it is what the build spends its time in.  JpegEncoder encodes a
@@ -119,11 +119,16 @@ class JpegEncoder:
         return out
 
 
-def probe(data) -> Optional[Tuple[int, int]]:
-    """(height, width) when the device decoder takes this JPEG file (bytes-like), else None (host codec)."""
+def _formats(progressive: bool) -> int:
+    return N.JPEGDEC_BASELINE | (N.JPEGDEC_PROGRESSIVE if progressive else 0)
+
+
+def probe(data, progressive: bool = False) -> Optional[Tuple[int, int]]:
+    """(height, width) when the device decoder takes this JPEG file (bytes-like), else None (host codec).  Progressive
+    files count only with progressive=True (the file is then walked to its end: every scan is checked)."""
     buf = np.frombuffer(data, dtype=np.uint8)
     h, w = ctypes.c_int(), ctypes.c_int()
-    rc = N.lib().rod_jpegdec_probe(buf.ctypes.data, buf.size, ctypes.byref(h), ctypes.byref(w))
+    rc = N.lib().rod_jpegdec_probe_ex(buf.ctypes.data, buf.size, _formats(progressive), ctypes.byref(h), ctypes.byref(w))
     return (h.value, w.value) if rc == N.ROD_OK else None
 
 
@@ -133,11 +138,13 @@ class JpegDecoder:
     given to decode(), row pitch 3 * width unless `pitches` says otherwise -- the layout of a CorruptionPlan built from
     `shapes`.  The constructor does the host work (markers, Huffman tables, scans copied without their byte stuffing into
     page-locked memory, on `host_threads` threads); `shapes[i]` is (h, w), or None where the device decoder does not take
-    the file (it takes baseline 4:2:0 / 4:2:2 / 4:4:4 / greyscale files; with or without restart
-    markers; not: progressive, EXIF rotation,
-    CMYK, not a JPEG ...): the caller reads those with the host codec.  No CPU decoding inside."""
+    the file (it takes baseline 4:2:0 / 4:2:2 / 4:4:4 / greyscale files, with or without restart markers, and with
+    progressive=True progressive files of the same layouts whose scans refine every coefficient to the last bit -- the
+    pixels of their baseline twin, as cv2.imread and PIL give them; not: EXIF rotation, CMYK, arithmetic coding, not a
+    JPEG ...): the caller reads those with the host codec.  No CPU decoding inside."""
 
-    def __init__(self, files: Sequence, offsets: Sequence[int], pitches: Optional[Sequence[int]] = None, host_threads: int = 8):
+    def __init__(self, files: Sequence, offsets: Sequence[int], pitches: Optional[Sequence[int]] = None, host_threads: int = 8,
+                 progressive: bool = False):
         N.require_device()
         n = len(files)
         self._bufs = [np.frombuffer(f, dtype=np.uint8) for f in files]   # keeps the file bytes alive for create()
@@ -146,7 +153,8 @@ class JpegDecoder:
         offs = (ctypes.c_uint64 * n)(*[int(o) for o in offsets])
         pit = (ctypes.c_int64 * n)(*[int(q) for q in pitches]) if pitches is not None else None
         handle = ctypes.c_void_p()
-        N.check(N.lib().rod_jpegdec_create(ptrs, lens, n, offs, pit, int(host_threads), ctypes.byref(handle)), "rod_jpegdec_create")
+        N.check(N.lib().rod_jpegdec_create_ex(ptrs, lens, n, offs, pit, int(host_threads), _formats(progressive), ctypes.byref(handle)),
+                "rod_jpegdec_create_ex")
         self._h = handle
         self._bufs = None   # the scans were copied
         self.n_images = n
@@ -178,6 +186,6 @@ class JpegDecoder:
         return st
 
 
-def sizes_of(files: Sequence) -> List[Optional[Tuple[int, int]]]:
+def sizes_of(files: Sequence, progressive: bool = False) -> List[Optional[Tuple[int, int]]]:
     """probe() for a list of files."""
-    return [probe(f) for f in files]
+    return [probe(f, progressive) for f in files]
