@@ -4,11 +4,21 @@
 // kernel = k taps of float32(1/k) on one row, BORDER_REFLECT_101, i.e. per channel
 //     out[x] = round(sum_{j=-r..r} in[reflect101(x + j)] / k)  ==  (2 S + k) / (2 k)   (odd k).
 //
-// Rows are independent, so one warp owns one row at a time: the row is staged in shared
-// memory with 16-byte cp.async copies at the SAME 16-byte phase as its destination address,
-// the reflected halo is written next to it, and every lane then produces 16 output bytes per
-// step from three 128-bit shared-memory loads and stores them with one 128-bit global store.
-// No block-level barrier is used (warps never share data), only __syncwarp().
+// Rows are independent.  A CTA runs one producer warp and up to 8 consumer warps around a ring of row slots in shared
+// memory.  The producer (one lane) claims 8-row tiles from a work counter, one claim ahead of use, and for each row waits
+// until its slot is free, writes the slot's descriptor and starts one bulk async copy (cp.async.bulk, completing on the
+// slot's "full" mbarrier) of the row's 16-byte-aligned interior, placed at the SAME 16-byte phase as the destination row.
+// Consumer warp i takes rows i, i + W, i + 2W, ... of the CTA's sequence: it loads the (at most two) partial 16-byte
+// edges itself, writes the reflected halo next to the row, and every lane then produces 16 output bytes per step from
+// three 128-bit shared-memory loads and stores them with one 128-bit global store; then it frees the slot.  Rows whose
+// source and destination phases differ are copied into the slot by the consumer byte by byte.
+// So the bytes of the next rows are in flight while the consumers compute, and the claims are off their path.
+//
+// The work counter and a "done" counter are a pair of the plan's blur counters.  Each CTA counts itself done after its
+// final, failing claim; the CTA that completes the count returns both to 0, so the next launch that takes the pair finds
+// it zeroed without a memset.
+
+#include <algorithm>
 
 #include "rod_internal.h"
 
@@ -22,50 +32,148 @@ struct BlurParams {
     uint8_t* dst;
     const uint8_t* opcodes;
     int k;
-    int row_buf_bytes;  // shared bytes per warp
-    unsigned int* counter;  // zeroed before the launch
+    int row_buf_bytes;      // shared bytes per row slot
+    int slots;              // row slots per CTA (>= consumer warps)
+    unsigned int* counters;  // {work counter, done counter}: 0 at the launch, returned to 0 by the last CTA
 };
 
-constexpr int kBlurLeft = 64;  // bytes in front of the 16-byte block that holds pixel 0 (>= 3*15 halo + 16)
+constexpr int kBlurLeft = 64;      // bytes in front of the 16-byte block that holds pixel 0 (>= 3*15 halo + 16)
+constexpr int kBlurMaxSlots = 16;  // row slots per CTA
+constexpr int kBlurCtasPerSm = 3;  // 16 slots of a 1360-wide row (4 224 B) each: 48 rows in flight per SM
 
-__device__ __forceinline__ void cp_async16(uint32_t smem_addr, const void* gptr) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_addr), "l"(gptr) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() {
-    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
-}
+// Per-slot header, in front of the row buffers.  The producer writes it before it arrives on `full`.
+struct BlurSlot {
+    uint64_t full, empty;  // mbarriers: full completes on the producer's arrival + the bulk copy, empty on the consumer's
+    const uint8_t* srow;   // nullptr: no more rows for this consumer
+    uint8_t* drow;
+    int32_t w, pad[3];
+};
+static_assert(sizeof(BlurSlot) % 16 == 0, "row buffers follow the headers at 16-byte alignment");
+
 __device__ __forceinline__ void stg16_blur(void* p, uint4 v) {
     asm volatile("st.global.L1::no_allocate.v4.u32 [%0], {%1,%2,%3,%4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z),
                  "r"(v.w)
                  : "memory");
 }
+__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
+    asm volatile(
+        "{\n.reg .pred p;\nBLUR_WAIT_%=:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+        "@!p bra BLUR_WAIT_%=;\n}" ::"r"(bar), "r"(parity)
+        : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+// claim the next tile.  ptxas still gives this atom its warp-aggregated form (a SHFL that waits for the result), but the
+// wait falls on the producer lane, one tile ahead of the consumers
+__device__ __forceinline__ unsigned int claim_tile(unsigned int* counter) {
+    unsigned int v;
+    asm volatile("atom.global.add.u32 %0, [%1], 1;" : "=r"(v) : "l"(counter));
+    return v;
+}
 
 template <int K>  // K == 9: specialised fast path; K == 0: generic odd k
-__global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
+__global__ void __launch_bounds__(32 * (kBlurRowsPerTile + 1), kBlurCtasPerSm) blur_rows_kernel(BlurParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
+    BlurSlot* slots = reinterpret_cast<BlurSlot*>(smem);
+    uint8_t* bufs = smem + (size_t)p.slots * sizeof(BlurSlot);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint8_t* buf = smem + (size_t)warp * p.row_buf_bytes;
-    const uint32_t buf_s = (uint32_t)__cvta_generic_to_shared(buf);
+    const int consumers = (int)(blockDim.x >> 5) - 1;  // the last warp is the producer
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < p.slots; ++s) {
+            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&slots[s].full)));
+            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(&slots[s].empty)));
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+
+    if (warp == consumers) {
+        // ---- producer: one lane claims tiles and feeds their rows into the ring in order
+        if (lane != 0) return;
+        int s = 0;
+        uint32_t ph = 0;  // parity of the ring pass the producer is filling
+        auto next_slot = [&]() -> BlurSlot& {
+            BlurSlot& sl = slots[s];
+            mbar_wait(smem_addr(&sl.empty), ph ^ 1u);  // the consumer of the previous pass has freed it
+            return sl;
+        };
+        auto advance = [&]() {
+            if (++s == p.slots) { s = 0; ph ^= 1u; }
+        };
+        unsigned int next = claim_tile(p.counters);
+        for (;;) {
+            const unsigned int ti = next;
+            if (ti >= (unsigned int)p.n_tiles) break;
+            next = claim_tile(p.counters);  // in flight while this tile's rows are issued
+            const Tile t = p.tiles[ti];
+            if (p.opcodes != nullptr && p.opcodes[t.img] != ROD_OP_BLUR) continue;
+            const DevImage im = p.images[t.img];
+            const int n = 3 * im.w;
+            for (int y = t.a; y < t.a + t.b; ++y) {
+                const uint8_t* srow = p.src + im.src_off + (int64_t)y * im.src_pitch;
+                uint8_t* drow = p.dst + im.dst_off + (int64_t)y * im.dst_pitch;
+                const int shift = (int)((uintptr_t)drow & 15);
+                const int jf0 = (shift != 0) ? 1 : 0, jf1 = (n + shift) >> 4;
+                BlurSlot& sl = next_slot();
+                sl.srow = srow;
+                sl.drow = drow;
+                sl.w = im.w;
+                const uint32_t full = smem_addr(&sl.full);
+                if (((((uintptr_t)srow ^ (uintptr_t)drow) & 15) == 0) && jf1 > jf0) {
+                    const uint32_t bytes = 16u * (uint32_t)(jf1 - jf0);
+                    const uint32_t dst_s = smem_addr(bufs + (size_t)s * p.row_buf_bytes + kBlurLeft + 16 * jf0);
+                    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(bytes) : "memory");
+                    asm volatile(
+                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_s),
+                        "l"(srow - shift + 16 * jf0), "r"(bytes), "r"(full)
+                        : "memory");
+                } else {
+                    mbar_arrive(full);
+                }
+                advance();
+            }
+        }
+        // every claim of this CTA is back: count it done; the last CTA to do so returns the pair to 0
+        __threadfence();
+        if (atomicAdd(p.counters + 1, 1u) == gridDim.x - 1) {
+            __threadfence();
+            atomicExch(p.counters, 0u);
+            atomicExch(p.counters + 1, 0u);
+        }
+        for (int c = 0; c < consumers; ++c) {  // one "no more rows" per consumer: the next `consumers` slots of the sequence
+            BlurSlot& sl = next_slot();
+            sl.srow = nullptr;
+            mbar_arrive(smem_addr(&sl.full));
+            advance();
+        }
+        return;
+    }
+
+    // ---- consumers: warp i takes slots i, i + consumers, ... of the ring
     const int k = (K == 0) ? p.k : K;
     const int halo = 3 * (k >> 1);
-
-    // each warp takes a whole tile (8 consecutive rows) at a time from a shared counter and filters its rows one by one
-    for (int sub = 8, ti = 0;;) {
-        if (sub >= 8) {
-            if (lane == 0) ti = (int)atomicAdd(p.counter, 1u);
-            ti = __shfl_sync(0xFFFFFFFFu, ti, 0);
-            sub = 0;
-        }
-        if (ti >= p.n_tiles) break;
-        const Tile t = p.tiles[ti];
-        const int wr = sub++;
-        if (p.opcodes != nullptr && p.opcodes[t.img] != ROD_OP_BLUR) { sub = 8; continue; }
-        if (wr >= t.b) { sub = 8; continue; }
-        const DevImage im = p.images[t.img];
-        const int y = t.a + wr;
-        const int n = 3 * im.w;
-        const uint8_t* srow = p.src + im.src_off + (int64_t)y * im.src_pitch;
-        uint8_t* drow = p.dst + im.dst_off + (int64_t)y * im.dst_pitch;
+    int s = warp;
+    uint32_t ph = 0;
+    for (;; s += consumers) {
+        if (s >= p.slots) { s -= p.slots; ph ^= 1u; }
+        BlurSlot& sl = slots[s];
+        // A parity wait only tells an mbarrier's current phase from the one before it.  The slot's previous pass may have
+        // gone to another consumer (the slot count need not be a multiple of the consumer count), and bulk copies into
+        // different slots complete out of order, so its "full" barrier can still be a phase behind: waiting on it directly
+        // could return on that stale phase.  The previous pass is over once its consumer has freed the slot ("empty"
+        // within one phase of it, since the producer waited for the pass before); only then does "full" mean this pass.
+        // The producer waits for the same event before it starts this pass's copy, so this costs no time.
+        mbar_wait(smem_addr(&sl.empty), ph ^ 1u);
+        mbar_wait(smem_addr(&sl.full), ph);
+        const uint8_t* srow = sl.srow;
+        if (srow == nullptr) break;
+        uint8_t* drow = sl.drow;
+        const int w = sl.w;
+        uint8_t* buf = bufs + (size_t)s * p.row_buf_bytes;
+        const int n = 3 * w;
         const int shift = (int)((uintptr_t)drow & 15);
         uint8_t* row = buf + kBlurLeft + shift;  // byte of pixel 0
         // chunk j covers row positions [16j - shift, 16j - shift + 16); chunks [jf0, jf1) lie fully inside [0, n)
@@ -73,14 +181,11 @@ __global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
         const int jf1 = (n + shift) >> 4;
         const bool right_edge = ((n + shift) & 15) != 0;
 
-        // ---- stage the row: smem byte (kBlurLeft + shift + i) = in[i]
+        // ---- complete the row: smem byte (kBlurLeft + shift + i) = in[i]
         if ((((uintptr_t)srow ^ (uintptr_t)drow) & 15) == 0) {
-            const uint8_t* sal = srow - shift;  // 16-byte aligned
-            for (int j = jf0 + lane; j < jf1; j += 32) cp_async16(buf_s + kBlurLeft + 16 * j, sal + 16 * j);
-            // the (at most two) partial chunks: one byte per lane
+            // the interior came with the bulk copy; the (at most two) partial chunks: one byte per lane
             const int i = (lane < 16) ? (lane - shift) : (16 * jf1 - shift + lane - 16);
             if (((lane < 16) ? (shift != 0) : right_edge) && i >= 0 && i < n) row[i] = srow[i];
-            cp_async_wait_all();
         } else {
             for (int i = lane; i < n; i += 32) row[i] = srow[i];
         }
@@ -92,8 +197,8 @@ __global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
                 const int px = (i >= 0) ? i / 3 : -((-i + 2) / 3);       // floor(i / 3)
                 const int c = i - 3 * px;
                 int rp;
-                if (im.w > (k >> 1)) rp = (px < 0) ? -px : 2 * (im.w - 1) - px;  // single reflection
-                else rp = reflect101(px, im.w);                                   // tiny rows: periodic
+                if (w > (k >> 1)) rp = (px < 0) ? -px : 2 * (w - 1) - px;  // single reflection
+                else rp = reflect101(px, w);                               // tiny rows: periodic
                 row[i] = row[3 * rp + c];
             }
         }
@@ -104,9 +209,9 @@ __global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
             for (int j = jf0 + lane; j < jf1; j += 32) {
                 const uint4* wp = reinterpret_cast<const uint4*>(buf + kBlurLeft + 16 * j - 16);
                 const uint4 a = wp[0], b = wp[1], c = wp[2];
-                const uint32_t w[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+                const uint32_t win[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
                 uint32_t out[4];
-                blur9_chunk16(w, out);
+                blur9_chunk16(win, out);
                 stg16_blur(dal + 16 * j, make_uint4(out[0], out[1], out[2], out[3]));
             }
             // partial chunks: lane 0 takes the left one, lane 1 the right one
@@ -114,9 +219,9 @@ __global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
                 const int j = (lane == 0) ? 0 : jf1;
                 const uint4* wp = reinterpret_cast<const uint4*>(buf + kBlurLeft + 16 * j - 16);
                 const uint4 a = wp[0], b = wp[1], c = wp[2];
-                const uint32_t w[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
+                const uint32_t win[12] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w};
                 uint32_t out[4];
-                blur9_chunk16(w, out);
+                blur9_chunk16(win, out);
                 const int lo = 16 * j - shift;
                 for (int bb = 0; bb < 16; ++bb) {
                     const int i = lo + bb;
@@ -149,7 +254,10 @@ __global__ void __launch_bounds__(256, 4) blur_rows_kernel(BlurParams p) {
                 }
             }
         }
-        __syncwarp();  // the row buffer is reused by this warp's next row
+        // the slot's bytes written here (edges, halo) must be ordered before the next bulk copy into it
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncwarp();
+        if (lane == 0) mbar_arrive(smem_addr(&sl.empty));
     }
 }
 
@@ -162,27 +270,28 @@ int launch_blur(const rod_plan* plan, const uint8_t* src, uint8_t* dst, int k, c
     p.tiles = tiles;
     p.n_tiles = n_tiles;
     p.src = src; p.dst = dst; p.opcodes = opcodes; p.k = k;
-    // per-warp buffer: kBlurLeft | (shift + 3w rounded up to 16) | 16 (right window) + halo, 16-byte multiple
+    // row slot: kBlurLeft | (shift + 3w rounded up to 16) | 16 (right window) + halo, 16-byte multiple
     const int row_bytes = 3 * plan->max_w;
     p.row_buf_bytes = kBlurLeft + ((15 + row_bytes + 15) & ~15) + 64;
-    // one row buffer per warp: very wide rows run with fewer warps per CTA (the kernel has no block-level coupling)
-    int warps = kBlurRowsPerTile;
-    while (warps > 1 && (size_t)p.row_buf_bytes * warps > 227 * 1024) --warps;
-    const size_t smem = (size_t)p.row_buf_bytes * warps;
-    if (smem > 227 * 1024) return ROD_ERR_UNSUPPORTED;  // a single row does not fit: wider than ~77 000 pixels
-    int ctas_per_sm = (int)((227 * 1024) / (smem + 1024));
-    if (ctas_per_sm < 1) ctas_per_sm = 1;
-    // measured on B200 (256 x 1360x765): 4 resident CTAs (32 warps) per SM -> 5.79 TB/s; 5 -> 5.62; 6 -> 5.57; 3 -> 5.66
-    if (ctas_per_sm > 4) ctas_per_sm = 4;
-    p.counter = plan->d_counters + (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
-    ROD_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(unsigned int), stream));
-    const int grid = grid_for(plan, (p.n_tiles + warps - 1) / warps, ctas_per_sm);
+    const size_t slot_bytes = sizeof(BlurSlot) + (size_t)p.row_buf_bytes;
+    constexpr size_t kSmem = 227 * 1024, kPerCta = 1024;  // per-SM budget; the runtime reserves 1 KB per CTA
+    // up to kBlurMaxSlots slots in a third of the SM; wider rows: at least one slot per consumer warp, down to one slot
+    size_t slots = std::min<size_t>(kBlurMaxSlots, (kSmem / kBlurCtasPerSm - kPerCta) / slot_bytes);
+    if (slots < (size_t)kBlurRowsPerTile) slots = std::min<size_t>(kBlurRowsPerTile, kSmem / slot_bytes);
+    if (slots < 1) return ROD_ERR_UNSUPPORTED;  // a single row does not fit: wider than ~77 000 pixels
+    p.slots = (int)slots;
+    const int consumers = std::min(kBlurRowsPerTile, p.slots);
+    const size_t smem = slots * slot_bytes;
+    const int ctas_per_sm = std::max(1, std::min(kBlurCtasPerSm, (int)(kSmem / (smem + kPerCta))));
+    p.counters = plan->d_blur_counters + 2 * (plan->launch_seq.fetch_add(1u) & (kCounterRing - 1u));
+    const int grid = grid_for(plan, n_tiles, ctas_per_sm);
+    const int threads = 32 * (consumers + 1);
     if (k == 9) {
         ROD_CUDA(cudaFuncSetAttribute(blur_rows_kernel<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        blur_rows_kernel<9><<<grid, 32 * warps, smem, stream>>>(p);
+        blur_rows_kernel<9><<<grid, threads, smem, stream>>>(p);
     } else {
         ROD_CUDA(cudaFuncSetAttribute(blur_rows_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        blur_rows_kernel<0><<<grid, 32 * warps, smem, stream>>>(p);
+        blur_rows_kernel<0><<<grid, threads, smem, stream>>>(p);
     }
     ROD_CUDA(cudaGetLastError());
     return ROD_OK;

@@ -330,6 +330,11 @@ extern "C" int rod_plan_create(const rod_image_desc* images, int n_images, rod_p
             plan->monotonic = false;
     }
     if (plan_alloc(plan, (void**)&plan->d_counters, kCounterRing * sizeof(unsigned int)) != cudaSuccess) { rod_plan_destroy(plan); return ROD_ERR_OOM; }
+    if (plan_alloc(plan, (void**)&plan->d_blur_counters, 2 * kCounterRing * sizeof(unsigned int)) != cudaSuccess) { rod_plan_destroy(plan); return ROD_ERR_OOM; }
+    // block-cache memory comes back recycled: zero the blur pairs once, done before the plan is handed out
+    e = cudaMemset(plan->d_blur_counters, 0, 2 * kCounterRing * sizeof(unsigned int));
+    if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+    if (e != cudaSuccess) { rod_plan_destroy(plan); return cuda_fail(e); }
     int rc = upload(plan, plan->h_images, &plan->d_images);
     if (rc == ROD_OK) rc = upload_tiles(plan, nt, &plan->noise_tiles);
     if (rc == ROD_OK) rc = upload_tiles(plan, bt, &plan->blur_tiles);
@@ -387,7 +392,7 @@ extern "C" void rod_plan_destroy(rod_plan* plan) {
     if (plan->d_patch_corrupted) cudaFree(plan->d_patch_corrupted);
     void* ptrs[] = {plan->d_images, plan->noise_tiles.d, plan->blur_tiles.d, plan->d_shapes, plan->d_tab, plan->d_lb,
                     plan->d_lb_tab, plan->lb_tiles.d, plan->d_scratch, plan->d_stage_src, plan->d_f2d_taps,
-                    plan->f2d_tiles.d, plan->d_counters, plan->d_stage_dst, plan->d_stage_noise, plan->d_stage_ops,
+                    plan->f2d_tiles.d, plan->d_counters, plan->d_blur_counters, plan->d_stage_dst, plan->d_stage_noise, plan->d_stage_ops,
                     plan->chw_tiles.d, plan->d_chw_off};
     for (void* p : ptrs) plan_free(plan, p);
     for (const TileList& l : plan->lowres) plan_free(plan, l.d);

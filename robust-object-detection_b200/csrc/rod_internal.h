@@ -92,6 +92,8 @@ struct rod_plan {
     // on several streams / from several host threads, so the slot index is taken atomically and the ring is long
     // enough (4096 launches) that a slot is never reused while its launch is still pending
     unsigned int* d_counters = nullptr;
+    // the blur launches' own ring of counter pairs (blur.cu): zeroed once here, and every launch leaves its pair at 0
+    unsigned int* d_blur_counters = nullptr;
     mutable std::atomic<unsigned int> launch_seq{0};
     bool monotonic = true;  // image extents are disjoint and increasing in both src and dst
     int gauss_generator = ROD_GAUSS_AUTO;  // Philox-mode Gaussian generator (rod_plan_set_gaussian_generator)
